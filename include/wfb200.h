@@ -403,6 +403,32 @@ int wfb_build_records_v1725(const uint8_t* blob_dev, int64_t blob_bytes, const i
                             const int16_t* channel_dev, const uint16_t* baseline_dev, const uint8_t* trunc_dev, int64_t n,
                             int32_t dt_ns, void* records_aos_dev, uint16_t* pool_dev, int64_t pool_len,
                             wfb_rec_meta* meta_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+/* The same for a part of a run read from a subset of its files: seq_dev[i] is the global index of waveform i
+ * (its index in the concatenation of ALL files of the run, in list order) and becomes the row's record_id;
+ * the local index columns must follow the files in list order.  The workspace is
+ * wfb_build_records_v1725_workspace_bytes(n). */
+int wfb_build_records_v1725_seq(const uint8_t* blob_dev, int64_t blob_bytes, const int64_t* payload_offset_dev,
+                                const int32_t* n_samples_dev, const int64_t* timestamp_dev, const int16_t* board_dev,
+                                const int16_t* channel_dev, const uint16_t* baseline_dev, const uint8_t* trunc_dev,
+                                const int64_t* seq_dev, int64_t n, int32_t dt_ns, void* records_aos_dev, uint16_t* pool_dev,
+                                int64_t pool_len, wfb_rec_meta* meta_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/* Time shards of a run built on several GPUs (distributed.build_records_sharded_v1725).  Rows are ordered by
+ * the key (timestamp, board, channel, record_id), record_id holding the global seq.
+ * wfb_record_split_points: for each of n_keys keys (int64 timestamp, board, channel, record_id, 4 per key)
+ * the number of the n sorted RECORDS rows whose key is smaller (lower bound).
+ * wfb_merge_record_runs: rows_in holds n_runs strictly increasing runs, run r at rows
+ * [run_offsets_host[r], run_offsets_host[r + 1]), and pool_in their samples in the same order (no gaps).
+ * Writes the merged rows with record_id = record_base + i and wave_offset = pool_base + the running sum of
+ * event_length, all other fields unchanged, the samples in output order (pool_len = the total) and
+ * wfb_rec_meta rows.  A run that is not strictly increasing: WFB_ERR_INVALID, nothing written.
+ * Synchronizes the stream once (after that check). */
+int wfb_record_split_points(const void* rows_dev, int64_t n, const int64_t* keys_dev, int64_t n_keys, int64_t* out_dev,
+                            void* stream);
+size_t wfb_merge_record_runs_workspace_bytes(int64_t n, int64_t n_runs);
+int wfb_merge_record_runs(const void* rows_in_dev, const uint16_t* pool_in_dev, int64_t n_in, const int64_t* run_offsets_host,
+                          int64_t n_runs, int64_t record_base, int64_t pool_base, void* rows_out_dev, uint16_t* pool_out_dev,
+                          int64_t pool_len, wfb_rec_meta* meta_out_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /* hit_merge (core/plugins/builtin/cpu/hit_merge.py:115-181 cluster chain, :256-322 merged rows) on
  * packed THRESHOLD_HIT rows: per hardware channel, hits ordered by absolute window start are chained

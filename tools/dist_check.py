@@ -10,7 +10,15 @@ rows never leave the device, the ranks exchange their boundary zones (one all_ga
 two counts.  With --verify 1 rank 0 additionally processes the WHOLE run on its own GPU and checks that the ranks'
 feature rows, hit rows, merged rows (after the channel-major assembly) and event ids equal the single-GPU ones byte
 for byte; at sizes that no single GPU holds (--verify 0) the check is structural: counts add up, every rank's windows
-lie between its cuts, event ids are contiguous across ranks."""
+lie between its cuts, event ids are contiguous across ranks.
+
+--source v1725 starts from files instead: every rank writes its own V1725 .bin files (file i seeded by i, board i, all
+16 channels, --samples per waveform; every file spans the same time range, so the exchange moves (P - 1) / P of every
+rank's records), builds its time shard with ``distributed.build_records_sharded_v1725`` and runs the same fused ->
+merge_group_sharded path.  It reports the time of every ingest stage, the exchange bytes and rate, the merge kernel's
+rate against its algorithmic bytes (4 L + 252 per record), the peak device memory, and the GPU name and power limit;
+with --verify 1 rank 0 rebuilds all files on one GPU and checks records, pool, features, hits, merged rows and event
+ids byte for byte."""
 import argparse
 import os
 import sys
@@ -23,18 +31,22 @@ import torch.distributed as dist
 
 from waveformanalysis_b200 import distributed as D
 from waveformanalysis_b200 import engine, ops
-from waveformanalysis_b200.dtypes import HIT_MERGED_DTYPE, THRESHOLD_HIT_DTYPE
+from waveformanalysis_b200.dtypes import HIT_MERGED_DTYPE, RECORDS_DTYPE, THRESHOLD_HIT_DTYPE
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--records-per-rank", type=int, default=1_000_000)
 ap.add_argument("--verify", type=int, default=1)
 ap.add_argument("--zone-rows", type=int, default=4096)
+ap.add_argument("--source", choices=("synth", "v1725"), default="synth")
+ap.add_argument("--files-per-rank", type=int, default=2)
+ap.add_argument("--samples", type=int, default=800)
 args = ap.parse_args()
 
 D.init_process_group("nccl")
 rank, ws, local = D.world()
 torch.cuda.set_device(local)
-n, L, NCH, SEED = args.records_per_rank, 800, 16, 4242
+n, L, NCH, SEED = args.records_per_rank, args.samples, 16, 4242
+DT_V1725 = 4
 THR, WINDOW, GAP = 15.0, 100.0, 50.0
 
 
@@ -49,14 +61,85 @@ def fused(run):
     return res, total
 
 
-run = engine.DeviceRun.synth(n, L, NCH, seed=SEED, record_base=rank * n)
+def v1725_file(i: int, n_events: int) -> np.ndarray:
+    """Stream of file i: board i, every event fires all 16 channels with L samples; seeded by i alone."""
+    rng = np.random.default_rng(1000 + i)
+    ev_dt = np.dtype([("hdr", "u1", 16), ("ch", [("hdr", "u1", 12), ("wave", "<i2", L)], 16)])
+    a = np.zeros(n_events, ev_dt)
+    a["hdr"][:, 4] = a["hdr"][:, 11] = 0xFF
+    size = 3 + L // 2
+    step = rng.integers(1, 4 * L, n_events)
+    step[::5] = 0  # events sharing a timestamp
+    t = np.cumsum(step).astype(np.int64)
+    ts = t[:, None] + rng.integers(0, 3, (n_events, 16))
+    ch = a["ch"]
+    ch["hdr"][..., 0], ch["hdr"][..., 1], ch["hdr"][..., 2] = size & 0xFF, (size >> 8) & 0xFF, (size >> 16) & 0x3F
+    for b in range(6):
+        ch["hdr"][..., 4 + b] = (ts >> (8 * b)) & 0xFF
+    ch["hdr"][..., 10], ch["hdr"][..., 11] = 8000 & 0xFF, 8000 >> 8
+    block = (8000 + rng.integers(-4, 5, 1 << 20)).astype(np.int16)
+    for k in range(0, len(block) - 40, 997):  # negative pulses
+        block[k:k + 12] -= 150
+    windows = np.lib.stride_tricks.sliding_window_view(block, L)
+    for e0 in range(0, n_events, 2048):
+        e1 = min(e0 + 2048, n_events)
+        ch["wave"][e0:e1] = windows[rng.integers(0, len(windows), (e1 - e0, 16))]
+    return a.view(np.uint8)
+
+
+def v1725_name(i: int) -> str:
+    return f"run_b{i}_seg0.bin"
+
+
+ingest = None
+if args.source == "v1725":
+    import shutil
+    import subprocess
+    import tempfile
+
+    F = ws * args.files_per_rank
+    ev_per_file = max(n // (NCH * args.files_per_rank), 1)
+    tmp = tempfile.mkdtemp(prefix=f"v1725_r{rank}_")
+    paths = [os.path.join(tmp, v1725_name(i)) for i in range(F)]  # every rank lists every file; it writes its own
+    mine = list(range(rank * args.files_per_rank, (rank + 1) * args.files_per_rank))
+    for i in mine:
+        v1725_file(i, ev_per_file).tofile(paths[i])
+    torch.cuda.reset_peak_memory_stats()
+    if ws > 1:
+        dist.barrier()
+    tw = time.perf_counter()
+    ingest = D.build_records_sharded_v1725(paths, dt_ns=DT_V1725, mine=mine)
+    torch.cuda.synchronize()
+    wall = time.perf_counter() - tw
+    peak = torch.cuda.max_memory_allocated()
+    shutil.rmtree(tmp, ignore_errors=True)
+    run = ingest["run"]
+    n = run.n
+    tm = ingest["timings"]
+    n_all = ingest["n_total"]
+    merge_bytes = (4 * L + 252) * run.n
+    gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", str(local)],
+                         capture_output=True, text=True).stdout.strip()
+    line = (f"rank {rank}: records {run.n} (base {ingest['record_base']}) | " +
+            " ".join(f"{k} {1e3 * v:.1f} ms" for k, v in tm.items()) +
+            f" | exchange {ingest['exchange_bytes'] / 1e9:.3f} GB received, {ingest['exchange_bytes'] / max(tm['exchange'], 1e-9) / 1e9:.1f} GB/s"
+            f" | merge {merge_bytes / max(tm['merge'], 1e-9) / 1e9:.0f} GB/s of {4 * L + 252} B/record"
+            f" | ingest wall {1e3 * wall:.1f} ms, {n_all / wall / 1e6:.1f} M records/s run-wide"
+            f" | peak device memory {peak / 1e9:.2f} GB ({peak / max(2 * run.pool_len, 1):.2f} x the shard's sample bytes) | {gpu}")
+    lines = D.gather_rows(np.frombuffer(line.encode().ljust(1024)[:1024], dtype="S1024")) if ws > 1 else [line.encode()]
+    if rank == 0:
+        print(f"v1725 ingest: world={ws} files={F} records={n_all} samples/record={L}")
+        for ln in lines:
+            print("  " + ln.decode().strip())
+else:
+    run = engine.DeviceRun.synth(n, L, NCH, seed=SEED, record_base=rank * n)
 res, total = fused(run)
 if ws > 1:
     dist.barrier()
 torch.cuda.synchronize()
 t0 = time.perf_counter()
 sh = D.merge_group_sharded((res["hits"][: total * 60], total), D.DeviceRows(THRESHOLD_HIT_DTYPE), time_window_ns=WINDOW, merge_gap_ns=GAP,
-                           span_ns=L * 2.0, zone_rows=args.zone_rows)
+                           span_ns=(run.lmax * DT_V1725 if ingest is not None else L * 2.0), zone_rows=args.zone_rows)
 torch.cuda.synchronize()
 if ws > 1:
     dist.barrier()
@@ -88,12 +171,24 @@ if args.verify:
     hits = D.gather_rows(hits_l)
     merged = D.gather_rows(merged_l)
     evs = D.gather_rows(ev_l)["e"]
+    if ingest is not None:
+        recs_all = D.gather_rows(run.records_rows[: n * 102].cpu().numpy().view(RECORDS_DTYPE))
+        pool_all = D.gather_rows(run.pool.cpu().numpy().view([("s", "<u2")]))["s"]
     if rank == 0:
         del run, res, sh
         torch.cuda.empty_cache()
-        full = engine.DeviceRun.synth(n * ws, L, NCH, seed=SEED)
+        if ingest is not None:
+            want_rec, want_pool = ops.build_records_from_v1725([v1725_file(i, ev_per_file) for i in range(F)],
+                                                               [v1725_name(i) for i in range(F)], DT_V1725)
+            assert recs_all.tobytes() == want_rec.tobytes(), "records differ"
+            assert np.array_equal(pool_all, want_pool), "wave_pool differs"
+            full = engine.DeviceRun.from_host(want_rec, want_pool)
+            del want_pool, pool_all
+        else:
+            full = engine.DeviceRun.synth(n * ws, L, NCH, seed=SEED)
+        n_all = full.n
         fres, ftotal = fused(full)
-        assert np.array_equal(feats.view(np.uint8).reshape(-1), fres["features"][: n * ws * 36].cpu().numpy()), "features differ"
+        assert np.array_equal(feats.view(np.uint8).reshape(-1), fres["features"][: n_all * 36].cpu().numpy()), "features differ"
         assert np.array_equal(hits.view(np.uint8).reshape(-1), fres["hits"][: ftotal * 60].cpu().numpy()), "hit rows differ"
         m = ops.hit_merge_device(fres["hits"][: ftotal * 60], ftotal, merge_gap_ns=GAP)
         g = ops.group_rows_device(m["merged"], m["n_clusters"], 72, WINDOW, abs_start=m["abs_start"], abs_end=m["abs_end"])
@@ -108,7 +203,8 @@ if args.verify:
         assert np.array_equal(got_ev, want_ev), "event ids differ"
         assert g["n_events"] == int(tot[3])
         merged_over = int((want_m["component_count"] > 1).sum())
-        msg += f" | byte-identical to the single-GPU run ({n * ws} records, {merged_over} clusters of several hits)"
+        what = "records, pool, " if ingest is not None else ""
+        msg += f" | {what}features, hits, merged rows and event ids byte-identical to the single-GPU run ({n_all} records, {merged_over} clusters of several hits)"
 if rank == 0:
     print("dist_check OK:", msg, f"backend={dist.get_backend() if ws > 1 else 'single'}")
 if ws > 1:

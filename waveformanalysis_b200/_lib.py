@@ -156,6 +156,10 @@ PROTOTYPES = {
     "wfb_v1725_scan_host": (C.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(_i64), C.POINTER(_i64)]),
     "wfb_build_records_v1725_workspace_bytes": (_sz, [_i64]),
     "wfb_build_records_v1725": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
+    "wfb_build_records_v1725_seq": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
+    "wfb_record_split_points": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp]),
+    "wfb_merge_record_runs_workspace_bytes": (_sz, [_i64, _i64]),
+    "wfb_merge_record_runs": (C.c_int, [_vp, _vp, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "wfb_hit_merge_workspace_bytes": (_sz, [_i64]),
     "wfb_hit_merge": (C.c_int, [_vp, _i64, _dbl, _dbl, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "wfb_filter_pool": (C.c_int, [_vp, _i32, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _sz, _i32, _vp]),

@@ -32,55 +32,10 @@ int sm_count() {
     return n;
 }
 
-// ---- RECORDS_DTYPE (102 B packed, 2-byte aligned rows) -> wfb_rec_meta -----------------------
-// field offsets: core/processing/dtypes.py:80-100
-//   timestamp i8@0  pid i4@8  board i2@12  channel i2@14  baseline f8@16  baseline_upstream f8@24
-//   polarity U8@32 (UTF-32, 32 B)  record_id i8@64  dt i4@72  trigger_type i2@76  flags u4@78
-//   wave_offset i8@82  event_length i4@90  time i8@94
-__device__ __forceinline__ unsigned long long rd64(const uint16_t* h) {
-    return (unsigned long long)h[0] | ((unsigned long long)h[1] << 16) | ((unsigned long long)h[2] << 32) |
-           ((unsigned long long)h[3] << 48);
-}
-__device__ __forceinline__ unsigned rd32(const uint16_t* h) { return (unsigned)h[0] | ((unsigned)h[1] << 16); }
-
 __global__ void records_unpack_kernel(const uint16_t* __restrict__ rows, long long n, wfb_rec_meta* __restrict__ meta) {
     long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const uint16_t* h = rows + i * (kRecordsRowBytes / 2);
-    wfb_rec_meta m;
-    m.timestamp = (long long)rd64(h + 0);
-    m.board = (short)h[6];
-    m.channel = (short)h[7];
-    m.baseline = __longlong_as_double((long long)rd64(h + 8));
-    // polarity: 'positive' / 'negative' / other, compared on the first UTF-32 code units and the
-    // terminator so that e.g. 'pos' is not mistaken for 'positive'
-    unsigned c0 = rd32(h + 16), c1 = rd32(h + 18), c7 = rd32(h + 30);
-    int pol = WFB_POL_UNKNOWN;
-    if (c7 == 'e') {
-        // full 8-character compare
-        const char* pos = "positive";
-        const char* neg = "negative";
-        bool isp = true, isn = true;
-        for (int k = 0; k < 8; ++k) {
-            unsigned ck = rd32(h + 16 + 2 * k);
-            isp = isp && ck == (unsigned)pos[k];
-            isn = isn && ck == (unsigned)neg[k];
-        }
-        pol = isp ? WFB_POL_POSITIVE : (isn ? WFB_POL_NEGATIVE : WFB_POL_UNKNOWN);
-    }
-    if (c0 == 'r' && c1 == 'a') {  // internal tag "rawpos" (waveformanalysis_b200/aos.py)
-        const char* rp = "rawpos";
-        bool isr = true;
-        for (int k = 0; k < 8; ++k) isr = isr && rd32(h + 16 + 2 * k) == (k < 6 ? (unsigned)rp[k] : 0u);
-        if (isr) pol = WFB_POL_RAW_POSITIVE;
-    }
-    m.polarity = (uint8_t)pol;
-    m.pad_[0] = m.pad_[1] = m.pad_[2] = 0;
-    m.record_id = (long long)rd64(h + 32);
-    m.dt = (int)rd32(h + 36);
-    m.wave_offset = (long long)rd64(h + 41);
-    m.event_length = (int)rd32(h + 45);
-    meta[i] = m;
+    meta[i] = rec_meta_from_row(rows + i * (kRecordsRowBytes / 2));
 }
 
 // keeps the first non-zero error flag of the chunks of one wfb_process_host call (the per-call flag in the workspace

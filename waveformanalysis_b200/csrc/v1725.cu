@@ -69,7 +69,7 @@ __global__ void __launch_bounds__(256) v1725_gather_kernel(const uint8_t* __rest
                                                           const double* __restrict__ baseline_f64,
                                                           const unsigned char* __restrict__ trunc,
                                                           const long long* __restrict__ order, const long long* __restrict__ len_incl,
-                                                          long long n, int dt_ns, long long ts_scale, int bl_start, int bl_end,
+                                                          const long long* __restrict__ seq, long long n, int dt_ns, long long ts_scale, int bl_start, int bl_end,
                                                           long long epoch_ns, long long blob_bytes, long long pool_len,
                                                           uint16_t* __restrict__ rows, uint16_t* __restrict__ pool,
                                                           wfb_rec_meta* __restrict__ meta) {
@@ -79,6 +79,7 @@ __global__ void __launch_bounds__(256) v1725_gather_kernel(const uint8_t* __rest
     const long long src = order[r];
     const int len = n_samples[src];
     const long long wave_offset = len_incl[r] - len;
+    const long long rid = seq != nullptr ? seq[src] : r;
     // payloads start on 4-byte boundaries of the stream; the destination only on 2-byte ones
     const uint16_t* in = reinterpret_cast<const uint16_t*>(blob + payload_off[src]);
     uint16_t* out = pool + wave_offset;
@@ -110,7 +111,7 @@ __global__ void __launch_bounds__(256) v1725_gather_kernel(const uint8_t* __rest
         m.channel = channel[src];
         m.polarity = WFB_POL_UNKNOWN;
         m.pad_[0] = m.pad_[1] = m.pad_[2] = 0;
-        m.record_id = r;
+        m.record_id = rid;
         meta[r] = m;
     }
     if (rows != nullptr) {
@@ -119,8 +120,8 @@ __global__ void __launch_bounds__(256) v1725_gather_kernel(const uint8_t* __rest
         t += epoch_ns;
         const unsigned fl = trunc != nullptr ? (unsigned)trunc[src] : 0u;
         uint16_t* row = rows + r * (kRecordsRowBytes / 2);
-        row[lane] = v1725_row_halfword(lane, ts, board[src], channel[src], bl, r, dt_ns, fl, wave_offset, len, t);
-        if (lane + 32 < 51) row[lane + 32] = v1725_row_halfword(lane + 32, ts, board[src], channel[src], bl, r, dt_ns, fl, wave_offset, len, t);
+        row[lane] = v1725_row_halfword(lane, ts, board[src], channel[src], bl, rid, dt_ns, fl, wave_offset, len, t);
+        if (lane + 32 < 51) row[lane + 32] = v1725_row_halfword(lane + 32, ts, board[src], channel[src], bl, rid, dt_ns, fl, wave_offset, len, t);
     }
 }
 
@@ -179,10 +180,12 @@ extern "C" size_t wfb_build_records_v1725_workspace_bytes(int64_t n) {
     return 6 * m + radix_sort_workspace_bytes(n) + scan_workspace_bytes(n) + 512;
 }
 
-// common device part: sort, ragged offsets, gather
+// common device part: sort, ragged offsets, gather.  seq_dev != NULL: record_id = seq[source index] instead of the
+// output position (a rank's part of a run numbered over all files, shard_records.cu)
 static int build_records_ragged(const uint8_t* blob_dev, int64_t blob_bytes, const int64_t* payload_offset_dev, const int32_t* n_samples_dev,
                                 const int64_t* timestamp_dev, long long ts_scale, const int16_t* board_dev, const int16_t* channel_dev,
-                                const uint16_t* baseline_u16_dev, const double* baseline_f64_dev, const uint8_t* flags_dev, int64_t n,
+                                const uint16_t* baseline_u16_dev, const double* baseline_f64_dev, const uint8_t* flags_dev,
+                                const int64_t* seq_dev, int64_t n,
                                 int32_t dt_ns, int32_t bl_start, int32_t bl_end, int64_t epoch_ns, void* records_aos_dev, uint16_t* pool_dev,
                                 int64_t pool_len, wfb_rec_meta* meta_dev, void* workspace_dev, size_t workspace_bytes, cudaStream_t st,
                                 const char* who) {
@@ -217,7 +220,8 @@ static int build_records_ragged(const uint8_t* blob_dev, int64_t blob_bytes, con
     if (rc != WFB_OK) return rc;
     v1725_gather_kernel<<<v_nb(n * 32), 256, 0, st>>>(blob_dev, reinterpret_cast<const long long*>(payload_offset_dev), n_samples_dev,
                                                       reinterpret_cast<const long long*>(timestamp_dev), board_dev, channel_dev,
-                                                      baseline_u16_dev, baseline_f64_dev, flags_dev, vA, len_incl, n, dt_ns, ts_scale,
+                                                      baseline_u16_dev, baseline_f64_dev, flags_dev, vA, len_incl,
+                                                      reinterpret_cast<const long long*>(seq_dev), n, dt_ns, ts_scale,
                                                       bl_start, bl_end, epoch_ns, blob_bytes, pool_len,
                                                       static_cast<uint16_t*>(records_aos_dev), pool_dev, meta_dev);
     WFB_CUDA(cudaGetLastError());
@@ -230,9 +234,20 @@ extern "C" int wfb_build_records_ragged(const void* samples_dev, int64_t samples
                                         int32_t bl_start, int32_t bl_end, int64_t epoch_ns, void* records_aos_dev, uint16_t* pool_dev,
                                         int64_t pool_len, wfb_rec_meta* meta_dev, void* workspace_dev, size_t workspace_bytes, void* stream) {
     return build_records_ragged(static_cast<const uint8_t*>(samples_dev), samples_bytes, sample_offset_dev, n_samples_dev, timestamp_ps_dev, 1,
-                                board_dev, channel_dev, nullptr, baselines_in_dev, nullptr, n, dt_ns, bl_start, bl_end, epoch_ns,
+                                board_dev, channel_dev, nullptr, baselines_in_dev, nullptr, nullptr, n, dt_ns, bl_start, bl_end, epoch_ns,
                                 records_aos_dev, pool_dev, pool_len, meta_dev, workspace_dev, workspace_bytes,
                                 static_cast<cudaStream_t>(stream), "wfb_build_records_ragged");
+}
+
+static int build_v1725(const uint8_t* blob_dev, int64_t blob_bytes, const int64_t* payload_offset_dev, const int32_t* n_samples_dev,
+                       const int64_t* timestamp_dev, const int16_t* board_dev, const int16_t* channel_dev, const uint16_t* baseline_dev,
+                       const uint8_t* trunc_dev, const int64_t* seq_dev, int64_t n, int32_t dt_ns, void* records_aos_dev, uint16_t* pool_dev,
+                       int64_t pool_len, wfb_rec_meta* meta_dev, void* workspace_dev, size_t workspace_bytes, void* stream, const char* who) {
+    WFB_REQUIRE(n == 0 || (baseline_dev && trunc_dev), "%s: NULL pointer", who);
+    WFB_REQUIRE(n == 0 || ((uintptr_t)blob_dev & 3) == 0, "%s: the stream must be 4-byte aligned", who);
+    return build_records_ragged(blob_dev, blob_bytes, payload_offset_dev, n_samples_dev, timestamp_dev, (long long)dt_ns * 1000ll, board_dev,
+                                channel_dev, baseline_dev, nullptr, trunc_dev, seq_dev, n, dt_ns, 0, 0, 0, records_aos_dev, pool_dev, pool_len,
+                                meta_dev, workspace_dev, workspace_bytes, static_cast<cudaStream_t>(stream), who);
 }
 
 extern "C" int wfb_build_records_v1725(const uint8_t* blob_dev, int64_t blob_bytes, const int64_t* payload_offset_dev,
@@ -240,9 +255,19 @@ extern "C" int wfb_build_records_v1725(const uint8_t* blob_dev, int64_t blob_byt
                                        const int16_t* channel_dev, const uint16_t* baseline_dev, const uint8_t* trunc_dev, int64_t n,
                                        int32_t dt_ns, void* records_aos_dev, uint16_t* pool_dev, int64_t pool_len,
                                        wfb_rec_meta* meta_dev, void* workspace_dev, size_t workspace_bytes, void* stream) {
-    WFB_REQUIRE(n == 0 || (baseline_dev && trunc_dev), "wfb_build_records_v1725: NULL pointer");
-    WFB_REQUIRE(n == 0 || ((uintptr_t)blob_dev & 3) == 0, "wfb_build_records_v1725: the stream must be 4-byte aligned");
-    return build_records_ragged(blob_dev, blob_bytes, payload_offset_dev, n_samples_dev, timestamp_dev, (long long)dt_ns * 1000ll, board_dev,
-                                channel_dev, baseline_dev, nullptr, trunc_dev, n, dt_ns, 0, 0, 0, records_aos_dev, pool_dev, pool_len, meta_dev,
-                                workspace_dev, workspace_bytes, static_cast<cudaStream_t>(stream), "wfb_build_records_v1725");
+    return build_v1725(blob_dev, blob_bytes, payload_offset_dev, n_samples_dev, timestamp_dev, board_dev, channel_dev, baseline_dev, trunc_dev,
+                       nullptr, n, dt_ns, records_aos_dev, pool_dev, pool_len, meta_dev, workspace_dev, workspace_bytes, stream,
+                       "wfb_build_records_v1725");
+}
+
+extern "C" int wfb_build_records_v1725_seq(const uint8_t* blob_dev, int64_t blob_bytes, const int64_t* payload_offset_dev,
+                                           const int32_t* n_samples_dev, const int64_t* timestamp_dev, const int16_t* board_dev,
+                                           const int16_t* channel_dev, const uint16_t* baseline_dev, const uint8_t* trunc_dev,
+                                           const int64_t* seq_dev, int64_t n, int32_t dt_ns, void* records_aos_dev, uint16_t* pool_dev,
+                                           int64_t pool_len, wfb_rec_meta* meta_dev, void* workspace_dev, size_t workspace_bytes,
+                                           void* stream) {
+    WFB_REQUIRE(n == 0 || seq_dev != nullptr, "wfb_build_records_v1725_seq: NULL seq");
+    return build_v1725(blob_dev, blob_bytes, payload_offset_dev, n_samples_dev, timestamp_dev, board_dev, channel_dev, baseline_dev, trunc_dev,
+                       seq_dev, n, dt_ns, records_aos_dev, pool_dev, pool_len, meta_dev, workspace_dev, workspace_bytes, stream,
+                       "wfb_build_records_v1725_seq");
 }

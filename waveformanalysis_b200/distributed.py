@@ -425,3 +425,426 @@ def assemble_merged(merged_all: np.ndarray, event_of_merged_all: np.ndarray):
     key = merged_all["board"].astype(np.int64) * 65536 + (merged_all["channel"].astype(np.int64) + 32768)
     o = np.argsort(key, kind="stable")
     return merged_all[o], np.asarray(event_of_merged_all)[o]
+
+
+# ------------------------------------------------------------------------------------------------
+# Time shards built straight from V1725 files: per-rank build, sample-sort exchange, merge
+# ------------------------------------------------------------------------------------------------
+# The single-GPU order of a V1725 run is lexsort((seq, channel, board, pid = 0, timestamp)) over all files, seq = the
+# waveform's index in the concatenation of all files in list order.  The key (timestamp, board, channel, seq) is
+# unique, so the order is exact whichever rank reads which file:
+#   1. every rank scans and builds only its own files, each row's record_id holding the global seq (the ranks learn
+#      the per-file waveform counts from one all-gather);
+#   2. every rank samples s = 256 x world_size keys of its sorted rows; all ranks pick the same world_size - 1
+#      splitters at the weighted quantiles of the gathered samples (plan_splitters);
+#   3. a lower-bound search cuts the local rows at the splitters: each destination's part is one contiguous row range
+#      and one contiguous sample range (the local wave_offsets are a running sum);
+#   4. all_to_all_single of the counts, then of the rows (102 B each) and of the samples (2 B each);
+#   5. one all-gather of the received counts gives the shard's global record and sample bases;
+#   6. the received runs (sorted, in source-rank order) are merged by rank and renumbered for the shard's place.
+# Every rank sends (P - 1) / P of its rows and samples on average: (P - 1) / P x (2 L + 102) bytes per record.
+
+SPLITTER_SAMPLES_PER_RANK = 256  # s = SPLITTER_SAMPLES_PER_RANK x world_size samples per rank
+
+
+def key_order(keys: np.ndarray, tie: np.ndarray | None = None) -> np.ndarray:
+    """The host restatement of the records order: indices that sort ``keys`` (int64 rows of timestamp, board, channel,
+    seq) ascending; ``tie`` (optional) breaks ties between equal keys, then the input order (stable)."""
+    k = np.asarray(keys, dtype=np.int64).reshape(-1, 4)
+    cols = (k[:, 3], k[:, 2], k[:, 1], k[:, 0])
+    return np.lexsort(((tie,) if tie is not None else ()) + cols)
+
+
+def record_keys(rec: np.ndarray) -> np.ndarray:
+    """(n, 4) int64 keys of RECORDS rows whose record_id holds seq."""
+    return np.stack([rec["timestamp"].astype(np.int64), rec["board"].astype(np.int64), rec["channel"].astype(np.int64),
+                     rec["record_id"].astype(np.int64)], axis=1).reshape(-1, 4)
+
+
+def lower_bounds(sorted_keys: np.ndarray, queries: np.ndarray) -> np.ndarray:
+    """For every key of ``queries`` (ascending) the number of ``sorted_keys`` that are smaller."""
+    q = np.asarray(queries, dtype=np.int64).reshape(-1, 4)
+    both = np.concatenate([q, np.asarray(sorted_keys, dtype=np.int64).reshape(-1, 4)])
+    o = key_order(both, tie=np.r_[np.zeros(len(q), np.int8), np.ones(len(both) - len(q), np.int8)])
+    place = np.empty(len(both), dtype=np.int64)
+    place[o] = np.arange(len(both))
+    return place[: len(q)] - np.arange(len(q))
+
+
+def splitter_samples(n: int, s: int):
+    """Positions of the (at most ``s``) sampled rows of ``n`` sorted rows and their weights: sample i stands for the
+    rows from its position up to the next sample's."""
+    k = min(int(n), int(s))
+    pos = (np.arange(k + 1, dtype=np.int64) * int(n)) // max(k, 1)
+    return pos[:k], np.diff(pos)
+
+
+def plan_splitters(keys: np.ndarray, weights: np.ndarray, n_shards: int) -> np.ndarray:
+    """The ``n_shards - 1`` splitters (int64 rows of timestamp, board, channel, seq) that cut the run into shards of
+    about equal counts, from the samples of every rank (``keys`` with their ``weights``, any order): splitter j is the
+    first sample (in key order) with at least j / n_shards of the total weight before it; past the last sample it is
+    a key above every record.  Every rank passes the same gathered samples and gets the same splitters."""
+    k = np.asarray(keys, dtype=np.int64).reshape(-1, 4)
+    w = np.asarray(weights, dtype=np.int64)
+    o = key_order(k)
+    k, w = k[o], w[o]
+    before = (np.cumsum(w) - w) * int(n_shards)
+    total = int(w.sum())
+    out = np.full((max(int(n_shards) - 1, 0), 4), np.iinfo(np.int64).max, dtype=np.int64)
+    for j in range(1, int(n_shards)):
+        m = int(np.searchsorted(before, j * total, side="left"))
+        if m < len(k):
+            out[j - 1] = k[m]
+    return out
+
+
+def default_file_owners(sizes, world_size: int) -> np.ndarray:
+    """Owner rank of every file: contiguous blocks of the list balanced by size (a file goes to the rank whose equal
+    share of the total bytes holds the file's middle byte)."""
+    sz = np.asarray(sizes, dtype=np.float64)
+    P = int(world_size)
+    if len(sz) == 0:
+        return np.zeros(0, dtype=np.int64)
+    total = float(sz.sum())
+    if total <= 0:
+        return (np.arange(len(sz), dtype=np.int64) * P) // len(sz)
+    mid = np.cumsum(sz) - sz / 2
+    return np.minimum((mid * P / total).astype(np.int64), P - 1)
+
+
+def _dist():
+    import torch.distributed as dist
+
+    if dist.is_available() and dist.is_initialized():
+        return dist, dist.get_rank(), dist.get_world_size()
+    return None, 0, 1
+
+
+def _allreduce_max(v: int) -> int:
+    import torch
+
+    dist, _, ws = _dist()
+    if ws == 1:
+        return int(v)
+    t = torch.tensor([int(v)], dtype=torch.int64, device=_device_for_collectives())
+    dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    return int(t.item())
+
+
+def _exchange(rows, pool, row_counts, sample_counts, backend):
+    """all_to_all_single of the per-destination counts, then of the row bytes and the sample bytes (uneven splits).
+    Returns the received (rows, pool) byte tensors and the per-source (rows, samples) counts."""
+    import torch
+
+    dist, _, P = _dist()
+    if P == 1:
+        return rows, pool, np.stack([row_counts, sample_counts], axis=1)
+    dev = _device_for_collectives()
+    c = torch.from_numpy(np.stack([row_counts, sample_counts], axis=1).reshape(-1).astype(np.int64)).to(dev)
+    rc = torch.empty_like(c)
+    dist.all_to_all_single(rc, c)
+    recv = rc.cpu().numpy().reshape(P, 2)
+    out_rows = backend.empty_bytes(int(recv[:, 0].sum()) * 102)
+    dist.all_to_all_single(out_rows, rows, output_split_sizes=(recv[:, 0] * 102).tolist(), input_split_sizes=(row_counts * 102).tolist())
+    out_pool = backend.empty_bytes(int(recv[:, 1].sum()) * 2)
+    dist.all_to_all_single(out_pool, pool, output_split_sizes=(recv[:, 1] * 2).tolist(), input_split_sizes=(sample_counts * 2).tolist())
+    return out_rows, out_pool, recv
+
+
+class HostRecords:
+    """Backend for the records of a rank held as numpy arrays (CPU tests over gloo): the oracle's scan, the host key
+    order for the local sort and the merge."""
+
+    def __init__(self, scan_fn):
+        self.scan_fn = scan_fn
+
+    def sync(self):
+        pass
+
+    def scan(self, blob):
+        s = dict(self.scan_fn(blob))
+        s["bytes"] = blob
+        return s
+
+    def upload(self, scans, names):
+        return scans, names
+
+    def build(self, up, dt_ns: int, seq: np.ndarray):
+        from . import ops
+        from .dtypes import RECORDS_DTYPE
+
+        scans, names = up
+        n = len(seq)
+        rec = np.zeros(n, dtype=RECORDS_DTYPE)
+        if n == 0:
+            return rec, np.zeros(0, dtype=np.uint16)
+        cat = {k: np.concatenate([s[k] for s in scans]) for k in ("payload_offset", "n_samples", "channel", "timestamp", "baseline", "trunc")}
+        board = np.concatenate([np.full(len(s["channel"]), ops.v1725_board_from_name(nm), dtype=np.int16) for s, nm in zip(scans, names)])
+        waves = [np.frombuffer(s["bytes"], dtype=np.uint8)[o:o + 2 * m].view(np.uint16)
+                 for s in scans for o, m in zip(s["payload_offset"].tolist(), s["n_samples"].tolist())]
+        ts = cat["timestamp"] * np.int64(int(dt_ns) * 1000)
+        order = key_order(np.stack([ts, board.astype(np.int64), cat["channel"].astype(np.int64), seq], axis=1))
+        rec["timestamp"], rec["board"], rec["channel"] = ts[order], board[order], cat["channel"][order]
+        rec["baseline"] = cat["baseline"][order].astype(np.float64)
+        rec["baseline_upstream"] = np.nan
+        rec["polarity"] = "unknown"
+        rec["record_id"] = seq[order]
+        rec["dt"] = int(dt_ns)
+        rec["flags"] = cat["trunc"][order]
+        lens = cat["n_samples"][order].astype(np.int64)
+        rec["event_length"] = lens
+        rec["wave_offset"] = np.cumsum(lens) - lens
+        rec["time"] = rec["timestamp"] // 1000
+        return rec, np.concatenate([waves[i] for i in order.tolist()]).astype(np.uint16, copy=False)
+
+    def count(self, local):
+        return len(local[0])
+
+    def n_samples(self, local):
+        return len(local[1])
+
+    def rows_at(self, local, idx):
+        return local[0][np.asarray(idx, dtype=np.int64)]
+
+    def split_points(self, local, splitters):
+        return lower_bounds(record_keys(local[0]), splitters)
+
+    def send_buffers(self, local):
+        import torch
+
+        return (torch.from_numpy(np.ascontiguousarray(local[0]).view(np.uint8).reshape(-1)),
+                torch.from_numpy(np.ascontiguousarray(local[1]).view(np.uint8).reshape(-1)))
+
+    def empty_bytes(self, nbytes: int):
+        import torch
+
+        return torch.empty(int(nbytes), dtype=torch.uint8)
+
+    def merge(self, rows, pool, run_offsets, record_base: int, pool_base: int):
+        from .dtypes import RECORDS_DTYPE
+
+        rec = rows.numpy().view(RECORDS_DTYPE)
+        samples = pool.numpy().view(np.uint16)
+        keys = record_keys(rec)
+        for a, b in zip(run_offsets[:-1], run_offsets[1:]):
+            k = keys[a:b]
+            if not (np.array_equal(key_order(k), np.arange(len(k))) and not np.any(np.all(k[1:] == k[:-1], axis=1))):
+                raise ValueError("wfb_merge_record_runs: a run is not strictly increasing in (timestamp, board, channel, record_id)")
+        order = key_order(keys)
+        lens = rec["event_length"].astype(np.int64)
+        out = rec[order].copy()
+        out_lens = lens[order]
+        out_start = np.cumsum(out_lens) - out_lens
+        out["record_id"] = int(record_base) + np.arange(len(out), dtype=np.int64)
+        out["wave_offset"] = int(pool_base) + out_start
+        in_start = (np.cumsum(lens) - lens)[order]
+        idx = np.arange(int(out_lens.sum()), dtype=np.int64) + np.repeat(in_start - out_start, out_lens)
+        return out, samples[idx]
+
+    def lmax(self, shard):
+        return int(shard[0]["event_length"].max()) if len(shard[0]) else 0
+
+    def run(self, shard, lmax: int, record_base: int, pool_base: int):
+        from types import SimpleNamespace
+
+        return SimpleNamespace(records=shard[0], pool=shard[1], n=len(shard[0]), lmax=lmax, pool_base=pool_base, row_base=record_base)
+
+
+class DeviceRecords:
+    """Backend for the records of a rank on its GPU: libwfb200's scan, build (with seq), split points and merge."""
+
+    def sync(self):
+        import torch
+
+        torch.cuda.synchronize()
+
+    def scan(self, blob):
+        from . import ops
+
+        return ops.v1725_scan(blob)
+
+    def upload(self, scans, names):
+        from . import ops
+
+        return ops.v1725_upload(scans, names)
+
+    def build(self, up, dt_ns: int, seq: np.ndarray):
+        from . import ops
+
+        rows, pool, _ = ops.build_records_v1725_device(up, dt_ns, seq=seq)
+        return rows, pool, up["n"]
+
+    def count(self, local):
+        return local[2]
+
+    def n_samples(self, local):
+        return int(local[1].numel())
+
+    def rows_at(self, local, idx):
+        import torch
+
+        from .dtypes import RECORDS_DTYPE
+
+        rows, _, n = local
+        i = torch.as_tensor(np.asarray(idx, dtype=np.int64), device=rows.device)
+        return rows[: n * 102].view(n, 102).index_select(0, i).cpu().numpy().reshape(-1).view(RECORDS_DTYPE)
+
+    def split_points(self, local, splitters):
+        from . import ops
+
+        return ops.record_split_points(local[0], local[2], splitters)
+
+    def send_buffers(self, local):
+        import torch
+
+        rows, pool, n = local
+        return rows[: n * 102], pool.view(torch.uint8)
+
+    def empty_bytes(self, nbytes: int):
+        import torch
+
+        return torch.empty(int(nbytes), dtype=torch.uint8, device="cuda")
+
+    def merge(self, rows, pool, run_offsets, record_base: int, pool_base: int):
+        import torch
+
+        from . import ops
+
+        rows_o, pool_o, meta = ops.merge_record_runs(rows, pool.view(torch.int16), run_offsets, record_base=record_base, pool_base=pool_base)
+        return rows_o, pool_o, meta, int(run_offsets[-1])
+
+    def lmax(self, shard):
+        import ctypes as C
+
+        import torch
+
+        from . import _lib
+        from .engine import _ptr, _stream
+
+        stats = np.zeros(3, dtype=np.int32)
+        scratch = torch.empty(4, dtype=torch.int32, device="cuda")
+        _lib.check(_lib.load().wfb_meta_stats(_ptr(shard[2]), shard[3], _ptr(scratch), C.c_void_p(stats.ctypes.data), _stream()),
+                   "wfb_meta_stats")
+        return max(int(stats[0]), 0)
+
+    def run(self, shard, lmax: int, record_base: int, pool_base: int):
+        from .engine import DeviceRun
+
+        rows, pool, meta, n = shard
+        return DeviceRun(meta, pool, n, 0, lmax, records_rows=rows, pool_base=pool_base, row_base=record_base)
+
+
+def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None) -> dict:
+    """This rank's time shard of the V1725 run made of ``paths`` (the full ordered file list, the same on every rank;
+    file names give the board id), without any process holding the whole run.
+
+    ``mine``: the indices of the files this rank reads (node-local disks); by default every rank reads a contiguous
+    block of the list balanced by file size, which needs every file's size on every rank.  A file claimed by no rank
+    or by two ranks raises ValueError on every rank; a file that cannot be read raises on every rank too.
+
+    Returns ``run`` (an ``engine.DeviceRun`` of rows [record_base, record_base + n) of the single-GPU build with its
+    pool slice, the run-wide longest record as ``lmax``: ``run.features_hits`` gives global event indices and
+    ``merge_group_sharded`` takes its hits unchanged), ``record_base``, ``n_total``, ``records_per_rank``,
+    ``exchange_bytes`` (row and sample bytes this rank received from the other ranks) and ``timings`` (seconds per
+    stage, each ended by a device synchronize)."""
+    import time
+
+    backend = backend if backend is not None else DeviceRecords()
+    dist, rank, P = _dist()
+    paths = [str(p) for p in paths]
+    F = len(paths)
+    T: dict = {}
+    err = None
+
+    if mine is None:
+        sizes = []
+        for p in paths:
+            try:
+                sizes.append(os.path.getsize(p))
+            except OSError as e:
+                err = err or e
+                sizes.append(0)
+        mine = np.flatnonzero(default_file_owners(sizes, P) == rank)
+    mine = np.asarray(mine, dtype=np.int64).reshape(-1)
+
+    # ownership, checked on the gathered claims so that every rank raises
+    claims = allgather_columns({"file": mine})["file"]
+    claimed = np.bincount(claims[(claims >= 0) & (claims < F)], minlength=F)
+    if len(claims) != int(claimed.sum()) or np.any(claimed != 1):
+        bad = sorted(set(np.flatnonzero(claimed != 1).tolist()) | set(claims[(claims < 0) | (claims >= F)].tolist()))
+        raise ValueError(f"every file must be read by exactly one rank: files {bad[:10]} are claimed by none, by several ranks or do not exist")
+
+    # read + scan the own files in list order (a rank's files are a subsequence of the list: local order = global order)
+    own = sorted(set(mine.tolist()))
+    t = time.perf_counter()
+    blobs, scans = [], []
+    try:
+        if err is None:
+            for f in own:
+                blobs.append(np.fromfile(paths[f], dtype=np.uint8))
+            T["read"] = time.perf_counter() - t
+            t = time.perf_counter()
+            scans = [backend.scan(b) for b in blobs]
+            T["scan"] = time.perf_counter() - t
+    except (OSError, ValueError) as e:
+        err = e
+    status = np.zeros(F + 1, dtype=np.int64)
+    status[0] = int(err is not None)
+    for f, s in zip(own, scans):
+        status[1 + f] = len(s["channel"])
+    table = _allgather_i64(status)
+    if table[:, 0].any():
+        if err is not None:
+            raise err
+        raise RuntimeError(f"ranks {np.flatnonzero(table[:, 0]).tolist()} could not read their V1725 files")
+    counts = table[:, 1:].sum(axis=0)
+    seq_base = np.cumsum(counts) - counts
+    seq = np.concatenate([seq_base[f] + np.arange(counts[f], dtype=np.int64) for f in own] or [np.zeros(0, np.int64)])
+
+    # 1. local build
+    t = time.perf_counter()
+    up = backend.upload(scans, [paths[f] for f in own])
+    del blobs, scans
+    backend.sync()
+    T["h2d"] = time.perf_counter() - t
+    t = time.perf_counter()
+    local = backend.build(up, int(dt_ns), seq)
+    del up  # the stream bytes
+    backend.sync()
+    T["build"] = time.perf_counter() - t
+
+    # 2. splitters, 3. split points
+    t = time.perf_counter()
+    n_local = backend.count(local)
+    pos, w = splitter_samples(n_local, SPLITTER_SAMPLES_PER_RANK * P)
+    k = record_keys(backend.rows_at(local, pos))
+    g = allgather_columns({"ts": k[:, 0], "board": k[:, 1], "channel": k[:, 2], "seq": k[:, 3], "w": w})
+    splitters = plan_splitters(np.stack([g["ts"], g["board"], g["channel"], g["seq"]], axis=1), g["w"], P)
+    cuts = np.r_[0, np.asarray(backend.split_points(local, splitters), dtype=np.int64), n_local]
+    inner = cuts[:-1][cuts[:-1] < n_local]
+    offs = np.r_[backend.rows_at(local, inner)["wave_offset"].astype(np.int64), np.full(P + 1 - len(inner), backend.n_samples(local))]
+    row_counts, sample_counts = np.diff(cuts), np.diff(offs)
+    T["splitters"] = time.perf_counter() - t
+
+    # 4. exchange
+    t = time.perf_counter()
+    send_rows, send_pool = backend.send_buffers(local)
+    rows, pool, recv = _exchange(send_rows, send_pool, row_counts, sample_counts, backend)
+    del local, send_rows, send_pool
+    backend.sync()
+    T["exchange"] = time.perf_counter() - t
+    others = np.arange(P) != rank
+    exchange_bytes = int((recv[others, 0] * 102 + recv[others, 1] * 2).sum())
+
+    # 5. global bases, 6. merge
+    n_recv, s_recv = int(recv[:, 0].sum()), int(recv[:, 1].sum())
+    bases = _allgather_i64([n_recv, s_recv])
+    record_base, pool_base = int(bases[:rank, 0].sum()), int(bases[:rank, 1].sum())
+    t = time.perf_counter()
+    shard = backend.merge(rows, pool, np.r_[0, np.cumsum(recv[:, 0])], record_base, pool_base)
+    del rows, pool
+    backend.sync()
+    T["merge"] = time.perf_counter() - t
+    lmax = _allreduce_max(backend.lmax(shard))
+    return dict(run=backend.run(shard, lmax, record_base, pool_base), record_base=record_base, pool_base=pool_base,
+                n_total=int(bases[:, 0].sum()), records_per_rank=bases[:, 0].copy(), exchange_bytes=exchange_bytes, timings=T)

@@ -533,14 +533,19 @@ def build_records_from_v1725(blobs, names, dt_ns: int):
     """V1725 .bin streams (bytes / uint8 arrays, one per file, with their file names for the board id)
     -> (records[RECORDS_DTYPE], wave_pool[uint16]) in the reference's order
     (records_builder.py:798-830 build_records_from_v1725_files)."""
+    up = v1725_upload([v1725_scan(b) for b in blobs], names)
+    if up["n"] == 0:
+        return np.zeros(0, dtype=RECORDS_DTYPE), np.zeros(0, dtype=np.uint16)
+    rows, pool, _ = build_records_v1725_device(up, dt_ns)
+    rec = rows[: up["n"] * 102].cpu().numpy().view(RECORDS_DTYPE)
+    return rec, pool.cpu().numpy().view(np.uint16)
+
+
+def v1725_upload(scans, names) -> dict:
+    """The streams of ``scans`` (v1725_scan of each file, in list order) at 16-byte aligned bases of ONE device buffer
+    and their index columns on the device (payload offsets rebased, board ids from ``names``)."""
     lib = _lib.load()
     torch = _torch()
-    scans = [v1725_scan(b) for b in blobs]
-    n = sum(len(s["channel"]) for s in scans)
-    total = sum(s["n_samples_total"] for s in scans)
-    if n == 0:
-        return np.zeros(0, dtype=RECORDS_DTYPE), np.zeros(0, dtype=np.uint16)
-    # one device buffer with every stream at a 16-byte aligned base, payload offsets rebased
     bases, cursor = [], 0
     for s in scans:
         bases.append(cursor)
@@ -548,20 +553,69 @@ def build_records_from_v1725(blobs, names, dt_ns: int):
     d_blob = torch.empty(cursor + 16, dtype=torch.uint8, device="cuda")
     for s, base in zip(scans, bases):
         if len(s["bytes"]):
-            d_blob[base:base + len(s["bytes"])].copy_(torch.from_numpy(s["bytes"].copy()))
-    off = np.concatenate([s["payload_offset"] + base for s, base in zip(scans, bases)])
-    board = np.concatenate([np.full(len(s["channel"]), v1725_board_from_name(nm), dtype=np.int16) for s, nm in zip(scans, names)])
-    cat = {k: np.concatenate([s[k] for s in scans]) for k in ("n_samples", "channel", "timestamp", "baseline", "trunc")}
+            _lib.check(lib.wfb_memcpy_h2d(C.c_void_p(d_blob.data_ptr() + base), _hp(s["bytes"]), len(s["bytes"]), _stream()), "wfb_memcpy_h2d")
+    off = np.concatenate([s["payload_offset"] + base for s, base in zip(scans, bases)] or [np.zeros(0, np.int64)])
+    board = np.concatenate([np.full(len(s["channel"]), v1725_board_from_name(nm), dtype=np.int16) for s, nm in zip(scans, names)]
+                           or [np.zeros(0, np.int16)])
+    up = {k: _dev(np.concatenate([s[k] for s in scans])) for k in ("n_samples", "channel", "timestamp", "baseline", "trunc")} if scans else {}
+    up.update(blob=d_blob, blob_bytes=cursor, payload_offset=_dev(off), board=_dev(board), n=len(off),
+              total=sum(s["n_samples_total"] for s in scans))
+    return up
+
+
+def build_records_v1725_device(up: dict, dt_ns: int, *, seq: np.ndarray | None = None, meta: bool = False):
+    """wfb_build_records_v1725 (``seq`` given: wfb_build_records_v1725_seq, record_id = seq) on the output of
+    v1725_upload -> device (rows uint8 [n * 102], pool int16 [total] with a 16-sample tail, meta uint8 [n * 48] or None)."""
+    lib = _lib.load()
+    torch = _torch()
+    n, total = up["n"], up["total"]
     rows = _empty(n * 102)
     pool = torch.empty(total + 16, dtype=torch.int16, device="cuda")[:total]
+    d_meta = torch.empty(max(n, 1) * 48, dtype=torch.uint8, device="cuda") if meta else None
+    if n == 0:
+        return rows, pool, d_meta
     ws = _empty(lib.wfb_build_records_v1725_workspace_bytes(n))
-    d = {k: _dev(v) for k, v in cat.items()}
-    d_off, d_board = _dev(off), _dev(board)
-    _lib.check(lib.wfb_build_records_v1725(_ptr(d_blob), cursor, _ptr(d_off), _ptr(d["n_samples"]), _ptr(d["timestamp"]), _ptr(d_board),
-                                           _ptr(d["channel"]), _ptr(d["baseline"]), _ptr(d["trunc"]), n, int(dt_ns), _ptr(rows), _ptr(pool),
-                                           total, C.c_void_p(0), _ptr(ws), ws.numel(), _stream()), "wfb_build_records_v1725")
-    rec = rows[: n * 102].cpu().numpy().view(RECORDS_DTYPE)
-    return rec, pool.cpu().numpy().view(np.uint16)
+    cols = (_ptr(up["blob"]), up["blob_bytes"], _ptr(up["payload_offset"]), _ptr(up["n_samples"]), _ptr(up["timestamp"]), _ptr(up["board"]),
+            _ptr(up["channel"]), _ptr(up["baseline"]), _ptr(up["trunc"]))
+    tail = (n, int(dt_ns), _ptr(rows), _ptr(pool), total, _ptr(d_meta), _ptr(ws), ws.numel(), _stream())
+    if seq is None:
+        _lib.check(lib.wfb_build_records_v1725(*cols, *tail), "wfb_build_records_v1725")
+    else:
+        d_seq = _dev(np.ascontiguousarray(seq, dtype=np.int64))
+        if len(d_seq) != n:
+            raise ValueError(f"seq has {len(d_seq)} entries for {n} waveforms")
+        _lib.check(lib.wfb_build_records_v1725_seq(*cols, _ptr(d_seq), *tail), "wfb_build_records_v1725_seq")
+    return rows, pool, d_meta
+
+
+def record_split_points(rows, n: int, keys: np.ndarray) -> np.ndarray:
+    """wfb_record_split_points: lower bound of every key (int64 rows of timestamp, board, channel, record_id) among
+    the first ``n`` sorted RECORDS rows of the device tensor ``rows``."""
+    lib = _lib.load()
+    k = np.ascontiguousarray(keys, dtype=np.int64).reshape(-1, 4)
+    if len(k) == 0:
+        return np.zeros(0, dtype=np.int64)
+    d_k = _dev(k.reshape(-1))
+    out = _torch().empty(len(k), dtype=_torch().int64, device="cuda")
+    _lib.check(lib.wfb_record_split_points(_ptr(rows), int(n), _ptr(d_k), len(k), _ptr(out), _stream()), "wfb_record_split_points")
+    return out.cpu().numpy()
+
+
+def merge_record_runs(rows, pool, run_offsets, *, record_base: int, pool_base: int):
+    """wfb_merge_record_runs: merge the sorted runs rows[run_offsets[r]:run_offsets[r + 1]] (device RECORDS rows, their
+    samples concatenated in the same order in ``pool``) -> device (rows, pool with a 16-sample tail, meta), numbered
+    from ``record_base`` / ``pool_base``."""
+    lib = _lib.load()
+    torch = _torch()
+    ro = np.ascontiguousarray(run_offsets, dtype=np.int64)
+    n, total = int(ro[-1]), int(pool.numel())
+    out_rows = _empty(n * 102)
+    out_pool = torch.empty(total + 16, dtype=torch.int16, device="cuda")[:total]
+    meta = torch.empty(max(n, 1) * 48, dtype=torch.uint8, device="cuda")
+    ws = _empty(lib.wfb_merge_record_runs_workspace_bytes(n, len(ro) - 1))
+    _lib.check(lib.wfb_merge_record_runs(_ptr(rows), _ptr(pool), n, _hp(ro), len(ro) - 1, int(record_base), int(pool_base), _ptr(out_rows),
+                                         _ptr(out_pool), total, _ptr(meta), _ptr(ws), ws.numel(), _stream()), "wfb_merge_record_runs")
+    return out_rows, out_pool, meta
 
 
 # --------------------------------------------------------------------------------------------
