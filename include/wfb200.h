@@ -340,6 +340,22 @@ int wfb_group_time_window(const int64_t* ts_sorted_dev, int64_t n, double time_w
                           int64_t* event_id_dev, int64_t* n_events_dev, void* workspace_dev,
                           size_t workspace_bytes, void* stream);
 
+/* The event table of wfb_group_time_window's events (event_grouping.py:99-283, the df_events columns).
+ * ts_sorted_dev int64[n] ascending and event_id_dev int64[n] as wfb_group_time_window wrote them (events are
+ * contiguous runs numbered 0 .. n_events - 1); channel_dev int16, area_dev / height_dev float32 (both optional) are
+ * indexed by INPUT row; order_dev int64[n] maps sorted position -> input row (NULL: the rows are already sorted).
+ * Writes offsets_dev[n_events + 1] (CSR), members_dev[n] (input rows, stably ordered by channel inside every event:
+ * np.lexsort((arange, channel, event))), t_min / t_max (timestamps of the first / last member in that order),
+ * dt_ns = (double)(t_max - t_min) / 1e3, n_hits, and the member-ordered timestamp / channel / area / height columns
+ * (member_area_dev / member_height_dev NULL exactly when their inputs are).  Events of up to 32 members are ranked by
+ * one warp each; larger ones by one stable radix sort of their rows.  Synchronises the stream once. */
+size_t wfb_event_table_workspace_bytes(int64_t n);
+int wfb_event_table(const int64_t* ts_sorted_dev, const int64_t* event_id_dev, int64_t n, int64_t n_events,
+                    const int16_t* channel_dev, const int64_t* order_dev, const float* area_dev, const float* height_dev,
+                    int64_t* offsets_dev, int64_t* members_dev, int64_t* t_min_dev, int64_t* t_max_dev, double* dt_ns_dev,
+                    int64_t* n_hits_dev, int64_t* member_ts_dev, int16_t* member_channel_dev, float* member_area_dev,
+                    float* member_height_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+
 /* K1 for records of different lengths (channels / parts with different waveform widths,
  * records_builder.py:212-302 per part + :870-945 merge): like wfb_build_records, but every record names its
  * own int16 samples (byte offset into samples_dev + count) and the wave_pool is ragged (wave_offset = running

@@ -18,7 +18,13 @@ rank's records), builds its time shard with ``distributed.build_records_sharded_
 merge_group_sharded path.  It reports the time of every ingest stage, the exchange bytes and rate, the merge kernel's
 rate against its algorithmic bytes (4 L + 252 per record), the peak device memory, and the GPU name and power limit;
 with --verify 1 rank 0 rebuilds all files on one GPU and checks records, pool, features, hits, merged rows and event
-ids byte for byte."""
+ids byte for byte.
+
+--events adds the df -> df_events -> df_paired leg on the same shards: ``distributed.df_sharded`` on the rank's feature
+rows, then ``distributed.events_sharded`` (time_window_ns = pair window = 100, 2 paired channels).  It reports the time of
+every stage (each ended by a device synchronize), gathered_bytes, the event counts and the peak device memory of the leg;
+with --verify 1 rank 0 runs the single-GPU chain (df columns, wfb_group_time_window, wfb_event_table, wfb_pair_events
+on the whole run) and checks the gathered df columns, event table, members and df_paired columns byte for byte."""
 import argparse
 import os
 import sys
@@ -40,6 +46,7 @@ ap.add_argument("--zone-rows", type=int, default=4096)
 ap.add_argument("--source", choices=("synth", "v1725"), default="synth")
 ap.add_argument("--files-per-rank", type=int, default=2)
 ap.add_argument("--samples", type=int, default=800)
+ap.add_argument("--events", action="store_true", help="also run the sharded df -> df_events -> df_paired leg")
 args = ap.parse_args()
 
 D.init_process_group("nccl")
@@ -162,6 +169,75 @@ assert int(tot[0]) == int(tot[1]), "hits were lost or duplicated by the ownershi
 msg = (f"world={ws} records/rank={n} hits={int(tot[0])} clusters={int(tot[2])} events={int(tot[3])} zone_rows={sh['zone_rows']} "
        f"gathered_bytes/rank={sh['gathered_bytes']} merge+group wall={1e3 * (t1 - t0):.1f} ms")
 
+EV_COLS = ("t_min", "t_max", "dt_ns", "n_hits", "members", "member_ts", "member_channel", "member_area", "member_height", "keep",
+           "delta_t", "area_ch", "height_ch")
+
+
+def events_leg() -> str:
+    """df_sharded + events_sharded on this rank's shard; with --verify the single-GPU chain on rank 0."""
+    import subprocess
+
+    torch.cuda.synchronize()
+    torch.cuda.reset_peak_memory_stats()
+    base_mem = torch.cuda.memory_allocated()
+    if ws > 1:
+        dist.barrier()
+    t = time.perf_counter()
+    df = D.df_sharded(run, res["features"])
+    torch.cuda.synchronize()
+    t_df = time.perf_counter() - t
+    t = time.perf_counter()
+    ev = D.events_sharded(df, time_window_ns=WINDOW, pair_window_ns=WINDOW, n_channels=2, start_channel_slice=6, zone_rows=args.zone_rows)
+    torch.cuda.synchronize()
+    t_ev = time.perf_counter() - t
+    peak = torch.cuda.max_memory_allocated() - base_mem
+    gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", str(local)],
+                         capture_output=True, text=True).stdout.strip()
+    line = (f"rank {rank}: df rows {df['n']} owned {ev['owned'][1] - ev['owned'][0]} events {ev['n_events']} (base {ev['event_base']}) | "
+            f"df_sharded {1e3 * t_df:.1f} ms | events_sharded {1e3 * t_ev:.1f} ms: " +
+            " ".join(f"{k} {1e3 * v:.1f} ms" for k, v in ev["timings"].items()) +
+            f" | gathered {ev['gathered_bytes']} B, zone_rows {ev['zone_rows']} | peak device memory of the leg {peak / 1e9:.3f} GB | {gpu}")
+    lines = D.gather_rows(np.frombuffer(line.encode().ljust(1024)[:1024], dtype="S1024")) if ws > 1 else [line.encode()]
+    if rank == 0:
+        print(f"events leg: world={ws} records/rank={n}")
+        for ln in lines:
+            print("  " + ln.decode().strip())
+    out = f"events={int(ev['events_per_rank'].sum())} gathered_bytes/rank={ev['gathered_bytes']}"
+    if not args.verify:
+        return out
+    host = lambda x: x.cpu().numpy()  # noqa: E731
+    got_df = {k: D.gather_rows(host(df["cols"][k])) for k in ("timestamp", "record_id", "area", "height", "channel")}
+    got_df["index"] = D.gather_rows(host(df["index"]))
+    got = {}
+    for k in EV_COLS:
+        a = np.ascontiguousarray(host(ev[k]))
+        rows = a.view(np.dtype((np.void, a.dtype.itemsize * a.shape[1]))).reshape(-1) if a.ndim > 1 else a  # one row per event
+        got[k] = D.gather_rows(rows)
+    feats = D.gather_rows(res["features"][: n * 36].cpu().numpy().view([("b", "u1", (36,))]))
+    return out + (verify_events(got_df, got, feats) if rank == 0 else "")
+
+
+def verify_events(got_df, got, feats) -> str:
+    from waveformanalysis_b200.engine import upload
+
+    n_all = len(feats)
+    rid = np.sort(got_df["record_id"])  # the whole run's record ids in row order (shards are contiguous record ranges)
+    want = ops.df_columns_device(upload(feats.view(np.uint8).reshape(-1)), n_all, upload(rid))
+    for k in ("timestamp", "record_id", "area", "height", "channel"):
+        assert want[k].cpu().numpy().tobytes() == got_df[k].tobytes(), f"df.{k} differs"
+    assert np.array_equal(want["order"].cpu().numpy(), got_df["index"]), "df index differs"
+    ts = want["timestamp"]
+    e, n_ev = ops.group_time_window_device(ts, n_all, WINDOW)
+    t = ops.event_table_device(ts, e, n_all, n_ev, want["channel"], area=want["area"], height=want["height"])
+    t.update(ops.pair_events_device(t["offsets"], n_ev, t["member_ts"], t["member_area"], t["member_height"], t["dt_ns"], WINDOW, 2))
+    for k in EV_COLS:
+        w = np.ascontiguousarray(t[k].cpu().numpy())
+        assert w.tobytes() == np.ascontiguousarray(got[k]).tobytes(), f"events.{k} differs"
+    return f" | df, df_events and df_paired columns byte-identical to the single-GPU chain ({n_all} rows, {n_ev} events)"
+
+
+if args.events:
+    msg += " | " + events_leg()
 if args.verify:
     feats_l = res["features"][: n * 36].cpu().numpy()
     hits_l = res["hits"][: total * 60].cpu().numpy().view(THRESHOLD_HIT_DTYPE)

@@ -848,3 +848,354 @@ def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None) -
     lmax = _allreduce_max(backend.lmax(shard))
     return dict(run=backend.run(shard, lmax, record_base, pool_base), record_base=record_base, pool_base=pool_base,
                 n_total=int(bases[:, 0].sum()), records_per_rank=bases[:, 0].copy(), exchange_bytes=exchange_bytes, timings=T)
+
+
+# ------------------------------------------------------------------------------------------------
+# Time-sharded df -> df_events -> df_paired: anchored windows cut at segment starts
+# ------------------------------------------------------------------------------------------------
+# The `df` rows of a rank are its time shard sorted by timestamp; concatenated in rank order they are the single-run
+# `df` when the shards are in time order (df_sharded checks that on gathered first / last timestamps).
+#
+# df_events groups the time-sorted rows into anchored windows (event_grouping.py:477-510).  A SEGMENT starts wherever
+# (double)ts[i] > (double)ts[i - 1] + W (k4_segment_flags_kernel): every segment start is an anchor whatever came
+# before it, and the anchors inside a segment depend on that segment alone.  So a cut at a segment start splits the
+# run into parts that group independently, and two counts per rank number the events globally.
+#
+# What travels: the first and the last K df rows of every rank (timestamp, area, height, channel: 24 B per row,
+# K = 4096 by default) in ONE all_gather, plus one all_gather of 8 bytes per rank.  The zones of two neighbouring
+# non-empty ranks are consecutive in the global order, so every rank finds the same segment starts in
+# tail[r] ++ head[next] and picks the one nearest to the nominal boundary.  Without one the zones are doubled; when
+# both zones already hold their whole shards the boundary is dropped: the rank after it owns nothing and its rows
+# (all of them in the gathered zones) go to the owner before it.  A run without gaps is therefore legal: one segment
+# spanning all ranks ends up with one owner.
+
+EVENT_ZONE_DTYPE = np.dtype({"names": ["timestamp", "area", "height", "channel"], "formats": ["<i8", "<f4", "<f4", "<i2"],
+                             "offsets": [0, 8, 12, 16], "itemsize": 24})
+
+
+def check_time_order(table: np.ndarray) -> None:
+    """``table``: one row (rows, first timestamp, last timestamp) per rank.  Raises ValueError when a non-empty
+    rank ends after the next non-empty rank starts (the same on every rank: the table is gathered)."""
+    t = np.asarray(table, dtype=np.int64).reshape(-1, 3)
+    live = np.flatnonzero(t[:, 0] > 0)
+    for a, b in zip(live[:-1], live[1:]):
+        if t[a, 2] > t[b, 1]:
+            raise ValueError(f"the df shards are not in time order: rank {a} ends at timestamp {t[a, 2]}, after rank {b} starts "
+                             f"at {t[b, 1]}; concatenated in rank order they would not be the run's df")
+
+
+def segment_starts(ts: np.ndarray, w_ps: float) -> np.ndarray:
+    """Positions i >= 1 of consecutive time-sorted rows where a segment starts: the kernel's float64 test
+    (double)ts[i] > (double)ts[i - 1] + W."""
+    t = np.asarray(ts, dtype=np.int64).astype(np.float64)
+    return np.flatnonzero(t[1:] > t[:-1] + float(w_ps)) + 1
+
+
+def plan_event_cuts(heads: list, tails: list, wholes: list, counts, w_ps: float):
+    """The global df rows every rank owns for df_events.  heads[r] / tails[r]: the first / last zone rows of rank r
+    (EVENT_ZONE_DTYPE, disjoint), wholes[r]: the two zones are the whole shard, counts[r]: its rows, w_ps: the window
+    in ps.  Returns (bounds, ok): bounds[r] = [lo, hi) of global rows owned by rank r (lo == hi: nothing); ok is False
+    when a boundary has no segment start inside zones that do not cover both shards yet (the caller doubles them)."""
+    counts = np.asarray(counts, dtype=np.int64)
+    R = len(counts)
+    base = np.r_[0, np.cumsum(counts)]
+    live = [r for r in range(R) if counts[r] > 0]
+    cuts: list = []  # cut between live[i] and live[i + 1]: a global row, or None (boundary dropped)
+    for a, b in zip(live[:-1], live[1:]):
+        za = np.concatenate([heads[a], tails[a]]) if wholes[a] else tails[a]
+        zb = np.concatenate([heads[b], tails[b]]) if wholes[b] else heads[b]
+        s = segment_starts(np.concatenate([za["timestamp"], zb["timestamp"]]), w_ps)
+        if len(s) == 0:
+            if wholes[a] and wholes[b]:
+                cuts.append(None)
+                continue
+            return None, False
+        g = int(base[a + 1]) - len(za) + s  # global rows of the candidates
+        cuts.append(int(g[np.argmin(np.abs(g - base[b]))]))
+    bounds = np.stack([base[:-1], base[:-1]], axis=1)
+    for i, r in enumerate(live):
+        lo = 0 if i == 0 else cuts[i - 1]
+        if lo is None:
+            continue
+        hi = next((c for c in cuts[i:] if c is not None), int(base[-1]))
+        bounds[r] = (lo, hi)
+    return bounds, True
+
+
+def _zone_rows_in(heads, tails, counts, ranks, lo: int, hi: int) -> np.ndarray:
+    """The zone rows of ``ranks`` (ascending) at global rows [lo, hi), in global order; every such row must be in the
+    zones (the cut plan guarantees it)."""
+    base = np.r_[0, np.cumsum(np.asarray(counts, dtype=np.int64))]
+    parts = []
+    for q in ranks:
+        b, n = int(base[q]), int(counts[q])
+        hq, tq = heads[q], tails[q]
+        pos = np.r_[b + np.arange(len(hq)), b + n - len(tq) + np.arange(len(tq))]
+        sel = (pos >= lo) & (pos < hi)
+        want = max(min(hi, b + n) - max(lo, b), 0)
+        if int(sel.sum()) != want:
+            raise RuntimeError(f"events_sharded: rank {q} has owned rows outside its gathered zones")
+        parts.append(np.concatenate([hq, tq])[sel])
+    return np.concatenate(parts) if parts else np.zeros(0, dtype=EVENT_ZONE_DTYPE)
+
+
+def _pack_zone(ts, area, height, channel) -> np.ndarray:
+    z = np.zeros(len(ts), dtype=EVENT_ZONE_DTYPE)
+    z["timestamp"], z["area"], z["height"], z["channel"] = ts, area, height, channel
+    return z
+
+
+class HostEvents:
+    """Backend for df columns held as numpy arrays (CPU tests: the compute is the oracle's ``df_columns``,
+    ``group_time_window`` and ``pair_events``).  ``run`` is the shard's RECORDS rows, ``features`` its
+    BASIC_FEATURES rows."""
+
+    def __init__(self, df_fn, group_fn, pair_fn):
+        self.df_fn, self.group_fn, self.pair_fn = df_fn, group_fn, pair_fn
+
+    def df_local(self, run, features, gains):
+        cols = dict(self.df_fn(features, record_id=np.asarray(run["record_id"], dtype=np.int64), gains=gains))
+        return cols, np.asarray(cols.pop("order"), dtype=np.int64), len(features)
+
+    def ts_ends(self, cols, n):
+        return (int(cols["timestamp"][0]), int(cols["timestamp"][n - 1])) if n else (0, 0)
+
+    def zone(self, cols, a, b):
+        return _pack_zone(cols["timestamp"][a:b], cols["area"][a:b], cols["height"][a:b], cols["channel"][a:b])
+
+    def assemble(self, cols, l0, l1, first, last):
+        return {k: np.concatenate([first[k], np.asarray(cols[k][l0:l1]), last[k]]) for k in EVENT_ZONE_DTYPE.names}
+
+    def iota(self, n, base):
+        return np.arange(n, dtype=np.int64) + base
+
+    def sync(self):
+        pass
+
+    def events(self, owned, time_window_ns, pair_window_ns, n_channels, timings=None):
+        ev = self.group_fn(owned["timestamp"], owned["channel"], time_window_ns)
+        m = np.asarray(ev["members"], dtype=np.int64)
+        res = dict(t_min=ev["t_min"], t_max=ev["t_max"], dt_ns=ev["dt_ns"], n_hits=np.asarray(ev["n_hits"], dtype=np.int64),
+                   offsets=np.asarray(ev["offsets"], dtype=np.int64), members=m, member_ts=owned["timestamp"][m],
+                   member_channel=owned["channel"][m], member_area=owned["area"][m], member_height=owned["height"][m])
+        p = self.pair_fn(res["offsets"], res["member_ts"], res["member_area"], res["member_height"], res["dt_ns"], pair_window_ns, n_channels)
+        res.update(keep=np.asarray(p["keep"], dtype=bool), delta_t=p["delta_t"], area_ch=p["area_ch"], height_ch=p["height_ch"],
+                   n_events=len(res["t_min"]))
+        return res
+
+
+class DeviceEvents:
+    """Backend for df columns that stay on the device: ``run`` is a ``DeviceRun``, ``features`` its BASIC_FEATURES rows
+    from ``DeviceRun.features_hits`` (uint8 tensor, 36 B per row); record_id is the rows' ``wfb_rec_meta.record_id``."""
+
+    def df_local(self, run, features, gains):
+        import torch
+
+        from . import ops
+
+        n = run.n
+        rid = run.meta[: n * 48].view(n, 48)[:, 40:48].contiguous().view(-1).view(torch.int64) if n else None  # wfb_rec_meta.record_id
+        cols = ops.df_columns_device(features[: n * 36] if n else None, n, rid, gains)
+        return cols, cols.pop("order"), n
+
+    def ts_ends(self, cols, n):
+        if not n:
+            return 0, 0
+        t = cols["timestamp"][[0, n - 1]].cpu().numpy()
+        return int(t[0]), int(t[1])
+
+    def zone(self, cols, a, b):
+        return _pack_zone(*(cols[k][a:b].cpu().numpy() for k in ("timestamp", "area", "height", "channel")))
+
+    def assemble(self, cols, l0, l1, first, last):
+        import torch
+
+        from .engine import upload
+
+        out = {}
+        for k in EVENT_ZONE_DTYPE.names:
+            parts = [upload(np.ascontiguousarray(z[k])) for z in (first,) if len(z)]
+            parts.append(cols[k][l0:max(l0, l1)])
+            parts += [upload(np.ascontiguousarray(z[k])) for z in (last,) if len(z)]
+            out[k] = torch.cat(parts) if len(parts) > 1 else parts[0]
+        return out
+
+    def iota(self, n, base):
+        import torch
+
+        return torch.arange(n, dtype=torch.int64, device="cuda") + base
+
+    def sync(self):
+        import torch
+
+        torch.cuda.synchronize()
+
+    def events(self, owned, time_window_ns, pair_window_ns, n_channels, timings=None):
+        import time
+
+        from . import ops
+
+        T = timings if timings is not None else {}
+        ts = owned["timestamp"]
+        n = int(ts.numel())
+        t = time.perf_counter()
+        ev, n_ev = ops.group_time_window_device(ts, n, time_window_ns)
+        self.sync()
+        T["group"], t = time.perf_counter() - t, time.perf_counter()
+        res = ops.event_table_device(ts, ev, n, n_ev, owned["channel"], area=owned["area"], height=owned["height"])
+        self.sync()
+        T["event_table"], t = time.perf_counter() - t, time.perf_counter()
+        res.update(ops.pair_events_device(res["offsets"], n_ev, res["member_ts"], res["member_area"], res["member_height"], res["dt_ns"],
+                                          pair_window_ns, n_channels))
+        self.sync()
+        T["pair"] = time.perf_counter() - t
+        res["n_events"] = n_ev
+        return res
+
+
+def df_sharded(run, features, *, gains: dict | None = None, backend=None) -> dict:
+    """This rank's part of the run's `df`: ``wfb_df_columns`` on the rank's feature rows, left where they are (device
+    tensors with ``DeviceEvents``, the default).  ``run`` / ``features``: the rank's time shard and its basic_features
+    rows (``DeviceRun`` + ``features_hits()["features"]``); record_id is the rows' record_id, global for the shards of
+    ``build_records_sharded_v1725`` and ``DeviceRun.synth(record_base=...)``.
+
+    The shards must be in time order: every rank gathers every non-empty rank's first and last timestamp and raises
+    ValueError (every rank alike) when one ends after the next one starts.  Returns ``cols`` (timestamp, record_id,
+    area, height, amp, max_abs_diff, board, channel [, area_pe, height_pe]; timestamp-sorted), ``index`` (row_base +
+    the local sort order: the DataFrame index), ``n``, ``row_base``, ``rows_per_rank`` and ``with_pe``."""
+    backend = backend if backend is not None else DeviceEvents()
+    _, rank, _ = _dist()
+    cols, order, n = backend.df_local(run, features, gains)
+    first, last = backend.ts_ends(cols, n)
+    table = _allgather_i64([n, first, last])
+    check_time_order(table)
+    me = rank if len(table) > 1 else 0
+    row_base = int(table[:me, 0].sum())
+    return dict(cols=cols, index=order + row_base, n=n, row_base=row_base, rows_per_rank=table[:, 0].copy(), with_pe=gains is not None)
+
+
+def events_sharded(df: dict, *, time_window_ns: float = 100.0, pair_window_ns: float = 100.0, n_channels: int = 2,
+                   start_channel_slice: int = 6, backend=None, zone_rows: int = 4096) -> dict:
+    """df_events + df_paired of a time-sharded `df` (``df_sharded``'s result) without gathering the rows.
+
+    Every rank exchanges its boundary zones (``zone_rows`` rows per end, doubled while a boundary has no segment
+    start in them), owns the global rows between its two cuts (assembled on its device: gathered zone rows, then the
+    untouched middle of its shard), groups them (``wfb_group_time_window``), builds the event table
+    (``wfb_event_table``) and pairs the events (``wfb_pair_events``, ``pair_window_ns``).  Returns the rank's events
+    with GLOBAL ids (``event_id``, ``t_min``, ``t_max``, ``dt_ns``, ``n_hits``), the CSR ``offsets`` with ``members``
+    (global df rows) and the member-ordered ``member_ts`` / ``member_channel`` / ``member_area`` / ``member_height``,
+    ``keep`` / ``delta_t`` / ``area_ch`` / ``height_ch``, ``event_base``, ``events_per_rank``, ``bounds`` (every rank's
+    owned [lo, hi)), ``zone_rows``, ``gathered_bytes`` (what this rank received in the collectives) and ``timings``
+    (seconds per stage, each ended by a device synchronize)."""
+    import time
+
+    backend = backend if backend is not None else DeviceEvents()
+    _, rank, _ = _dist()
+    cols, n = df["cols"], int(df["n"])
+    w_ps = float(time_window_ns) * 1e3
+    k = max(int(zone_rows), 1)
+    gathered = 0
+    T: dict = {}
+    t = time.perf_counter()
+    while True:
+        head, tail, whole = event_zones(backend, cols, n, k)
+        heads, tails, wholes, counts, nbytes = _allgather_zones(head, tail, k, whole, n)
+        gathered += nbytes
+        bounds, ok = plan_event_cuts(heads, tails, wholes, counts, w_ps)
+        if ok:
+            break
+        k *= 2
+    R = len(heads)
+    me = rank if R > 1 else 0
+    T["zones"] = time.perf_counter() - t
+    res = owned_events(backend, cols, me, heads, tails, counts, bounds, time_window_ns=time_window_ns, pair_window_ns=pair_window_ns,
+                       n_channels=n_channels, timings=T)
+    table = _allgather_i64([res["n_events"]])
+    gathered += table.nbytes if R > 1 else 0
+    res["event_base"] = int(table[:me, 0].sum())
+    res["event_id"] = backend.iota(res["n_events"], res["event_base"])
+    res.update(events_per_rank=table[:, 0].copy(), bounds=bounds, zone_rows=k, gathered_bytes=gathered, n_channels=int(n_channels),
+               start_channel_slice=int(start_channel_slice), pair_window_ns=float(pair_window_ns), timings=T)
+    return res
+
+
+def event_zones(backend, cols, n: int, k: int):
+    """The first and the last (at most) ``k`` df rows of a rank as EVENT_ZONE_DTYPE rows, disjoint, and whether they
+    are the whole shard."""
+    kh = min(k, n)
+    kt = min(k, n - kh)
+    return backend.zone(cols, 0, kh), backend.zone(cols, n - kt, n), kh + kt == n
+
+
+def owned_events(backend, cols, me: int, heads, tails, counts, bounds, *, time_window_ns: float, pair_window_ns: float,
+                 n_channels: int, timings: dict | None = None) -> dict:
+    """The local part of events_sharded on rank ``me``, given every rank's zones and the plan: assemble the owned rows
+    (lower ranks' zone rows, the rank's own rows between the cuts, upper ranks' zone rows), group them, build the event
+    table and pair the events.  ``members`` are global df rows; ``owned`` is the rank's [lo, hi)."""
+    R = len(counts)
+    lo, hi = (int(x) for x in bounds[me])
+    base, n = int(sum(counts[:me])), int(counts[me])
+    l0, l1 = min(max(lo - base, 0), n), min(max(hi - base, 0), n)
+    first = _zone_rows_in(heads, tails, counts, range(me), lo, hi)
+    last = _zone_rows_in(heads, tails, counts, range(me + 1, R), lo, hi)
+    import time
+
+    t = time.perf_counter()
+    owned = backend.assemble(cols, l0, l1, first, last)
+    backend.sync()
+    if timings is not None:
+        timings["assemble"] = time.perf_counter() - t
+    res = backend.events(owned, float(time_window_ns), float(pair_window_ns), int(n_channels), timings)
+    res["members"] = res["members"] + lo
+    res["owned"] = (lo, hi)
+    return res
+
+
+def _host(x) -> np.ndarray:
+    return x.cpu().numpy() if hasattr(x, "cpu") else np.asarray(x)
+
+
+def gather_event_frames(df_sh: dict, ev_sh: dict):
+    """(df, df_events, df_paired) of the WHOLE run on every rank, equal to what B200DataFramePlugin,
+    B200GroupedEventsPlugin and B200PairedEventsPlugin return for the run.  Every rank receives every row, member and
+    event, so this holds the whole run in each process (like ``gather_rows``): it is for checks and small runs, the
+    sharded results themselves stay distributed."""
+    import pandas as pd
+
+    from .plugins.dataframe import DF_COLUMNS, df_frame, pair_events_frame, paired_frame
+    from .plugins.grouping import DF_EVENTS_COLUMNS, events_frame
+
+    cols, with_pe = df_sh["cols"], bool(df_sh["with_pe"])
+    names = list(DF_COLUMNS) + (["area_pe", "height_pe"] if with_pe else [])
+    host = {k: _host(cols[k]) for k in names}
+    rows = np.zeros(int(df_sh["n"]), dtype=[("index", "<i8")] + [(k, host[k].dtype) for k in names])
+    rows["index"] = _host(df_sh["index"])
+    for k in names:
+        rows[k] = host[k]
+    rows = gather_rows(rows)
+    df = df_frame({k: rows[k] for k in names}, rows["index"], with_pe)
+
+    nc, start = ev_sh["n_channels"], ev_sh["start_channel_slice"]
+    n_ev = int(ev_sh["n_events"])
+    ev_rows = np.zeros(n_ev, dtype=[("event_id", "<i8"), ("t_min", "<i8"), ("t_max", "<i8"), ("dt_ns", "<f8"), ("n_hits", "<i8"),
+                                    ("keep", "u1"), ("delta_t", "<f8"), ("area_ch", "<f4", (nc,)), ("height_ch", "<f4", (nc,))])
+    for k in ev_rows.dtype.names:
+        ev_rows[k] = _host(ev_sh[k]).reshape(ev_rows[k].shape)
+    ev_rows = gather_rows(ev_rows)
+    m = len(_host(ev_sh["member_ts"]))
+    mem = np.zeros(m, dtype=[("ts", "<i8"), ("channel", "<i2"), ("area", "<f4"), ("height", "<f4")])
+    mem["ts"], mem["channel"] = _host(ev_sh["member_ts"]), _host(ev_sh["member_channel"])
+    mem["area"], mem["height"] = _host(ev_sh["member_area"]), _host(ev_sh["member_height"])
+    mem = gather_rows(mem)
+
+    if len(df) == 0:
+        df_events = pd.DataFrame(columns=DF_EVENTS_COLUMNS)
+        return df, df_events, pair_events_frame(df_events, nc, start, ev_sh["pair_window_ns"])
+    offsets = np.r_[0, np.cumsum(ev_rows["n_hits"])].astype(np.int64)
+    table = {k: np.ascontiguousarray(ev_rows[k]) for k in ("event_id", "t_min", "t_max", "dt_ns", "n_hits")}
+    table["offsets"] = offsets
+    df_events = events_frame(table, np.ascontiguousarray(mem["channel"]), np.ascontiguousarray(mem["area"]),
+                             np.ascontiguousarray(mem["height"]), np.ascontiguousarray(mem["ts"]))
+    out = dict(keep=ev_rows["keep"].astype(bool), delta_t=np.ascontiguousarray(ev_rows["delta_t"]),
+               area_ch=np.ascontiguousarray(ev_rows["area_ch"]).reshape(-1, nc), height_ch=np.ascontiguousarray(ev_rows["height_ch"]).reshape(-1, nc))
+    return df, df_events, paired_frame(df_events, offsets, out, nc, start)

@@ -395,34 +395,73 @@ def group_hit_windows(hits: np.ndarray, time_window_ns: float, component_rows=No
 
 
 def group_time_window(timestamps: np.ndarray, channels: np.ndarray, time_window_ns: float) -> dict:
-    """Anchored fixed-window clustering (event_grouping.py:99-283, 477-510): device time sort +
-    anchor search + event ids; member ordering by channel on the host."""
-    lib = _lib.load()
+    """Anchored fixed-window clustering (event_grouping.py:99-283, 477-510) on the device: stable time sort, anchor
+    search, event ids and the event table (members stably ordered by channel, t_min / t_max / dt/ns / n_hits).
+    ``channels`` must fit int16 (the project's channel dtype)."""
     torch = _torch()
     ts_in = np.asarray(timestamps, dtype=np.int64)
     n = len(ts_in)
     if n == 0:
         z = np.zeros(0, dtype=np.int64)
         return dict(event_id=z, t_min=z, t_max=z, dt_ns=np.zeros(0), n_hits=z, offsets=np.zeros(1, np.int64), members=z)
-    ts_sorted, order = sort_pairs(ts_in, np.arange(n, dtype=np.int64))
-    d_ts = _dev(ts_sorted)
-    ev = torch.empty(n, dtype=torch.int64, device="cuda")
+    ch_in = np.asarray(channels)
+    ch16 = ch_in.astype(np.int16)
+    if len(ch16) != n or not np.array_equal(ch16, ch_in):
+        raise ValueError("group_time_window: channels must be int16 values, one per timestamp")
+    lib = _lib.load()
+    d_ts = _dev(ts_in)
+    d_sorted, d_order = torch.empty_like(d_ts), torch.empty_like(d_ts)
+    ws = _empty(lib.wfb_sort_workspace_bytes(n))
+    _lib.check(lib.wfb_sort_pairs_i64(_ptr(d_ts), _ptr(torch.arange(n, dtype=torch.int64, device="cuda")), _ptr(d_sorted), _ptr(d_order),
+                                      n, _ptr(ws), ws.numel(), _stream()), "wfb_sort_pairs_i64")
+    ev, n_events = group_time_window_device(d_sorted, n, time_window_ns)
+    t = event_table_device(d_sorted, ev, n, n_events, _dev(ch16), order=d_order)
+    host = {k: t[k].cpu().numpy() for k in ("offsets", "members", "t_min", "t_max", "dt_ns", "n_hits")}
+    return dict(event_id=np.arange(n_events, dtype=np.int64), t_min=host["t_min"], t_max=host["t_max"], dt_ns=host["dt_ns"],
+                n_hits=host["n_hits"], offsets=host["offsets"], members=host["members"])
+
+
+def group_time_window_device(d_ts_sorted, n: int, time_window_ns: float):
+    """wfb_group_time_window on time-sorted int64 timestamps already on the device: (event ids int64[n] tensor,
+    number of events)."""
+    lib = _lib.load()
+    torch = _torch()
+    n = int(n)
+    ev = torch.empty(max(n, 1), dtype=torch.int64, device="cuda")
+    if n == 0:
+        return ev[:0], 0
     n_ev = torch.zeros(1, dtype=torch.int64, device="cuda")
     ws = _empty(lib.wfb_group_workspace_bytes(n))
-    _lib.check(lib.wfb_group_time_window(_ptr(d_ts), n, float(time_window_ns), _ptr(ev), _ptr(n_ev), _ptr(ws), ws.numel(), _stream()),
+    _lib.check(lib.wfb_group_time_window(_ptr(d_ts_sorted), n, float(time_window_ns), _ptr(ev), _ptr(n_ev), _ptr(ws), ws.numel(), _stream()),
                "wfb_group_time_window")
-    ev_sorted = ev.cpu().numpy()
-    n_events = int(n_ev.item())
-    ch = np.asarray(channels)[order]
-    inner = np.lexsort((np.arange(n), ch, ev_sorted))  # by event, then channel (stable)
-    members = order[inner]
-    counts = np.bincount(ev_sorted, minlength=n_events)
-    offsets = np.zeros(n_events + 1, dtype=np.int64)
-    np.cumsum(counts, out=offsets[1:])
-    ts_m = ts_in[members]
-    t_min, t_max = ts_m[offsets[:-1]], ts_m[offsets[1:] - 1]
-    return dict(event_id=np.arange(n_events, dtype=np.int64), t_min=t_min, t_max=t_max, dt_ns=(t_max - t_min) / 1e3,
-                n_hits=counts.astype(np.int64), offsets=offsets, members=members)
+    return ev[:n], int(n_ev.item())
+
+
+def event_table_device(d_ts_sorted, d_event_id, n: int, n_events: int, d_channel, *, order=None, area=None, height=None) -> dict:
+    """wfb_event_table: the CSR event table of wfb_group_time_window's events, all device tensors: ``offsets``,
+    ``members`` (input rows), ``t_min``, ``t_max``, ``dt_ns``, ``n_hits`` and the member-ordered ``member_ts``,
+    ``member_channel`` and - when ``area`` / ``height`` (float32, by input row) are given - ``member_area`` /
+    ``member_height``.  ``order``: sorted position -> input row (None: the rows are the sorted rows)."""
+    lib = _lib.load()
+    torch = _torch()
+    n, n_events = int(n), int(n_events)
+    dev = "cuda"
+    out = dict(offsets=torch.zeros(n_events + 1, dtype=torch.int64, device=dev), members=torch.empty(n, dtype=torch.int64, device=dev),
+               t_min=torch.empty(n_events, dtype=torch.int64, device=dev), t_max=torch.empty(n_events, dtype=torch.int64, device=dev),
+               dt_ns=torch.empty(n_events, dtype=torch.float64, device=dev), n_hits=torch.empty(n_events, dtype=torch.int64, device=dev),
+               member_ts=torch.empty(n, dtype=torch.int64, device=dev), member_channel=torch.empty(n, dtype=torch.int16, device=dev))
+    if area is not None:
+        out["member_area"] = torch.empty(n, dtype=torch.float32, device=dev)
+    if height is not None:
+        out["member_height"] = torch.empty(n, dtype=torch.float32, device=dev)
+    if n == 0:
+        return out
+    ws = _empty(lib.wfb_event_table_workspace_bytes(n))
+    _lib.check(lib.wfb_event_table(_ptr(d_ts_sorted), _ptr(d_event_id), n, n_events, _ptr(d_channel), _ptr(order), _ptr(area), _ptr(height),
+                                   _ptr(out["offsets"]), _ptr(out["members"]), _ptr(out["t_min"]), _ptr(out["t_max"]), _ptr(out["dt_ns"]),
+                                   _ptr(out["n_hits"]), _ptr(out["member_ts"]), _ptr(out["member_channel"]), _ptr(out.get("member_area")),
+                                   _ptr(out.get("member_height")), _ptr(ws), ws.numel(), _stream()), "wfb_event_table")
+    return out
 
 
 # --------------------------------------------------------------------------------------------
@@ -802,12 +841,22 @@ def df_columns(features: np.ndarray, record_id: np.ndarray | None = None, gains:
     ``gains``: {(board, channel): gain_adc_per_pe > 0} or None (no calibrated columns)."""
     from .dtypes import BASIC_FEATURES_DTYPE
 
-    lib = _lib.load()
-    torch = _torch()
     features = np.ascontiguousarray(features)
     if features.dtype != BASIC_FEATURES_DTYPE:
         raise ValueError("df_columns expects packed BASIC_FEATURES rows")
     n = len(features)
+    d_feat = _dev(features) if n else None
+    d_rid = _dev(np.asarray(record_id, dtype=np.int64)) if record_id is not None and n else None
+    cols = df_columns_device(d_feat, n, d_rid, gains)
+    return {k: v.cpu().numpy() for k, v in cols.items()}
+
+
+def df_columns_device(d_feat, n: int, d_record_id=None, gains: dict | None = None) -> dict:
+    """``df_columns`` on packed BASIC_FEATURES rows that live on the device (uint8 tensor, 36 B per row) with an
+    optional int64 device ``record_id`` column: the same columns, left on the device."""
+    lib = _lib.load()
+    torch = _torch()
+    n = int(n)
     with_pe = gains is not None
     cols = dict(order=torch.empty(n, dtype=torch.int64, device="cuda"), timestamp=torch.empty(n, dtype=torch.int64, device="cuda"),
                 record_id=torch.empty(n, dtype=torch.int64, device="cuda"), area=torch.empty(n, dtype=torch.float32, device="cuda"),
@@ -821,16 +870,14 @@ def df_columns(features: np.ndarray, record_id: np.ndarray | None = None, gains:
         rules = (_lib.GainRule * max(len(gains or {}), 1))()
         for i, ((b, c), g) in enumerate((gains or {}).items()):
             rules[i].board, rules[i].channel, rules[i].gain = int(b), int(c), float(g)
-        d_feat = _dev(features)
-        d_rid = _dev(np.asarray(record_id, dtype=np.int64)) if record_id is not None else None
         ws = _empty(lib.wfb_df_columns_workspace_bytes(n))
-        _lib.check(lib.wfb_df_columns(_ptr(d_feat), _ptr(d_rid) if d_rid is not None else None, n, rules, len(gains or {}), int(with_pe),
+        _lib.check(lib.wfb_df_columns(_ptr(d_feat), _ptr(d_record_id) if d_record_id is not None else None, n, rules, len(gains or {}), int(with_pe),
                                       _ptr(cols["order"]), _ptr(cols["timestamp"]), _ptr(cols["record_id"]), _ptr(cols["area"]),
                                       _ptr(cols["height"]), _ptr(cols["amp"]), _ptr(cols["max_abs_diff"]), _ptr(cols["board"]),
                                       _ptr(cols["channel"]), _ptr(cols["area_pe"]) if with_pe else None,
                                       _ptr(cols["height_pe"]) if with_pe else None, _ptr(ws), ws.numel(), _stream()), "wfb_df_columns")
         torch.cuda.current_stream().synchronize()  # `rules` (host) must outlive the staged copy
-    return {k: v.cpu().numpy() for k, v in cols.items()}
+    return cols
 
 
 def _range_struct(bounds) -> "_lib.Range":
@@ -887,14 +934,26 @@ def pair_events(offsets: np.ndarray, member_ts: np.ndarray, member_area: np.ndar
     d_off, d_ts = _dev(offsets), _dev(np.asarray(member_ts, dtype=np.int64))
     d_a, d_h = _dev(np.asarray(member_area, dtype=np.float32)), _dev(np.asarray(member_height, dtype=np.float32))
     d_dt = _dev(np.asarray(dt_ns, dtype=np.float64))
+    out = pair_events_device(d_off, n_ev, d_ts, d_a, d_h, d_dt, time_window_ns, nc)
+    return dict(keep=out["keep"].cpu().numpy().astype(bool), delta_t=out["delta_t"].cpu().numpy(),
+                area_ch=out["area_ch"].cpu().numpy(), height_ch=out["height_ch"].cpu().numpy())
+
+
+def pair_events_device(d_offsets, n_events: int, d_member_ts, d_member_area, d_member_height, d_dt_ns, time_window_ns: float,
+                       n_channels: int) -> dict:
+    """wfb_pair_events on CSR events that live on the device: ``keep`` (uint8), ``delta_t`` and the (n_events,
+    n_channels) ``area_ch`` / ``height_ch``, all device tensors."""
+    lib = _lib.load()
+    torch = _torch()
+    n_ev, nc = int(n_events), int(n_channels)
     keep = torch.empty(n_ev, dtype=torch.uint8, device="cuda")
     delta = torch.empty(n_ev, dtype=torch.float64, device="cuda")
     a_ch = torch.empty(max(n_ev * nc, 1), dtype=torch.float32, device="cuda")
     h_ch = torch.empty(max(n_ev * nc, 1), dtype=torch.float32, device="cuda")
-    _lib.check(lib.wfb_pair_events(_ptr(d_off), n_ev, _ptr(d_ts), _ptr(d_a), _ptr(d_h), _ptr(d_dt), float(time_window_ns), nc, _ptr(keep),
-                                   _ptr(delta), _ptr(a_ch), _ptr(h_ch), _stream()), "wfb_pair_events")
-    return dict(keep=keep.cpu().numpy().astype(bool), delta_t=delta.cpu().numpy(),
-                area_ch=a_ch.cpu().numpy()[: n_ev * nc].reshape(n_ev, nc), height_ch=h_ch.cpu().numpy()[: n_ev * nc].reshape(n_ev, nc))
+    if n_ev:
+        _lib.check(lib.wfb_pair_events(_ptr(d_offsets), n_ev, _ptr(d_member_ts), _ptr(d_member_area), _ptr(d_member_height), _ptr(d_dt_ns),
+                                       float(time_window_ns), nc, _ptr(keep), _ptr(delta), _ptr(a_ch), _ptr(h_ch), _stream()), "wfb_pair_events")
+    return dict(keep=keep, delta_t=delta, area_ch=a_ch[: n_ev * nc].view(n_ev, nc), height_ch=h_ch[: n_ev * nc].view(n_ev, nc))
 
 
 # --------------------------------------------------------------------------------------------

@@ -154,12 +154,22 @@ class B200DataFramePlugin(Plugin):
         have_channels = len(feats) > 0
         gains, enabled = self._resolve_gain_map(context, run_id, have_channels)
         cols = ops.df_columns(feats, rid, gains if enabled else None)
-        data = {k: cols[k] for k in ("timestamp", "record_id", "area", "height", "amp", "max_abs_diff", "board", "channel")}
-        if enabled:
-            data["area_pe"] = cols["area_pe"]
-            data["height_pe"] = cols["height_pe"]
-        # sort_values keeps the original row labels: the index is the sort permutation
-        return pd.DataFrame(data, index=pd.Index(cols["order"], dtype=np.int64))
+        return df_frame(cols, cols["order"], enabled)
+
+
+DF_COLUMNS = ("timestamp", "record_id", "area", "height", "amp", "max_abs_diff", "board", "channel")
+
+
+def df_frame(cols: dict, index, with_pe: bool):
+    """The `df` DataFrame of ``df_columns`` output (host arrays); ``index`` = the rows' labels."""
+    import pandas as pd
+
+    data = {k: cols[k] for k in DF_COLUMNS}
+    if with_pe:
+        data["area_pe"] = cols["area_pe"]
+        data["height_pe"] = cols["height_pe"]
+    # sort_values keeps the original row labels: the index is the sort permutation
+    return pd.DataFrame(data, index=pd.Index(index, dtype=np.int64))
 
 
 class B200PairedEventsPlugin(Plugin):
@@ -205,6 +215,13 @@ def pair_events_frame(df_events, n_channels: int, start_channel_slice: int, time
         _, area = _csr_of(df_events, areas_key, np.float32)
         _, height = _csr_of(df_events, heights_key, np.float32)
     out = ops.pair_events(offsets, ts, area, height, df_events["dt/ns"].to_numpy(dtype=np.float64), float(tw), n_channels)
+    return paired_frame(df_events, offsets, out, n_channels, start_channel_slice)
+
+
+def paired_frame(df_events, offsets: np.ndarray, out: dict, n_channels: int, start_channel_slice: int):
+    """df_paired from the events frame, its CSR ``offsets`` and the pair_events columns of ALL its events (``keep``,
+    ``delta_t``, ``area_ch``, ``height_ch``).  The float64 widening of a per-channel column depends on every kept
+    event, so this runs once on the whole run's events."""
     keep = out["keep"]
     df_paired = df_events[keep].copy()
     if "delta_t" not in df_paired.columns and not df_paired.empty:

@@ -117,17 +117,26 @@ class B200GroupedEventsPlugin(Plugin):
         ts = df["timestamp"].to_numpy()
         ch = df["channel"].to_numpy()
         ev = ops.group_time_window(ts, ch, float(tw))
-        m, off = ev["members"], ev["offsets"]
+        m = ev["members"]
         areas, heights = df[area_col].to_numpy(), df[height_col].to_numpy()
-        out = pd.DataFrame({
-            "event_id": ev["event_id"], "t_min": ev["t_min"], "t_max": ev["t_max"], "dt/ns": ev["dt_ns"],
-            "n_hits": ev["n_hits"].astype(np.int32),
-            "channels": _ragged(ch, m, off), "areas": _ragged(areas, m, off),
-            "heights": _ragged(heights, m, off), "timestamps": _ragged(ts, m, off),
-        })
-        # the flat member arrays, for B200PairedEventsPlugin (saves re-flattening the object columns).  Kept beside the
-        # frame, not in df.attrs: the Context saves DataFrames with to_parquet, which json-dumps the attrs
-        # (core/storage/memmap.py:886)
-        stash_member_arrays(out, {"offsets": off, "timestamps": ts[m], "areas": areas[m].astype(np.float32),
-                                  "heights": heights[m].astype(np.float32)})
-        return out
+        return events_frame(ev, ch[m], areas[m], heights[m], ts[m])
+
+
+def events_frame(ev: dict, channels, areas, heights, timestamps):
+    """The df_events DataFrame of an event table (``event_id``, ``t_min``, ``t_max``, ``dt_ns``, ``n_hits``, CSR
+    ``offsets``) and its member columns, already in member order."""
+    import pandas as pd
+
+    off = np.asarray(ev["offsets"], dtype=np.int64)
+    split = (lambda v: np.split(v, off[1:-1])) if len(off) > 1 else (lambda v: [])
+    out = pd.DataFrame({
+        "event_id": ev["event_id"], "t_min": ev["t_min"], "t_max": ev["t_max"], "dt/ns": ev["dt_ns"],
+        "n_hits": np.asarray(ev["n_hits"]).astype(np.int32),
+        "channels": split(channels), "areas": split(areas), "heights": split(heights), "timestamps": split(timestamps),
+    })
+    # the flat member arrays, for B200PairedEventsPlugin (saves re-flattening the object columns).  Kept beside the
+    # frame, not in df.attrs: the Context saves DataFrames with to_parquet, which json-dumps the attrs
+    # (core/storage/memmap.py:886)
+    stash_member_arrays(out, {"offsets": off, "timestamps": timestamps, "areas": np.asarray(areas).astype(np.float32),
+                              "heights": np.asarray(heights).astype(np.float32)})
+    return out
