@@ -356,6 +356,25 @@ int wfb_event_table(const int64_t* ts_sorted_dev, const int64_t* event_id_dev, i
                     int64_t* n_hits_dev, int64_t* member_ts_dev, int16_t* member_channel_dev, float* member_area_dev,
                     float* member_height_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
+/* The event table of chain-clustered hit windows (event_grouping.py:418-471, the hit_grouped columns).
+ * order_dev / event_id_dev int64[n] as wfb_group_hit_windows / wfb_group_abs_windows wrote them (order sorted by
+ * (abs_start, dt, timestamp, record_id, input row); every event a contiguous run of it, numbered 0 .. n_events - 1);
+ * board_dev / channel_dev int16, dt_dev int32 and abs_start_dev / abs_end_dev float64 are indexed by INPUT row
+ * (timestamp and record_id enter through order).  Writes offsets_dev[n_events + 1] (CSR), members_dev[n] (input rows
+ * in the order np.lexsort((record_id, timestamp, abs_start, dt, channel, board, event)), ties in input row order),
+ * t_min = (int64) min abs_start and t_max = (int64) max abs_end of every event (truncated toward zero),
+ * dt_ns = (double)(t_max - t_min) / 1e3 and n_hits.  rows_dev (optional, packed THRESHOLD_HIT or HIT_MERGED rows of
+ * row_bytes = 60 or 72, 4-byte aligned) is gathered into member_rows_dev in member order.  Events of up to 32 members
+ * are ranked by one warp each; larger ones by two stable radix sorts of their positions, by (board, channel, dt) and
+ * then by event.  Synchronises the stream once. */
+size_t wfb_hit_event_table_workspace_bytes(int64_t n);
+int wfb_hit_event_table(const int64_t* order_dev, const int64_t* event_id_dev, int64_t n, int64_t n_events,
+                        const int16_t* board_dev, const int16_t* channel_dev, const int32_t* dt_dev,
+                        const double* abs_start_dev, const double* abs_end_dev, const void* rows_dev, int32_t row_bytes,
+                        int64_t* offsets_dev, int64_t* members_dev, int64_t* t_min_dev, int64_t* t_max_dev,
+                        double* dt_ns_dev, int64_t* n_hits_dev, void* member_rows_dev, void* workspace_dev,
+                        size_t workspace_bytes, void* stream);
+
 /* K1 for records of different lengths (channels / parts with different waveform widths,
  * records_builder.py:212-302 per part + :870-945 merge): like wfb_build_records, but every record names its
  * own int16 samples (byte offset into samples_dev + count) and the wave_pool is ragged (wave_offset = running

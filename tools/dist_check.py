@@ -24,7 +24,14 @@ ids byte for byte.
 rows, then ``distributed.events_sharded`` (time_window_ns = pair window = 100, 2 paired channels).  It reports the time of
 every stage (each ended by a device synchronize), gathered_bytes, the event counts and the peak device memory of the leg;
 with --verify 1 rank 0 runs the single-GPU chain (df columns, wfb_group_time_window, wfb_event_table, wfb_pair_events
-on the whole run) and checks the gathered df columns, event table, members and df_paired columns byte for byte."""
+on the whole run) and checks the gathered df columns, event table, members and df_paired columns byte for byte.
+
+--hit-events adds the hit_grouped event table on the rows merge_group_sharded left on every rank:
+``distributed.hit_events_sharded`` with the device backend (wfb_hit_event_table).  It reports the table's stage time
+(ended by a device synchronize), the events and member rows of every rank and the peak extra device memory of the stage;
+with --verify 1 every rank gathers the hit_grouped frame of the whole run (``distributed.gather_hit_grouped_frame``) and
+rank 0 checks it against ``ops.group_hit_windows`` on the single-GPU hit_merged rows, packaged as B200HitGroupedPlugin
+does."""
 import argparse
 import os
 import sys
@@ -47,6 +54,7 @@ ap.add_argument("--source", choices=("synth", "v1725"), default="synth")
 ap.add_argument("--files-per-rank", type=int, default=2)
 ap.add_argument("--samples", type=int, default=800)
 ap.add_argument("--events", action="store_true", help="also run the sharded df -> df_events -> df_paired leg")
+ap.add_argument("--hit-events", action="store_true", help="also build the sharded hit_grouped event table")
 args = ap.parse_args()
 
 D.init_process_group("nccl")
@@ -236,8 +244,56 @@ def verify_events(got_df, got, feats) -> str:
     return f" | df, df_events and df_paired columns byte-identical to the single-GPU chain ({n_all} rows, {n_ev} events)"
 
 
+def gpu_name() -> str:
+    import subprocess
+
+    return subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", str(local)],
+                          capture_output=True, text=True).stdout.strip()
+
+
+def hit_events_leg():
+    """hit_events_sharded on this rank's merge_group_sharded result; with --verify the gathered hit_grouped frame."""
+    torch.cuda.synchronize()
+    torch.cuda.reset_peak_memory_stats()
+    base_mem = torch.cuda.memory_allocated()
+    if ws > 1:
+        dist.barrier()
+    t = time.perf_counter()
+    hev = D.hit_events_sharded(sh, D.DeviceRows(THRESHOLD_HIT_DTYPE))
+    torch.cuda.synchronize()
+    t_tab = time.perf_counter() - t
+    peak = torch.cuda.max_memory_allocated() - base_mem
+    line = (f"rank {rank}: events {hev['n_events']} (base {hev['event_base']}) member rows {int(hev['members'].numel())} | "
+            f"hit_events_sharded {1e3 * t_tab:.2f} ms | peak extra device memory {peak / 1e9:.3f} GB | {gpu_name()}")
+    lines = D.gather_rows(np.frombuffer(line.encode().ljust(1024)[:1024], dtype="S1024")) if ws > 1 else [line.encode()]
+    if rank == 0:
+        print(f"hit events leg: world={ws} records/rank={n}")
+        for ln in lines:
+            print("  " + ln.decode().strip())
+    frame = D.gather_hit_grouped_frame(hev) if args.verify else None
+    return f"hit events={int(hev['events_per_rank'].sum())}", frame
+
+
+def frames_equal(got, want) -> bool:
+    if list(got.columns) != list(want.columns) or len(got) != len(want) or not got.index.equals(want.index):
+        return False
+    for c in want.columns:
+        if got[c].dtype != want[c].dtype:
+            return False
+        if want[c].dtype == object:
+            if not all(a.dtype == b.dtype and np.array_equal(a, b) for a, b in zip(got[c], want[c])):
+                return False
+        elif not np.array_equal(got[c].to_numpy(), want[c].to_numpy()):
+            return False
+    return True
+
+
 if args.events:
     msg += " | " + events_leg()
+hit_frame = None
+if args.hit_events:
+    out, hit_frame = hit_events_leg()
+    msg += " | " + out
 if args.verify:
     feats_l = res["features"][: n * 36].cpu().numpy()
     hits_l = res["hits"][: total * 60].cpu().numpy().view(THRESHOLD_HIT_DTYPE)
@@ -278,6 +334,16 @@ if args.verify:
             assert np.array_equal(got_m[f], want_m[f], equal_nan=want_m[f].dtype.kind == "f"), f"hit_merged.{f} differs"
         assert np.array_equal(got_ev, want_ev), "event ids differ"
         assert g["n_events"] == int(tot[3])
+        if hit_frame is not None:
+            from waveformanalysis_b200.dtypes import HIT_MERGED_COMPONENTS_DTYPE
+            from waveformanalysis_b200.plugins.grouping import hit_grouped_frame, hit_member_columns
+
+            comps = np.zeros(ftotal, dtype=HIT_MERGED_COMPONENTS_DTYPE)
+            comps["merged_index"] = m["cluster_index"][:ftotal].cpu().numpy()
+            comps["hit_index"] = m["order"][:ftotal].cpu().numpy()
+            table = ops.group_hit_windows(want_m, WINDOW, comps, hits)
+            assert frames_equal(hit_frame, hit_grouped_frame(table, hit_member_columns(want_m[table["members"]]))), "hit_grouped differs"
+            msg += f" | hit_grouped frame equal to ops.group_hit_windows on the single-GPU hit_merged ({len(hit_frame)} events)"
         merged_over = int((want_m["component_count"] > 1).sum())
         what = "records, pool, " if ingest is not None else ""
         msg += f" | {what}features, hits, merged rows and event ids byte-identical to the single-GPU run ({n_all} records, {merged_over} clusters of several hits)"

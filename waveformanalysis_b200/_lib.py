@@ -171,6 +171,8 @@ PROTOTYPES = {
     "wfb_group_time_window": (C.c_int, [_vp, _i64, _dbl, _vp, _vp, _vp, _sz, _vp]),
     "wfb_event_table_workspace_bytes": (_sz, [_i64]),
     "wfb_event_table": (C.c_int, [_vp, _vp, _i64, _i64] + [_vp] * 14 + [_vp, _sz, _vp]),
+    "wfb_hit_event_table_workspace_bytes": (_sz, [_i64]),
+    "wfb_hit_event_table": (C.c_int, [_vp, _vp, _i64, _i64] + [_vp] * 6 + [_i32] + [_vp] * 7 + [_vp, _sz, _vp]),
     "wfb_df_columns_workspace_bytes": (_sz, [_i64]),
     "wfb_df_columns": (C.c_int, [_vp, _vp, _i64, _vp, _i32, _i32] + [_vp] * 11 + [_vp, _sz, _vp]),
     "wfb_s1s2_classify": (C.c_int, [_vp, _i64, _vp, _i64, C.POINTER(S1S2Params), _vp, _vp]),

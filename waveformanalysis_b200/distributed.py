@@ -312,7 +312,17 @@ class HostRows:
         clusters, merged, comps = self.merge_fn(owned, merge_gap_ns=merge_gap_ns, max_total_width_ns=max_total_width_ns)
         ev = self.group_fn(merged, time_window_ns, component_rows=comps, component_hits=owned)
         return dict(merged=merged, event_of_merged=np.asarray(ev["event_of_hit"], dtype=np.int64), n_events=len(ev["t_min"]),
-                    n_clusters=len(merged))
+                    n_clusters=len(merged), grouping=ev)
+
+    def hit_events(self, sh):
+        ev = sh["grouping"]
+        m = np.asarray(ev["members"], dtype=np.int64)
+        res = {k: np.asarray(ev[k]) for k in ("t_min", "t_max", "dt_ns", "n_hits", "offsets")}
+        res.update(members=m, member_rows=sh["merged"][m])
+        return res
+
+    def iota(self, n, base):
+        return np.arange(n, dtype=np.int64) + base
 
 
 class DeviceRows:
@@ -355,7 +365,18 @@ class DeviceRows:
         t, n = owned
         m = ops.hit_merge_device(t, n, merge_gap_ns=merge_gap_ns, max_total_width_ns=max_total_width_ns)
         g = ops.group_rows_device(m["merged"], m["n_clusters"], 72, time_window_ns, abs_start=m["abs_start"], abs_end=m["abs_end"])
-        return dict(merged=m["merged"], event_of_merged=g["event_of_row"], n_events=g["n_events"], n_clusters=m["n_clusters"], detail=m)
+        return dict(merged=m["merged"], event_of_merged=g["event_of_row"], n_events=g["n_events"], n_clusters=m["n_clusters"], detail=m,
+                    grouping=g)
+
+    def hit_events(self, sh):
+        from . import ops
+
+        return ops.hit_event_table_device(sh["merged"], sh["n_clusters"], 72, sh["grouping"])
+
+    def iota(self, n, base):
+        import torch
+
+        return torch.arange(n, dtype=torch.int64, device="cuda") + base
 
 
 def merge_group_sharded(rows, backend, *, time_window_ns: float, merge_gap_ns: float = 0.0, max_total_width_ns: float = 10000.0,
@@ -386,6 +407,24 @@ def merge_group_sharded(rows, backend, *, time_window_ns: float, merge_gap_ns: f
         raise RuntimeError("no gap wider than the grouping window between two time shards: the run cannot be cut here")
     R = len(heads)
     me = rank if R > 1 else 0
+    owned = owned_hit_rows(backend, rows, me, heads, tails, counts, cuts)
+    res = backend.merge_and_group(owned, merge_gap_ns, max_total_width_ns, time_window_ns)
+    table = _allgather_i64([res["n_clusters"], res["n_events"]])
+    gathered += table.nbytes
+    res["cluster_base"] = int(table[:rank, 0].sum())
+    res["event_base"] = int(table[:rank, 1].sum())
+    res["event_of_merged"] = res["event_of_merged"][: res["n_clusters"]] + res["event_base"]
+    res["clusters_per_rank"], res["events_per_rank"] = table[:, 0].copy(), table[:, 1].copy()
+    res["cuts"], res["gathered_bytes"], res["zone_rows"], res["owned"] = cuts, gathered, k, owned
+    return res
+
+
+def owned_hit_rows(backend, rows, me: int, heads, tails, counts, cuts):
+    """The hit rows rank ``me`` owns in merge_group_sharded, given every rank's zones, row counts and the cuts: lower
+    ranks' zone rows, the rank's own rows and upper ranks' zone rows whose window starts between its two cuts, in global
+    record order (``rows``: the rank's rows as the backend holds them)."""
+    R, n = len(heads), int(counts[me])
+    head, tail = heads[me], tails[me]
     live = [r for r in range(R) if counts[r] > 0]
     lo_cut, hi_cut = -np.inf, np.inf
     if me in live:
@@ -405,17 +444,48 @@ def merge_group_sharded(rows, backend, *, time_window_ns: float, merge_gap_ns: f
     upper = [inside(z) for q in range(me + 1, R) for z in (heads[q], tails[q])]
     first = np.concatenate(lower + [inside(head)]) if n or lower else head[:0]
     last = np.concatenate([inside(tail)] + upper) if n or upper else head[:0]
-    k_head, k_tail = len(head), len(tail)
-    owned = backend.assemble(rows, k_head, k_tail, first, last)
-    res = backend.merge_and_group(owned, merge_gap_ns, max_total_width_ns, time_window_ns)
-    table = _allgather_i64([res["n_clusters"], res["n_events"]])
-    gathered += table.nbytes
-    res["cluster_base"] = int(table[:rank, 0].sum())
-    res["event_base"] = int(table[:rank, 1].sum())
-    res["event_of_merged"] = res["event_of_merged"][: res["n_clusters"]] + res["event_base"]
-    res["clusters_per_rank"], res["events_per_rank"] = table[:, 0].copy(), table[:, 1].copy()
-    res["cuts"], res["gathered_bytes"], res["zone_rows"], res["owned"] = cuts, gathered, k, owned
+    return backend.assemble(rows, len(head), len(tail), first, last)
+
+
+def hit_events_sharded(sh: dict, backend) -> dict:
+    """hit_grouped's event table of a time-sharded run: every rank tabulates the events it owns after
+    ``merge_group_sharded`` (``sh``, left unchanged) with the same ``backend`` - ``wfb_hit_event_table`` on its device with
+    ``DeviceRows``, the grouping function's own table with ``HostRows``.  No collective: every event lies on one rank, and
+    ``sh["event_base"]`` (already gathered) numbers them globally.
+
+    Returns ``event_id`` (global), ``t_min``, ``t_max``, ``dt_ns``, ``n_hits``, the CSR ``offsets``, ``members`` (indices
+    into the rank's ``sh["merged"]`` rows), ``member_rows`` (those rows in member order: HIT_MERGED rows, packed on the
+    device with ``DeviceRows``), ``n_events``, ``event_base`` and ``events_per_rank``.  Concatenated in rank order, the
+    tables equal the single-GPU table of the whole run: a rank's merged rows keep their global relative order, so ties
+    resolve alike."""
+    res = dict(backend.hit_events(sh))
+    n_ev, base = int(sh["n_events"]), int(sh["event_base"])
+    res.update(event_id=backend.iota(n_ev, base), n_events=n_ev, event_base=base, events_per_rank=np.asarray(sh["events_per_rank"]).copy())
     return res
+
+
+def gather_hit_grouped_frame(ev_sh: dict):
+    """The hit_grouped DataFrame of the WHOLE run on every rank (``hit_events_sharded``'s result), equal to what
+    B200HitGroupedPlugin returns for the run.  Every rank receives every event and member row, so this holds the whole
+    run in each process (like ``gather_rows``): it is for checks and small runs."""
+    import pandas as pd
+
+    from .dtypes import HIT_MERGED_DTYPE
+    from .plugins.grouping import HIT_GROUPED_COLUMNS, hit_grouped_frame, hit_member_columns
+
+    n_ev = int(ev_sh["n_events"])
+    ev_rows = np.zeros(n_ev, dtype=[("event_id", "<i8"), ("t_min", "<i8"), ("t_max", "<i8"), ("dt_ns", "<f8"), ("n_hits", "<i8")])
+    for k in ev_rows.dtype.names:
+        ev_rows[k] = _host(ev_sh[k])
+    ev_rows = gather_rows(ev_rows)
+    m = len(_host(ev_sh["members"]))
+    mem = np.ascontiguousarray(_host(ev_sh["member_rows"])).view(np.uint8).reshape(-1)[: m * HIT_MERGED_DTYPE.itemsize]
+    mem = gather_rows(mem.view(HIT_MERGED_DTYPE))
+    if len(ev_rows) == 0:
+        return pd.DataFrame(columns=HIT_GROUPED_COLUMNS)
+    table = {k: np.ascontiguousarray(ev_rows[k]) for k in ("event_id", "t_min", "t_max", "dt_ns", "n_hits")}
+    table["offsets"] = np.r_[0, np.cumsum(ev_rows["n_hits"])].astype(np.int64)
+    return hit_grouped_frame(table, hit_member_columns(mem))
 
 
 def assemble_merged(merged_all: np.ndarray, event_of_merged_all: np.ndarray):

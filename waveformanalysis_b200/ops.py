@@ -327,9 +327,10 @@ def width_integral(records: np.ndarray, pool: np.ndarray, *, q_low=0.10, q_high=
 def group_hit_windows(hits: np.ndarray, time_window_ns: float, component_rows=None, component_hits=None) -> dict:
     """Chain clustering of absolute hit windows (event_grouping.py:287-471).  Rows merged across records
     (sample window -1) take their window from the component hits (``hit_merged_components`` rows +
-    ``hit_threshold``), a small host reduction; everything after the windows runs on the device.  The sort, running maximum, boundary flags and event ids are computed on the
-    device; the per-event member ordering (a small lexsort) and the ragged packaging stay on the
-    host.  Returns the same dict as the oracle."""
+    ``hit_threshold``), a small host reduction; everything after the windows runs on the device: the sort,
+    running maximum, boundary flags and event ids (wfb_group_hit_windows / wfb_group_abs_windows), then the
+    event table (wfb_hit_event_table: member order, t_min / t_max / dt/ns / n_hits).  Returns the same dict
+    as the oracle, plus ``order``."""
     lib = _lib.load()
     torch = _torch()
     if time_window_ns < 0:
@@ -376,22 +377,36 @@ def group_hit_windows(hits: np.ndarray, time_window_ns: float, component_rows=No
         _lib.check(lib.wfb_group_hit_windows(_ptr(d_ts), _ptr(d_pos), _ptr(d_s), _ptr(d_e), _ptr(d_dt), _ptr(d_rid), nh, float(time_window_ns),
                                              _ptr(order), _ptr(ev), _ptr(a0), _ptr(a1), _ptr(n_ev), _ptr(ws), ws.numel(), _stream()),
                    "wfb_group_hit_windows")
-    event_of_hit = ev.cpu().numpy()
-    abs0, abs1 = a0.cpu().numpy(), a1.cpu().numpy()
     n_events = int(n_ev.item())
-    morder = np.lexsort((hits["record_id"].astype(np.int64), hits["timestamp"].astype(np.int64), abs0, hits["dt"].astype(np.int32),
-                         hits["channel"].astype(np.int16), hits["board"].astype(np.int16), event_of_hit))
-    counts = np.bincount(event_of_hit, minlength=n_events)
-    offsets = np.zeros(n_events + 1, dtype=np.int64)
-    np.cumsum(counts, out=offsets[1:])
-    tmin = np.full(n_events, np.inf)
-    tmax = np.full(n_events, -np.inf)
-    np.minimum.at(tmin, event_of_hit, abs0)
-    np.maximum.at(tmax, event_of_hit, abs1)
-    t_min, t_max = tmin.astype(np.int64), tmax.astype(np.int64)
-    return dict(event_id=np.arange(n_events, dtype=np.int64), t_min=t_min, t_max=t_max, dt_ns=(t_max - t_min) / 1e3,
-                n_hits=counts.astype(np.int64), offsets=offsets, members=morder.astype(np.int64), event_of_hit=event_of_hit,
+    t = _hit_event_table(order, ev, nh, n_events, _dev(hits["board"].astype(np.int16)), _dev(hits["channel"].astype(np.int16)), d_dt, a0, a1)
+    host = {k: t[k].cpu().numpy() for k in ("offsets", "members", "t_min", "t_max", "dt_ns", "n_hits")}
+    return dict(event_id=np.arange(n_events, dtype=np.int64), t_min=host["t_min"], t_max=host["t_max"], dt_ns=host["dt_ns"],
+                n_hits=host["n_hits"], offsets=host["offsets"], members=host["members"], event_of_hit=ev.cpu().numpy(),
                 order=order.cpu().numpy())
+
+
+def _hit_event_table(d_order, d_event_id, n: int, n_events: int, d_board, d_channel, d_dt, d_abs_start, d_abs_end, *, rows=None,
+                     row_bytes: int = 0) -> dict:
+    """wfb_hit_event_table on device columns indexed by input row (``order`` / ``event_id`` as the grouping wrote them):
+    device tensors ``offsets``, ``members``, ``t_min``, ``t_max``, ``dt_ns``, ``n_hits`` and - when ``rows`` (packed rows
+    of ``row_bytes``) is given - ``member_rows`` (uint8, the rows in member order)."""
+    lib = _lib.load()
+    torch = _torch()
+    n, n_events = int(n), int(n_events)
+    dev = "cuda"
+    out = dict(offsets=torch.zeros(n_events + 1, dtype=torch.int64, device=dev), members=torch.empty(n, dtype=torch.int64, device=dev),
+               t_min=torch.empty(n_events, dtype=torch.int64, device=dev), t_max=torch.empty(n_events, dtype=torch.int64, device=dev),
+               dt_ns=torch.empty(n_events, dtype=torch.float64, device=dev), n_hits=torch.empty(n_events, dtype=torch.int64, device=dev))
+    if rows is not None:
+        out["member_rows"] = torch.empty(n * int(row_bytes), dtype=torch.uint8, device=dev)
+    if n == 0:
+        return out
+    ws = _empty(lib.wfb_hit_event_table_workspace_bytes(n))
+    _lib.check(lib.wfb_hit_event_table(_ptr(d_order), _ptr(d_event_id), n, n_events, _ptr(d_board), _ptr(d_channel), _ptr(d_dt),
+                                       _ptr(d_abs_start), _ptr(d_abs_end), _ptr(rows), int(row_bytes), _ptr(out["offsets"]), _ptr(out["members"]),
+                                       _ptr(out["t_min"]), _ptr(out["t_max"]), _ptr(out["dt_ns"]), _ptr(out["n_hits"]), _ptr(out.get("member_rows")),
+                                       _ptr(ws), ws.numel(), _stream()), "wfb_hit_event_table")
+    return out
 
 
 def group_time_window(timestamps: np.ndarray, channels: np.ndarray, time_window_ns: float) -> dict:
@@ -985,13 +1000,14 @@ def hit_merge_device(d_hits, n: int, *, merge_gap_ns: float = 0.0, max_total_wid
 
 def group_rows_device(d_rows, n: int, row_bytes: int, time_window_ns: float, abs_start=None, abs_end=None) -> dict:
     """Chain clustering (event_grouping.py:287-471) of packed hit rows on the device: ``event_of_row`` (int64[n], in row
-    order), ``n_events``; ``abs_start`` / ``abs_end`` default to the rows' own sample windows."""
+    order), ``n_events``, the sort ``order`` and the rows' ``dt`` / ``abs_start`` / ``abs_end`` (what
+    ``hit_event_table_device`` takes); ``abs_start`` / ``abs_end`` default to the rows' own sample windows."""
     lib = _lib.load()
     torch = _torch()
     n = int(n)
     ev = torch.empty(max(n, 1), dtype=torch.int64, device="cuda")
     if n == 0:
-        return dict(event_of_row=ev[:0], n_events=0)
+        return dict(event_of_row=ev[:0], n_events=0, order=ev[:0])
     ts = torch.empty(n, dtype=torch.int64, device="cuda")
     dt = torch.empty(n, dtype=torch.int32, device="cuda")
     rid = torch.empty(n, dtype=torch.int64, device="cuda")
@@ -1006,7 +1022,19 @@ def group_rows_device(d_rows, n: int, row_bytes: int, time_window_ns: float, abs
     ws = _empty(lib.wfb_group_workspace_bytes(n))
     _lib.check(lib.wfb_group_abs_windows(_ptr(ts), _ptr(abs_start), _ptr(abs_end), _ptr(dt), _ptr(rid), n, float(time_window_ns), _ptr(order),
                                          _ptr(ev), _ptr(n_ev), _ptr(ws), ws.numel(), _stream()), "wfb_group_abs_windows")
-    return dict(event_of_row=ev, n_events=int(n_ev.item()), abs_start=abs_start, abs_end=abs_end)
+    return dict(event_of_row=ev, n_events=int(n_ev.item()), abs_start=abs_start, abs_end=abs_end, order=order, dt=dt)
+
+
+def hit_event_table_device(d_rows, n: int, row_bytes: int, group: dict) -> dict:
+    """wfb_hit_event_table on packed hit rows that stay on the device (uint8 tensor, ``row_bytes`` = 60 or 72 per row) and
+    their grouping ``group`` (``group_rows_device``'s result): device tensors ``offsets``, ``members`` (row indices),
+    ``t_min``, ``t_max``, ``dt_ns``, ``n_hits`` and ``member_rows`` (the packed rows in member order)."""
+    n, rb = int(n), int(row_bytes)
+    if n == 0:
+        return _hit_event_table(None, None, 0, 0, None, None, None, None, None, rows=d_rows, row_bytes=rb)
+    bc = d_rows[: n * rb].view(n, rb)[:, 48:52].contiguous().view(_torch().int16).view(n, 2)  # board, channel
+    return _hit_event_table(group["order"], group["event_of_row"], n, group["n_events"], bc[:, 0].contiguous(), bc[:, 1].contiguous(),
+                            group["dt"], group["abs_start"], group["abs_end"], rows=d_rows, row_bytes=rb)
 
 
 def filter_run_device(run: DeviceRun, cfg: dict):

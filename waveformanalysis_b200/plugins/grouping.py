@@ -32,11 +32,6 @@ def member_arrays_of(frame):
     return _MEMBER_ARRAYS.get(id(frame))
 
 
-def _ragged(values: np.ndarray, members: np.ndarray, offsets: np.ndarray) -> list:
-    flat = values[members]
-    return np.split(flat, offsets[1:-1]) if len(offsets) > 1 else []
-
-
 class B200HitGroupedPlugin(Plugin):
     provides = "hit_grouped"
     depends_on = ["hit_merged", "hit_merged_components", "hit_threshold"]
@@ -80,20 +75,7 @@ class B200HitGroupedPlugin(Plugin):
             comp_rows = context.get_data(run_id, "hit_merged_components")
             comp_hits = context.get_data(run_id, "hit_threshold")
         ev = ops.group_hit_windows(hits, time_window_ns, comp_rows, comp_hits)
-        m, off = ev["members"], ev["offsets"]
-        return pd.DataFrame({
-            "event_id": ev["event_id"], "t_min": ev["t_min"], "t_max": ev["t_max"], "dt/ns": ev["dt_ns"],
-            "n_hits": ev["n_hits"],
-            "dt": _ragged(hits["dt"].astype(np.int32), m, off),
-            "boards": _ragged(hits["board"].astype(np.int16), m, off),
-            "channels": _ragged(hits["channel"].astype(np.int16), m, off),
-            "heights": _ragged(hits["height"].astype(np.float32), m, off),
-            "integrals": _ragged(hits["integral"].astype(np.float32), m, off),
-            "timestamps": _ragged(hits["timestamp"].astype(np.int64), m, off),
-            "record_ids": _ragged(hits["record_id"].astype(np.int64), m, off),
-            "sample_starts": _ragged(hits[sn].astype(np.int32), m, off),
-            "sample_ends": _ragged(hits[en].astype(np.int32), m, off),
-        }, columns=HIT_GROUPED_COLUMNS)
+        return hit_grouped_frame(ev, hit_member_columns(hits[ev["members"]]))
 
 
 class B200GroupedEventsPlugin(Plugin):
@@ -140,3 +122,26 @@ def events_frame(ev: dict, channels, areas, heights, timestamps):
     stash_member_arrays(out, {"offsets": off, "timestamps": timestamps, "areas": np.asarray(areas).astype(np.float32),
                               "heights": np.asarray(heights).astype(np.float32)})
     return out
+
+
+def hit_member_columns(rows: np.ndarray) -> dict:
+    """The hit_grouped list columns of hit rows (hit_merged with sample_start / sample_end, or edge_start / edge_end)
+    already in member order, flat, in the plugin's dtypes."""
+    names = rows.dtype.names
+    sn, en = ("sample_start", "sample_end") if "sample_start" in names else ("edge_start", "edge_end")
+    return {"dt": rows["dt"].astype(np.int32), "boards": rows["board"].astype(np.int16), "channels": rows["channel"].astype(np.int16),
+            "heights": rows["height"].astype(np.float32), "integrals": rows["integral"].astype(np.float32),
+            "timestamps": rows["timestamp"].astype(np.int64), "record_ids": rows["record_id"].astype(np.int64),
+            "sample_starts": rows[sn].astype(np.int32), "sample_ends": rows[en].astype(np.int32)}
+
+
+def hit_grouped_frame(ev: dict, members: dict):
+    """The hit_grouped DataFrame of an event table (``event_id``, ``t_min``, ``t_max``, ``dt_ns``, ``n_hits``, CSR
+    ``offsets``) and its flat member columns (``hit_member_columns``), already in member order."""
+    import pandas as pd
+
+    off = np.asarray(ev["offsets"], dtype=np.int64)
+    split = (lambda v: np.split(v, off[1:-1])) if len(off) > 1 else (lambda v: [])
+    cols = {"event_id": ev["event_id"], "t_min": ev["t_min"], "t_max": ev["t_max"], "dt/ns": ev["dt_ns"], "n_hits": ev["n_hits"]}
+    cols.update({k: split(v) for k, v in members.items()})
+    return pd.DataFrame(cols, columns=HIT_GROUPED_COLUMNS)
