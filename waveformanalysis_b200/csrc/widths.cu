@@ -276,7 +276,7 @@ struct ChargeSrc {
         else if (mode == 1) sig = (double)__fsub_rn(b32, (float)wi);
         else if (mode == 2) sig = (double)__fsub_rn((float)wi, b32);
         else sig = __dsub_rn((double)wi, b);
-        return fmax(sig, 0.0);
+        return (sig > 0.0 || isnan(sig)) ? sig : 0.0;  // np.maximum(sig, 0.0) keeps a NaN (fmax would drop it)
     }
 };
 
@@ -421,8 +421,12 @@ __global__ void __launch_bounds__(128) width_integral_kernel(const T* __restrict
     double q = 0.0;
     int lo = 0, hi = 0;
     bool done = false;
+    if (L > 0 && isnan(m.baseline)) {  // every signal sample is NaN: np.sum is NaN, the quantile indices stay 0
+        q = __longlong_as_double(0x7ff8000000000000ll);
+        done = true;
+    }
     if constexpr (sizeof(T) == 2) {
-        if (L >= 8 && (reinterpret_cast<uintptr_t>(pool + off) & 15) == 0) {
+        if (!done && L >= 8 && (reinterpret_cast<uintptr_t>(pool + off) & 15) == 0) {
             const uint4* ch = reinterpret_cast<const uint4*>(pool + off);
             switch (x.mode) {
                 case 0: width_integral_fast<T, 0>(ch, L, ChargeTerm<T, 0>{x.b, x.b32}, q_low, q_high, q, lo, hi); break;

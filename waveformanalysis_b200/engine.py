@@ -326,6 +326,7 @@ class DeviceRun:
         self.row_base = int(row_base)
         self._ws = None
         self.dt_range = None  # (min, max) of the records' dt, when it was reduced on the device
+        self.lmin = None  # shortest event_length, when it is known without a pass over the records (fixed-length runs)
 
     @property
     def pool_len(self) -> int:
@@ -380,7 +381,9 @@ class DeviceRun:
         rows = torch.empty(n * 102, dtype=torch.uint8, device="cuda") if with_rows else None
         _lib.check(lib.wfb_synth_fill(_ptr(pool), _ptr(meta), _ptr(rows), n, n_samples, n_channels, dt_ns, seed, int(record_base), _stream()),
                    "wfb_synth_fill")
-        return cls(meta, pool, n, 0, n_samples, records_rows=rows, pool_base=int(record_base) * n_samples, row_base=int(record_base))
+        run = cls(meta, pool, n, 0, n_samples, records_rows=rows, pool_base=int(record_base) * n_samples, row_base=int(record_base))
+        run.lmin = n_samples
+        return run
 
     def workspace(self):
         torch = _torch()

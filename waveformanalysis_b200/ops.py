@@ -1037,15 +1037,38 @@ def hit_event_table_device(d_rows, n: int, row_bytes: int, group: dict) -> dict:
                             group["dt"], group["abs_start"], group["abs_end"], rows=d_rows, row_bytes=rb)
 
 
+def _sg_tables_by_length(w0: int, poly: int, wcap: int):
+    """SG tables of every effective window a record of length 0..wcap can get (min(w0, L), forced odd, identity when
+    <= poly): (concatenated tables, int32 offset per length, -1 = identity).  The table of the longest records comes
+    first, at offset 0."""
+    eff = np.minimum(w0, np.arange(wcap + 1))
+    eff = eff - (eff % 2 == 0)
+    tables, at = [], {}
+    cursor = 0
+    for w in sorted(set(eff.tolist()), reverse=True):
+        if w <= poly or w <= 0:
+            continue
+        at[w] = cursor
+        tables.append(sg_tables(int(w), poly))
+        cursor += len(tables[-1])
+    lut = np.array([at.get(w, -1) for w in eff.tolist()], dtype=np.int32)
+    return (np.concatenate(tables) if tables else np.zeros(1)), lut
+
+
 def filter_run_device(run: DeviceRun, cfg: dict):
     """wfb_filter_pool on a device-resident run with ONE configuration for every record (benchmarks, multi-GPU shards):
-    returns the float32 pool as a device tensor, nothing crosses PCIe.  ``cfg`` as ``filter_pool``'s ``default``."""
+    returns the float32 pool as a device tensor, nothing crosses PCIe.  ``cfg`` as ``filter_pool``'s ``default``.
+
+    An SG record shorter than the window is filtered with its own effective window min(window, L) (forced odd; left
+    unchanged when that is <= poly): one table per effective window, the record's table offset looked up on the device
+    from its event_length.  A run whose records are all at least the window long (``run.lmin``) uses one table."""
     lib = _lib.load()
     torch = _torch()
     n, L = run.n, max(run.lmax, 1)
     cfgs = (_lib.FilterCfg * 1)()
     tab = np.zeros(1)
     toff = -1
+    d_toff = None
     if cfg["filter_type"] == "BW":
         sos = np.asarray(cfg["sos"], dtype=np.float64)
         zi = sos_zi(sos)
@@ -1058,14 +1081,20 @@ def filter_run_device(run: DeviceRun, cfg: dict):
     else:
         w0, poly = int(cfg["sg_window_size"]), int(cfg["sg_poly_order"])
         cfgs[0].type, cfgs[0].sg_window, cfgs[0].sg_poly = 0, w0, poly
-        w = min(w0, L)
-        w -= (w % 2 == 0)
-        if w > poly and w > 0:
-            tab, toff = sg_tables(int(w), poly), 0
+        wcap = min(w0, L)
+        if run.lmin is not None and run.lmin >= wcap:  # every record gets the same window
+            w = wcap - (wcap % 2 == 0)
+            if w > poly and w > 0:
+                tab, toff = sg_tables(int(w), poly), 0
+        elif n:
+            tab, lut = _sg_tables_by_length(w0, poly, wcap)
+            lens = run.meta[: n * 48].view(n, 48)[:, 24:28].contiguous().view(torch.int32).view(-1)  # wfb_rec_meta.event_length
+            d_toff = upload(lut)[lens.clamp(0, wcap).long()]
     d_cfg = upload(np.frombuffer(bytes(cfgs), dtype=np.uint8).copy())
     d_idx = torch.zeros(max(n, 1), dtype=torch.int32, device="cuda")
     d_tab = upload(np.ascontiguousarray(tab, dtype=np.float64))
-    d_toff = torch.full((max(n, 1),), toff, dtype=torch.int32, device="cuda")
+    if d_toff is None:
+        d_toff = torch.full((max(n, 1),), toff, dtype=torch.int32, device="cuda")
     d_out = torch.empty(run.pool_len + 16, dtype=torch.float32, device="cuda")[: run.pool_len]
     ws = _empty(lib.wfb_filter_workspace_bytes(n, L)) if cfg["filter_type"] == "BW" else None
     _lib.check(lib.wfb_filter_pool(_ptr(run.pool), run.pool_is_f32, run.pool_len, _ptr(run.meta), n, _ptr(d_cfg), 1, _ptr(d_idx), _ptr(d_tab),
