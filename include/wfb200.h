@@ -384,6 +384,16 @@ int wfb_build_records_ragged(const void* samples_dev, int64_t samples_bytes, con
                              const int16_t* channel_dev, const double* baselines_in_dev, int64_t n, int32_t dt_ns,
                              int32_t bl_start, int32_t bl_end, int64_t epoch_ns, void* records_aos_dev, uint16_t* pool_dev,
                              int64_t pool_len, wfb_rec_meta* meta_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+/* The same for a part of a run read from a subset of its row groups (distributed.build_records_sharded): seq_dev[i]
+ * is the global index of row i (its index in the concatenation of ALL groups of the run, in group order) and
+ * becomes the row's record_id; the local rows must follow the groups in group order.  Rows come out ordered by
+ * (timestamp, board, channel, seq).  The workspace is wfb_build_records_v1725_workspace_bytes(n). */
+int wfb_build_records_ragged_seq(const void* samples_dev, int64_t samples_bytes, const int64_t* sample_offset_dev,
+                                 const int32_t* n_samples_dev, const int64_t* timestamp_ps_dev, const int16_t* board_dev,
+                                 const int16_t* channel_dev, const double* baselines_in_dev, const int64_t* seq_dev, int64_t n,
+                                 int32_t dt_ns, int32_t bl_start, int32_t bl_end, int64_t epoch_ns, void* records_aos_dev,
+                                 uint16_t* pool_dev, int64_t pool_len, wfb_rec_meta* meta_dev, void* workspace_dev,
+                                 size_t workspace_bytes, void* stream);
 
 /* `hit` = scipy.signal.find_peaks per record (core/plugins/builtin/cpu/peak_finding.py:213-565
  * HitFinderPlugin._compute_peaks / _find_peaks_in_waveform / _calculate_peak_height).

@@ -20,6 +20,12 @@ rate against its algorithmic bytes (4 L + 252 per record), the peak device memor
 with --verify 1 rank 0 rebuilds all files on one GPU and checks records, pool, features, hits, merged rows and event
 ids byte for byte.
 
+--source raw does the same from raw digitizer rows, as a rank gets them from the reference's format_reader: every rank
+generates its --groups-per-rank per-channel groups (group g seeded by g alone, board g // 16, channel g % 16, --samples
+per row, or 3/4 of that in odd groups with --mixed-widths; every group spans the same time range) and builds its time
+shard with ``distributed.build_records_sharded``.  It reports the same figures; with --verify 1 rank 0 rebuilds all
+groups with ops.build_records (one width) or ops.build_records_ragged (several) and checks the same outputs.
+
 --events adds the df -> df_events -> df_paired leg on the same shards: ``distributed.df_sharded`` on the rank's feature
 rows, then ``distributed.events_sharded`` (time_window_ns = pair window = 100, 2 paired channels).  It reports the time of
 every stage (each ended by a device synchronize), gathered_bytes, the event counts and the peak device memory of the leg;
@@ -50,8 +56,10 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--records-per-rank", type=int, default=1_000_000)
 ap.add_argument("--verify", type=int, default=1)
 ap.add_argument("--zone-rows", type=int, default=4096)
-ap.add_argument("--source", choices=("synth", "v1725"), default="synth")
+ap.add_argument("--source", choices=("synth", "v1725", "raw"), default="synth")
 ap.add_argument("--files-per-rank", type=int, default=2)
+ap.add_argument("--groups-per-rank", type=int, default=2)
+ap.add_argument("--mixed-widths", action="store_true", help="--source raw: odd groups have 3/4 of --samples per row")
 ap.add_argument("--samples", type=int, default=800)
 ap.add_argument("--events", action="store_true", help="also run the sharded df -> df_events -> df_paired leg")
 ap.add_argument("--hit-events", action="store_true", help="also build the sharded hit_grouped event table")
@@ -61,7 +69,7 @@ D.init_process_group("nccl")
 rank, ws, local = D.world()
 torch.cuda.set_device(local)
 n, L, NCH, SEED = args.records_per_rank, args.samples, 16, 4242
-DT_V1725 = 4
+DT_INGEST = 4
 THR, WINDOW, GAP = 15.0, 100.0, 50.0
 
 
@@ -106,10 +114,52 @@ def v1725_name(i: int) -> str:
     return f"run_b{i}_seg0.bin"
 
 
+def raw_group(g: int, m: int):
+    """Raw rows of group g (timestamps_ps, boards, channels, int16 samples): one channel over the whole run; seeded by g."""
+    rng = np.random.default_rng(2000 + g)
+    width = L - L // 4 if args.mixed_widths and g % 2 else L
+    step = rng.integers(1, 4 * L, m)
+    step[::5] = 0  # rows sharing a timestamp
+    ts = (np.cumsum(step) + rng.integers(0, 3, m)) * (DT_INGEST * 1000)
+    block = (8000 + rng.integers(-4, 5, 1 << 20)).astype(np.int16)
+    for k in range(0, len(block) - 40, 997):  # negative pulses
+        block[k:k + 12] -= 150
+    windows = np.lib.stride_tricks.sliding_window_view(block, width)
+    samples = np.empty((m, width), dtype=np.int16)
+    for r0 in range(0, m, 1 << 15):
+        r1 = min(r0 + (1 << 15), m)
+        samples[r0:r1] = windows[rng.integers(0, len(windows), r1 - r0)]
+    return ts.astype(np.int64), np.full(m, g // NCH, np.int16), np.full(m, g % NCH, np.int16), samples
+
+
+def report_ingest(title: str, wall: float, peak: int):
+    """Print every rank's ingest line on rank 0: stage times, exchange, merge rate against its algorithmic bytes (read and
+    write of the samples and the row, write of the 48 B meta), peak memory, GPU.  Returns (run, n, n_total)."""
+    import subprocess
+
+    run = ingest["run"]
+    tm = ingest["timings"]
+    n_all = ingest["n_total"]
+    per_record = 4 * run.pool_len / max(run.n, 1) + 252
+    gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", str(local)],
+                         capture_output=True, text=True).stdout.strip()
+    line = (f"rank {rank}: records {run.n} (base {ingest['record_base']}) | " +
+            " ".join(f"{k} {1e3 * v:.1f} ms" for k, v in tm.items()) +
+            f" | exchange {ingest['exchange_bytes'] / 1e9:.3f} GB received, {ingest['exchange_bytes'] / max(tm['exchange'], 1e-9) / 1e9:.1f} GB/s"
+            f" | merge {per_record * run.n / max(tm['merge'], 1e-9) / 1e9:.0f} GB/s of {per_record:.0f} B/record"
+            f" | ingest wall {1e3 * wall:.1f} ms, {n_all / wall / 1e6:.1f} M records/s run-wide"
+            f" | peak device memory {peak / 1e9:.2f} GB ({peak / max(2 * run.pool_len, 1):.2f} x the shard's sample bytes) | {gpu}")
+    lines = D.gather_rows(np.frombuffer(line.encode().ljust(1024)[:1024], dtype="S1024")) if ws > 1 else [line.encode()]
+    if rank == 0:
+        print(f"{title} records={n_all} samples/record={L}")
+        for ln in lines:
+            print("  " + ln.decode().strip())
+    return run, run.n, n_all
+
+
 ingest = None
 if args.source == "v1725":
     import shutil
-    import subprocess
     import tempfile
 
     F = ws * args.files_per_rank
@@ -123,29 +173,27 @@ if args.source == "v1725":
     if ws > 1:
         dist.barrier()
     tw = time.perf_counter()
-    ingest = D.build_records_sharded_v1725(paths, dt_ns=DT_V1725, mine=mine)
+    ingest = D.build_records_sharded_v1725(paths, dt_ns=DT_INGEST, mine=mine)
     torch.cuda.synchronize()
     wall = time.perf_counter() - tw
     peak = torch.cuda.max_memory_allocated()
     shutil.rmtree(tmp, ignore_errors=True)
-    run = ingest["run"]
-    n = run.n
-    tm = ingest["timings"]
-    n_all = ingest["n_total"]
-    merge_bytes = (4 * L + 252) * run.n
-    gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", str(local)],
-                         capture_output=True, text=True).stdout.strip()
-    line = (f"rank {rank}: records {run.n} (base {ingest['record_base']}) | " +
-            " ".join(f"{k} {1e3 * v:.1f} ms" for k, v in tm.items()) +
-            f" | exchange {ingest['exchange_bytes'] / 1e9:.3f} GB received, {ingest['exchange_bytes'] / max(tm['exchange'], 1e-9) / 1e9:.1f} GB/s"
-            f" | merge {merge_bytes / max(tm['merge'], 1e-9) / 1e9:.0f} GB/s of {4 * L + 252} B/record"
-            f" | ingest wall {1e3 * wall:.1f} ms, {n_all / wall / 1e6:.1f} M records/s run-wide"
-            f" | peak device memory {peak / 1e9:.2f} GB ({peak / max(2 * run.pool_len, 1):.2f} x the shard's sample bytes) | {gpu}")
-    lines = D.gather_rows(np.frombuffer(line.encode().ljust(1024)[:1024], dtype="S1024")) if ws > 1 else [line.encode()]
-    if rank == 0:
-        print(f"v1725 ingest: world={ws} files={F} records={n_all} samples/record={L}")
-        for ln in lines:
-            print("  " + ln.decode().strip())
+    run, n, n_all = report_ingest(f"v1725 ingest: world={ws} files={F}", wall, peak)
+elif args.source == "raw":
+    G = ws * args.groups_per_rank
+    rows_per_group = max(n // args.groups_per_rank, 1)
+    groups = {g: raw_group(g, rows_per_group) for g in range(rank * args.groups_per_rank, (rank + 1) * args.groups_per_rank)}
+    torch.cuda.reset_peak_memory_stats()
+    if ws > 1:
+        dist.barrier()
+    tw = time.perf_counter()
+    ingest = D.build_records_sharded(groups, n_groups=G, dt_ns=DT_INGEST)
+    torch.cuda.synchronize()
+    wall = time.perf_counter() - tw
+    peak = torch.cuda.max_memory_allocated()
+    del groups
+    widths = f"{L} and {L - L // 4}" if args.mixed_widths else f"{L}"
+    run, n, n_all = report_ingest(f"raw ingest: world={ws} groups={G} widths={widths}", wall, peak)
 else:
     run = engine.DeviceRun.synth(n, L, NCH, seed=SEED, record_base=rank * n)
 res, total = fused(run)
@@ -154,7 +202,7 @@ if ws > 1:
 torch.cuda.synchronize()
 t0 = time.perf_counter()
 sh = D.merge_group_sharded((res["hits"][: total * 60], total), D.DeviceRows(THRESHOLD_HIT_DTYPE), time_window_ns=WINDOW, merge_gap_ns=GAP,
-                           span_ns=(run.lmax * DT_V1725 if ingest is not None else L * 2.0), zone_rows=args.zone_rows)
+                           span_ns=(run.lmax * DT_INGEST if ingest is not None else L * 2.0), zone_rows=args.zone_rows)
 torch.cuda.synchronize()
 if ws > 1:
     dist.barrier()
@@ -310,8 +358,17 @@ if args.verify:
         del run, res, sh
         torch.cuda.empty_cache()
         if ingest is not None:
-            want_rec, want_pool = ops.build_records_from_v1725([v1725_file(i, ev_per_file) for i in range(F)],
-                                                               [v1725_name(i) for i in range(F)], DT_V1725)
+            if args.source == "v1725":
+                want_rec, want_pool = ops.build_records_from_v1725([v1725_file(i, ev_per_file) for i in range(F)],
+                                                                   [v1725_name(i) for i in range(F)], DT_INGEST)
+            else:
+                gs = [raw_group(g, rows_per_group) for g in range(G)]
+                ts, b, c = (np.concatenate([x[k] for x in gs]) for k in range(3))
+                if len({x[3].shape[1] for x in gs}) > 1:
+                    want_rec, want_pool = ops.build_records_ragged(ts, b, c, [x[3] for x in gs], dt_ns=DT_INGEST)
+                else:
+                    want_rec, want_pool = ops.build_records(ts, b, c, np.vstack([x[3] for x in gs]), dt_ns=DT_INGEST)
+                del gs, ts, b, c
             assert recs_all.tobytes() == want_rec.tobytes(), "records differ"
             assert np.array_equal(pool_all, want_pool), "wave_pool differs"
             full = engine.DeviceRun.from_host(want_rec, want_pool)

@@ -151,6 +151,8 @@ PROTOTYPES = {
     "wfb_release_cache": (C.c_int, []),
     "wfb_group_abs_windows": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _dbl, _vp, _vp, _vp, _vp, _sz, _vp]),
     "wfb_build_records_ragged": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _i64, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
+    "wfb_build_records_ragged_seq": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _i64, _vp, _vp, _i64, _vp, _vp,
+                                               _sz, _vp]),
     "wfb_find_peaks_workspace_bytes": (_sz, [_i64]),
     "wfb_find_peaks": (C.c_int, [_vp, _i64, _vp, _i64, C.POINTER(PeakParams), _vp, _i64, _vp, _vp, _vp, _sz, _vp]),
     "wfb_v1725_scan_host": (C.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(_i64), C.POINTER(_i64)]),

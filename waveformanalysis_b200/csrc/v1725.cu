@@ -239,6 +239,19 @@ extern "C" int wfb_build_records_ragged(const void* samples_dev, int64_t samples
                                 static_cast<cudaStream_t>(stream), "wfb_build_records_ragged");
 }
 
+extern "C" int wfb_build_records_ragged_seq(const void* samples_dev, int64_t samples_bytes, const int64_t* sample_offset_dev,
+                                            const int32_t* n_samples_dev, const int64_t* timestamp_ps_dev, const int16_t* board_dev,
+                                            const int16_t* channel_dev, const double* baselines_in_dev, const int64_t* seq_dev, int64_t n,
+                                            int32_t dt_ns, int32_t bl_start, int32_t bl_end, int64_t epoch_ns, void* records_aos_dev,
+                                            uint16_t* pool_dev, int64_t pool_len, wfb_rec_meta* meta_dev, void* workspace_dev,
+                                            size_t workspace_bytes, void* stream) {
+    WFB_REQUIRE(n == 0 || seq_dev != nullptr, "wfb_build_records_ragged_seq: NULL seq");
+    return build_records_ragged(static_cast<const uint8_t*>(samples_dev), samples_bytes, sample_offset_dev, n_samples_dev, timestamp_ps_dev, 1,
+                                board_dev, channel_dev, nullptr, baselines_in_dev, nullptr, seq_dev, n, dt_ns, bl_start, bl_end, epoch_ns,
+                                records_aos_dev, pool_dev, pool_len, meta_dev, workspace_dev, workspace_bytes,
+                                static_cast<cudaStream_t>(stream), "wfb_build_records_ragged_seq");
+}
+
 static int build_v1725(const uint8_t* blob_dev, int64_t blob_bytes, const int64_t* payload_offset_dev, const int32_t* n_samples_dev,
                        const int64_t* timestamp_dev, const int16_t* board_dev, const int16_t* channel_dev, const uint16_t* baseline_dev,
                        const uint8_t* trunc_dev, const int64_t* seq_dev, int64_t n, int32_t dt_ns, void* records_aos_dev, uint16_t* pool_dev,

@@ -513,6 +513,10 @@ def assemble_merged(merged_all: np.ndarray, event_of_merged_all: np.ndarray):
 #   5. one all-gather of the received counts gives the shard's global record and sample bases;
 #   6. the received runs (sorted, in source-rank order) are merged by rank and renumbered for the shard's place.
 # Every rank sends (P - 1) / P of its rows and samples on average: (P - 1) / P x (2 L + 102) bytes per record.
+#
+# Raw rows (build_records_sharded: VX2730 CSV groups, anything a format_reader parses, raw_arrays) take the same
+# steps 2-6.  Their single-GPU order is the same lexsort over the groups concatenated in group-index order, and both
+# single-GPU builders break ties by input position, so seq = a row's index in that concatenation gives the same key.
 
 SPLITTER_SAMPLES_PER_RANK = 256  # s = SPLITTER_SAMPLES_PER_RANK x world_size samples per rank
 
@@ -622,11 +626,12 @@ def _exchange(rows, pool, row_counts, sample_counts, backend):
 
 
 class HostRecords:
-    """Backend for the records of a rank held as numpy arrays (CPU tests over gloo): the oracle's scan, the host key
-    order for the local sort and the merge."""
+    """Backend for the records of a rank held as numpy arrays (CPU tests over gloo): the oracle's scan (V1725 files)
+    and baseline mean (raw rows), the host key order for the local sort and the merge."""
 
-    def __init__(self, scan_fn):
+    def __init__(self, scan_fn=None, baseline_fn=None):
         self.scan_fn = scan_fn
+        self.baseline_fn = baseline_fn
 
     def sync(self):
         pass
@@ -666,6 +671,36 @@ class HostRecords:
         rec["wave_offset"] = np.cumsum(lens) - lens
         rec["time"] = rec["timestamp"] // 1000
         return rec, np.concatenate([waves[i] for i in order.tolist()]).astype(np.uint16, copy=False)
+
+    def upload_raw(self, ts, board, channel, blocks):
+        return ts, board, channel, blocks
+
+    def build_raw(self, up, dt_ns: int, baseline_window, epoch_ns, seq: np.ndarray):
+        """The oracle's build_records over raw rows of any widths, ordered by (timestamp, board, channel, seq)."""
+        from .dtypes import RECORDS_DTYPE
+
+        ts, board, channel, blocks = up
+        n = len(seq)
+        rec = np.zeros(n, dtype=RECORDS_DTYPE)
+        if n == 0:
+            return rec, np.zeros(0, dtype=np.uint16)
+        lens = np.concatenate([np.full(len(b), b.shape[1], dtype=np.int64) for b in blocks])
+        baseline = np.concatenate([self.baseline_fn(b.view(np.int16), *baseline_window) for b in blocks])
+        samples = np.concatenate([b.reshape(-1).view(np.uint16) for b in blocks])
+        order = key_order(np.stack([ts, board.astype(np.int64), channel.astype(np.int64), seq], axis=1))
+        rec["timestamp"], rec["board"], rec["channel"] = ts[order], board[order], channel[order]
+        rec["baseline"] = baseline[order]
+        rec["baseline_upstream"] = np.nan
+        rec["polarity"] = "unknown"
+        rec["record_id"] = seq[order]
+        rec["dt"] = int(dt_ns)
+        out_lens = lens[order]
+        out_start = np.cumsum(out_lens) - out_lens
+        rec["event_length"] = out_lens
+        rec["wave_offset"] = out_start
+        rec["time"] = rec["timestamp"] // 1000 + (0 if epoch_ns is None else int(epoch_ns))
+        in_start = (np.cumsum(lens) - lens)[order]
+        return rec, samples[np.arange(int(out_lens.sum()), dtype=np.int64) + np.repeat(in_start - out_start, out_lens)]
 
     def count(self, local):
         return len(local[0])
@@ -742,6 +777,17 @@ class DeviceRecords:
         from . import ops
 
         rows, pool, _ = ops.build_records_v1725_device(up, dt_ns, seq=seq)
+        return rows, pool, up["n"]
+
+    def upload_raw(self, ts, board, channel, blocks):
+        from . import ops
+
+        return ops.raw_upload(ts, board, channel, blocks)
+
+    def build_raw(self, up, dt_ns: int, baseline_window, epoch_ns, seq: np.ndarray):
+        from . import ops
+
+        rows, pool, _ = ops.build_records_ragged_device(up, dt_ns=dt_ns, baseline_window=baseline_window, epoch_ns=epoch_ns, seq=seq)
         return rows, pool, up["n"]
 
     def count(self, local):
@@ -878,10 +924,22 @@ def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None) -
     backend.sync()
     T["h2d"] = time.perf_counter() - t
     t = time.perf_counter()
-    local = backend.build(up, int(dt_ns), seq)
+    built = [backend.build(up, int(dt_ns), seq)]
     del up  # the stream bytes
     backend.sync()
     T["build"] = time.perf_counter() - t
+    return _time_shard(built, backend, T)
+
+
+def _time_shard(built: list, backend, T: dict) -> dict:
+    """Stages 2-6 of the distributed time sort on a rank's locally built rows (record_id = global seq, sorted by
+    (timestamp, board, channel, seq)): splitters, split points, exchange, global bases, merge, run-wide lmax.
+    ``built`` holds the local build and is emptied, so that the rows are freed once they are sent; ``T`` gets the
+    stage timings.  Returns the dict of build_records_sharded_v1725."""
+    import time
+
+    _, rank, P = _dist()
+    local = built.pop()
 
     # 2. splitters, 3. split points
     t = time.perf_counter()
@@ -918,6 +976,98 @@ def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None) -
     lmax = _allreduce_max(backend.lmax(shard))
     return dict(run=backend.run(shard, lmax, record_base, pool_base), record_base=record_base, pool_base=pool_base,
                 n_total=int(bases[:, 0].sum()), records_per_rank=bases[:, 0].copy(), exchange_bytes=exchange_bytes, timings=T)
+
+
+def _check_group(g: int, cols) -> tuple:
+    """One raw row group -> (timestamps_ps int64, boards int16, channels int16, samples 2-D int16 / uint16); ValueError
+    when the columns do not describe the same rows."""
+    try:
+        ts, board, channel, samples = cols
+    except (TypeError, ValueError):
+        raise ValueError(f"group {g}: expected (timestamps_ps, boards, channels, samples)") from None
+    samples = np.asarray(samples)
+    if samples.ndim != 2 or samples.dtype not in (np.int16, np.uint16):
+        raise ValueError(f"group {g}: samples must be a 2-D int16 array, got {samples.dtype} {samples.shape}")
+    out = (np.asarray(ts, dtype=np.int64).reshape(-1), np.asarray(board, dtype=np.int16).reshape(-1),
+           np.asarray(channel, dtype=np.int16).reshape(-1), samples)
+    if not len(out[0]) == len(out[1]) == len(out[2]) == len(samples):
+        raise ValueError(f"group {g}: {len(out[0])} timestamps, {len(out[1])} boards, {len(out[2])} channels and {len(samples)} "
+                         "sample rows")
+    return out
+
+
+def build_records_sharded(groups, *, n_groups: int, dt_ns: int, baseline_window=(0, 40), epoch_ns: int | None = None,
+                          backend=None) -> dict:
+    """This rank's time shard of a run made of ``n_groups`` groups of raw rows, without any process holding the whole
+    run: the result of ``ops.build_records`` / ``ops.build_records_ragged`` (as ``plugins.records.build_bundle`` picks
+    them) on all groups concatenated in group-index order.
+
+    ``groups`` maps a global group index to ``(timestamps_ps, boards, channels, samples)`` (``samples`` a 2-D int16
+    array, one row per waveform) for the groups THIS rank read, e.g. one per-channel file group parsed by the
+    reference's ``format_reader``.  Groups may have different widths.  A group index outside [0, n_groups), a group
+    claimed by no rank or by two ranks, a group whose columns differ in length, and ``n_groups``, ``dt_ns``,
+    ``baseline_window`` or ``epoch_ns`` differing between ranks raise ValueError on every rank.
+
+    Each row's seq is its index in the concatenation of all groups; every rank builds its own rows with record_id =
+    seq (``wfb_build_records_ragged_seq``), which orders them by (timestamp, board, channel, seq), the single-GPU
+    order, and the distributed time sort of build_records_sharded_v1725 does the rest.  Returns the same dict;
+    ``timings`` has h2d, build, splitters, exchange and merge."""
+    import time
+
+    backend = backend if backend is not None else DeviceRecords()
+    T: dict = {}
+    err = None
+    own: list = []
+    cols: list = []
+    params = np.zeros(6, dtype=np.int64)
+    try:
+        bl0, bl1 = (int(x) for x in baseline_window)
+        params[:] = [int(n_groups), int(dt_ns), bl0, bl1, epoch_ns is None, 0 if epoch_ns is None else int(epoch_ns)]
+        if int(dt_ns) <= 0 or int(n_groups) < 0:
+            raise ValueError(f"dt_ns must be positive and n_groups non-negative, got {dt_ns} and {n_groups}")
+        items = sorted((int(g), c) for g, c in dict(groups).items())
+        own = [g for g, _ in items]
+        cols = [_check_group(g, c) for g, c in items]
+    except (TypeError, ValueError) as e:
+        err, own, cols = e, [], []
+
+    # parameters and local errors first (fixed size, so a rank with different arguments cannot stall the gather)
+    table = _allgather_i64(np.r_[int(err is not None), params])
+    if table[:, 0].any():
+        if err is not None:
+            raise err
+        raise ValueError(f"ranks {np.flatnonzero(table[:, 0]).tolist()} were given malformed row groups or arguments")
+    if np.any(table[:, 1:] != table[:1, 1:]):
+        raise ValueError("n_groups, dt_ns, baseline_window and epoch_ns must be the same on every rank")
+
+    # ownership, checked on the gathered claims so that every rank raises
+    G = int(n_groups)
+    g = allgather_columns({"group": np.asarray(own, dtype=np.int64), "rows": np.array([len(c[0]) for c in cols], dtype=np.int64)})
+    claims = g["group"]
+    inside = (claims >= 0) & (claims < G)
+    claimed = np.bincount(claims[inside], minlength=G)
+    if not inside.all() or np.any(claimed != 1):
+        bad = sorted(set(np.flatnonzero(claimed != 1).tolist()) | set(claims[~inside].tolist()))
+        raise ValueError(f"every group must be read by exactly one rank: groups {bad[:10]} are claimed by none, by several ranks "
+                         f"or are outside [0, {G})")
+    counts = np.zeros(G, dtype=np.int64)
+    counts[claims] = g["rows"]
+    seq_base = np.cumsum(counts) - counts
+    seq = np.concatenate([seq_base[f] + np.arange(counts[f], dtype=np.int64) for f in own] or [np.zeros(0, np.int64)])
+
+    # 1. local build (the rank's groups in increasing index: its input order is the global order restricted to them)
+    t = time.perf_counter()
+    ts, board, channel = (np.concatenate([c[k] for c in cols] or [np.zeros(0, dt)]) for k, dt in enumerate((np.int64, np.int16, np.int16)))
+    up = backend.upload_raw(ts, board, channel, [c[3] for c in cols])
+    del cols, ts, board, channel
+    backend.sync()
+    T["h2d"] = time.perf_counter() - t
+    t = time.perf_counter()
+    built = [backend.build_raw(up, int(dt_ns), (int(params[2]), int(params[3])), epoch_ns, seq)]
+    del up
+    backend.sync()
+    T["build"] = time.perf_counter() - t
+    return _time_shard(built, backend, T)
 
 
 # ------------------------------------------------------------------------------------------------

@@ -43,16 +43,26 @@ def build_records_ragged(timestamps_ps, boards, channels, sample_blocks, *, dt_n
                          epoch_ns: int | None = None):
     """Like build_records for parts of different waveform widths: ``sample_blocks`` is a list of int16
     matrices (n_k, L_k) whose rows follow each other in the order of the per-record columns."""
-    lib = _lib.load()
+    up = raw_upload(timestamps_ps, boards, channels, sample_blocks, baselines=baselines)
+    n = up["n"]
+    if n == 0:
+        return np.zeros(0, dtype=RECORDS_DTYPE), np.zeros(0, dtype=np.uint16)
+    rows, pool, _ = build_records_ragged_device(up, dt_ns=dt_ns, baseline_window=baseline_window, epoch_ns=epoch_ns)
+    rec = rows[: n * 102].cpu().numpy().view(RECORDS_DTYPE)
+    return rec, pool.cpu().numpy().view(np.uint16)
+
+
+def raw_upload(timestamps_ps, boards, channels, sample_blocks, *, baselines=None) -> dict:
+    """Raw rows on the device for build_records_ragged_device: the int16 / uint16 matrices of ``sample_blocks`` at
+    16-byte aligned bases of ONE device buffer, every row's byte offset and length, and the per-row columns (which
+    follow the blocks' rows in order)."""
     torch = _torch()
     blocks = [np.ascontiguousarray(b) for b in sample_blocks]
     for b in blocks:
         if b.dtype not in (np.int16, np.uint16) or b.ndim != 2:
             raise ValueError(f"sample blocks must be 2-D int16 arrays, got {b.dtype} {b.shape}")
     n = sum(len(b) for b in blocks)
-    if n == 0:
-        return np.zeros(0, dtype=RECORDS_DTYPE), np.zeros(0, dtype=np.uint16)
-    offs, lens, cursor = [], [], 0
+    offs, lens, cursor = [np.zeros(0, np.int64)], [np.zeros(0, np.int32)], 0
     for b in blocks:
         offs.append(cursor + np.arange(len(b), dtype=np.int64) * (b.shape[1] * 2))
         lens.append(np.full(len(b), b.shape[1], dtype=np.int32))
@@ -63,21 +73,45 @@ def build_records_ragged(timestamps_ps, boards, channels, sample_blocks, *, dt_n
         if b.nbytes:
             d_blob[base:base + b.nbytes].copy_(upload(b.reshape(-1).view(np.uint8)))
         base += (b.nbytes + 15) & ~15
-    off, ln = np.concatenate(offs), np.concatenate(lens)
-    total = int(ln.astype(np.int64).sum())
-    d_off, d_len = _dev(off), _dev(ln)
-    d_ts = _dev(np.asarray(timestamps_ps, dtype=np.int64))
-    d_b = _dev(np.asarray(boards, dtype=np.int16))
-    d_c = _dev(np.asarray(channels, dtype=np.int16))
-    d_bl = _dev(np.asarray(baselines, dtype=np.float64)) if baselines is not None else None
+    ln = np.concatenate(lens)
+    cols = {"timestamp": (timestamps_ps, np.int64), "board": (boards, np.int16), "channel": (channels, np.int16)}
+    if baselines is not None:
+        cols["baseline"] = (baselines, np.float64)
+    up = {k: np.asarray(v, dtype=t).reshape(-1) for k, (v, t) in cols.items()}
+    for k, v in up.items():
+        if len(v) != n:
+            raise ValueError(f"{k} has {len(v)} entries for {n} sample rows")
+    up = {k: _dev(v) for k, v in up.items()}
+    up.update(blob=d_blob, blob_bytes=cursor, sample_offset=_dev(np.concatenate(offs)), n_samples=_dev(ln), n=n,
+              total=int(ln.astype(np.int64).sum()))
+    return up
+
+
+def build_records_ragged_device(up: dict, *, dt_ns: int, baseline_window=(0, 40), epoch_ns: int | None = None,
+                                seq: np.ndarray | None = None, meta: bool = False):
+    """wfb_build_records_ragged (``seq`` given: wfb_build_records_ragged_seq, record_id = seq) on the output of
+    raw_upload -> device (rows uint8 [n * 102], pool int16 [total] with a 16-sample tail, meta uint8 [n * 48] or None)."""
+    lib = _lib.load()
+    torch = _torch()
+    n, total = up["n"], up["total"]
     rows = _empty(n * 102)
     pool = torch.empty(total + 16, dtype=torch.int16, device="cuda")[:total]
+    d_meta = torch.empty(max(n, 1) * 48, dtype=torch.uint8, device="cuda") if meta else None
+    if n == 0:
+        return rows, pool, d_meta
     ws = _empty(lib.wfb_build_records_v1725_workspace_bytes(n))
-    _lib.check(lib.wfb_build_records_ragged(_ptr(d_blob), cursor, _ptr(d_off), _ptr(d_len), _ptr(d_ts), _ptr(d_b), _ptr(d_c), _ptr(d_bl), n,
-                                            int(dt_ns), int(baseline_window[0]), int(baseline_window[1]), int(epoch_ns or 0), _ptr(rows),
-                                            _ptr(pool), total, C.c_void_p(0), _ptr(ws), ws.numel(), _stream()), "wfb_build_records_ragged")
-    rec = rows[: n * 102].cpu().numpy().view(RECORDS_DTYPE)
-    return rec, pool.cpu().numpy().view(np.uint16)
+    cols = (_ptr(up["blob"]), up["blob_bytes"], _ptr(up["sample_offset"]), _ptr(up["n_samples"]), _ptr(up["timestamp"]), _ptr(up["board"]),
+            _ptr(up["channel"]), _ptr(up.get("baseline")))
+    tail = (n, int(dt_ns), int(baseline_window[0]), int(baseline_window[1]), int(epoch_ns or 0), _ptr(rows), _ptr(pool), total, _ptr(d_meta),
+            _ptr(ws), ws.numel(), _stream())
+    if seq is None:
+        _lib.check(lib.wfb_build_records_ragged(*cols, *tail), "wfb_build_records_ragged")
+    else:
+        d_seq = _dev(np.ascontiguousarray(seq, dtype=np.int64))
+        if len(d_seq) != n:
+            raise ValueError(f"seq has {len(d_seq)} entries for {n} rows")
+        _lib.check(lib.wfb_build_records_ragged_seq(*cols, _ptr(d_seq), *tail), "wfb_build_records_ragged_seq")
+    return rows, pool, d_meta
 
 
 
