@@ -335,21 +335,31 @@ __device__ __forceinline__ void blk_stream(const FHArgs& a, const uint16_t* pool
     const int nseg = (nblk + bps - 1) / bps;
     const bool known = r.pol == WFB_POL_POSITIVE || r.pol == WFB_POL_NEGATIVE;
     const float b32 = (float)r.b_feat;
-    int plainA = 0, plainB = 0, plainHa = 0, plainHb = 0;
+    // Block ranges of the record, computed once.  Block B holds 32 samples of the record iff 0 <= 32 B - mis <= len - 32;
+    // the blocks of [f0, f0 + fn0) and [f1, f1 + fn1) also take the straight feature path (whole chunks inside the area
+    // slice, none in the height slice, unknown polarity).  A test is one unsigned compare: in front of a range the
+    // difference wraps above its length.
+    const unsigned whn = (unsigned)max(0, r.len - 31);
+    int f0 = 0, f1 = 0;
+    unsigned fn0 = 0u, fn1 = 0u;
     if (FEAT && r.len > 0 && !known) {
-        const int vlo = mis + max(c0, 1);
-        const int vhi = mis + min(c1, r.len);
-        plainA = (vlo + 7) >> 3;
-        plainB = vhi >> 3;
-        if (p1 > p0) { plainHa = (mis + p0) >> 3; plainHb = (mis + p1 + 7) >> 3; }
+        const int wh0 = (((mis + 7) >> 3) + 3) >> 2, wh1 = (vtotal >> 3) >> 2;  // the blocks of 32 record samples
+        const int lo = max(wh0, (((mis + max(c0, 1) + 7) >> 3) + 3) >> 2);
+        const int hi = min(wh1, ((mis + min(c1, r.len)) >> 3) >> 2);
+        const int ha = (p1 > p0) ? ((mis + p0) >> 3) >> 2 : 0;                // blocks in front of the height slice
+        const int hb = (p1 > p0) ? (((mis + p1 + 7) >> 3) + 3) >> 2 : 0;      // blocks behind it
+        f0 = lo;
+        fn0 = (unsigned)max(0, min(hi, ha) - lo);
+        f1 = max(lo, hb);
+        fn1 = (unsigned)max(0, hi - f1);
     }
-    const int wholeA = (mis + 7) >> 3, wholeB = vtotal >> 3;  // chunks [wholeA, wholeB) hold 8 samples of the record
     const unsigned xm16 = r.positive ? 0xffffu : 0u;
+    const int kfull = r.degen ? -1 : r.kmax;    // a block is FULL <=> its largest key <= kfull (never with a negative threshold)
     // hit state of the lane
     bool open = false;                          // the last sample of the previous block is above threshold
     unsigned fa_key = 0xffffffffu, fa_sum = 0u; // FULL blocks since the lane's last item
     unsigned hprev = 0u;                        // last word of the previous block
-    unsigned* myslot = nullptr;                 // the item pushed in the previous step (waits for its next word)
+    int myslot = -1;                            // word 17 of the item pushed in the previous step (waits for its next word)
     int qn_c = 0, qn_i = 0, qh = 0;             // complete / incomplete items, ring head (warp-uniform)
 
     auto issue = [&](int s) {
@@ -374,17 +384,24 @@ __device__ __forceinline__ void blk_stream(const FHArgs& a, const uint16_t* pool
         __syncwarp();
         if (bytes) tma_bulk_g2s(ring.slot + b * ring.buf_stride, pool + (r.off - mis) + (long long)clo * 8, bytes, &ring.bars[b]);
     };
+    // |x[i] - x[i-1]| of the four words of chunk q, packed, given the word in front of it
+    auto absdiff4 = [](const uint4& q, unsigned pw, unsigned& e0, unsigned& e1, unsigned& e2, unsigned& e3) {
+        const unsigned g0 = __funnelshift_r(pw, q.x, 16), g1 = __funnelshift_r(q.x, q.y, 16);
+        const unsigned g2 = __funnelshift_r(q.y, q.z, 16), g3 = __funnelshift_r(q.z, q.w, 16);
+        e0 = __vmaxu2(q.x, g0) - __vminu2(q.x, g0);
+        e1 = __vmaxu2(q.y, g1) - __vminu2(q.y, g1);
+        e2 = __vmaxu2(q.z, g2) - __vminu2(q.z, g2);
+        e3 = __vmaxu2(q.w, g3) - __vminu2(q.w, g3);
+    };
     auto feat_plain = [&](const uint4& q, unsigned csum) {
-        unsigned f0 = __funnelshift_r(fs.prev_w, q.x, 16), f1 = __funnelshift_r(q.x, q.y, 16);
-        unsigned f2 = __funnelshift_r(q.y, q.z, 16), f3 = __funnelshift_r(q.z, q.w, 16);
-        unsigned e0 = __vmaxu2(q.x, f0) - __vminu2(q.x, f0), e1 = __vmaxu2(q.y, f1) - __vminu2(q.y, f1);
-        unsigned e2 = __vmaxu2(q.z, f2) - __vminu2(q.z, f2), e3 = __vmaxu2(q.w, f3) - __vminu2(q.w, f3);
+        unsigned e0, e1, e2, e3;
+        absdiff4(q, fs.prev_w, e0, e1, e2, e3);
         fs.pdiff = __vimax3_u16x2(fs.pdiff, __vmaxu2(e0, e1), __vmaxu2(e2, e3));
         fs.isum32 += csum;
         fs.prev_w = q.w;
     };
-    auto csum4 = [](const uint4& q) {
-        unsigned cs = __dp2a_lo(q.x, 0x0101u, 0u);
+    auto csum4 = [](const uint4& q, unsigned cs = 0u) {  // cs + the eight samples of q
+        cs = __dp2a_lo(q.x, 0x0101u, cs);
         cs = __dp2a_lo(q.y, 0x0101u, cs);
         cs = __dp2a_lo(q.z, 0x0101u, cs);
         return __dp2a_lo(q.w, 0x0101u, cs);
@@ -396,14 +413,13 @@ __device__ __forceinline__ void blk_stream(const FHArgs& a, const uint16_t* pool
         const int lo = max(mis - v0, 0), hi = min(vtotal - v0, 8);
         const int i0 = v0 - mis;
         const bool whole = lo == 0 && hi == 8;
-        if (vc >= plainA && vc < plainB && (vc < plainHa || vc >= plainHb)) {
+        // inside the area slice and the record (not its first sample), outside the height slice, unknown polarity
+        const bool plain = !known && i0 >= max(c0, 1) && i0 + 8 <= min(c1, r.len) && (p1 <= p0 || i0 + 8 <= p0 || i0 >= p1);
+        if (plain) {
             feat_plain(q, csum4(q));
         } else if (whole) {
-            const unsigned pw = (i0 > 0) ? fs.prev_w : (q.x << 16);
-            unsigned f0 = __funnelshift_r(pw, q.x, 16), f1 = __funnelshift_r(q.x, q.y, 16);
-            unsigned f2 = __funnelshift_r(q.y, q.z, 16), f3 = __funnelshift_r(q.z, q.w, 16);
-            unsigned e0 = __vmaxu2(q.x, f0) - __vminu2(q.x, f0), e1 = __vmaxu2(q.y, f1) - __vminu2(q.y, f1);
-            unsigned e2 = __vmaxu2(q.z, f2) - __vminu2(q.z, f2), e3 = __vmaxu2(q.w, f3) - __vminu2(q.w, f3);
+            unsigned e0, e1, e2, e3;
+            absdiff4(q, (i0 > 0) ? fs.prev_w : (q.x << 16), e0, e1, e2, e3);
             fs.pdiff = __vmaxu2(fs.pdiff, __vmaxu2(__vmaxu2(e0, e1), __vmaxu2(e2, e3)));
             const int jlo = max(0, p0 - i0), jhi = min(8, p1 - i0);
             if (jhi > jlo) {
@@ -464,54 +480,35 @@ __device__ __forceinline__ void blk_stream(const FHArgs& a, const uint16_t* pool
         }
         const uint8_t* buf = ring.slot + b * ring.buf_stride;
         const int tend = drain ? 1 : min(bps, nblk - s * bps);
+        const int qmin = drain ? 1 : 32;  // a round runs when 32 complete items wait; the drain takes what is left
+        if (drain) myslot = -1;           // the items of the last block lie behind their records: no next word
         for (int t = 0; t < tend; ++t) {
-            const int vc0 = s * sc + 4 * t;  // first chunk of the block
-            const int B = vc0 >> 2;
-            // the items pushed one step ago get the first word of their next block (the items of the last step lie
-            // behind their records and need none); a round runs when 32 complete items wait
-            if (myslot != nullptr && !drain) {
-                myslot[17] = *reinterpret_cast<const unsigned*>(buf + t * 64) ^ (SGN ? 0x80008000u : 0u);
-                myslot = nullptr;
-            }
+            const int B = s * bps + t;
+            const uint4* blk = reinterpret_cast<const uint4*>(buf + t * 64);
+            // the items pushed one step ago get the first word of their next block
+            if (myslot >= 0) bq[myslot] = reinterpret_cast<const unsigned*>(blk)[0] ^ (SGN ? 0x80008000u : 0u);
+            myslot = -1;
             qn_c += qn_i;
-            qn_i = 0;
-            while (qn_c >= 32 || (drain && qn_c > 0)) {
+            while (qn_c >= qmin) {
                 const int take = min(qn_c, 32);
                 blk_round(ws, bq, qh, take, r, a, sink);
                 qh = (qh + take) & (kBQRing - 1);
                 qn_c -= take;
             }
             if (drain) break;
-            uint4 q0 = *reinterpret_cast<const uint4*>(buf + t * 64);
-            uint4 q1 = *reinterpret_cast<const uint4*>(buf + t * 64 + 16);
-            uint4 q2 = *reinterpret_cast<const uint4*>(buf + t * 64 + 32);
-            uint4 q3 = *reinterpret_cast<const uint4*>(buf + t * 64 + 48);
+            uint4 q0 = blk[0], q1 = blk[1], q2 = blk[2], q3 = blk[3];
             if (SGN) {  // int16 -> offset binary
                 q0.x ^= 0x80008000u; q0.y ^= 0x80008000u; q0.z ^= 0x80008000u; q0.w ^= 0x80008000u;
                 q1.x ^= 0x80008000u; q1.y ^= 0x80008000u; q1.z ^= 0x80008000u; q1.w ^= 0x80008000u;
                 q2.x ^= 0x80008000u; q2.y ^= 0x80008000u; q2.z ^= 0x80008000u; q2.w ^= 0x80008000u;
                 q3.x ^= 0x80008000u; q3.y ^= 0x80008000u; q3.z ^= 0x80008000u; q3.w ^= 0x80008000u;
             }
-            const bool wholeblk = vc0 >= wholeA && vc0 + 4 <= wholeB;  // 32 samples of the record
-            unsigned s0 = 0u, s1 = 0u, s2 = 0u, s3 = 0u;
-            if (wholeblk) { s0 = csum4(q0); s1 = csum4(q1); s2 = csum4(q2); s3 = csum4(q3); }
-            if (FEAT) {
-                const bool fast = wholeblk && vc0 >= plainA && vc0 + 4 <= plainB && (vc0 + 4 <= plainHa || vc0 >= plainHb);
-                if (fast) {
-                    feat_plain(q0, s0); feat_plain(q1, s1); feat_plain(q2, s2); feat_plain(q3, s3);
-                } else {
-#pragma unroll 1
-                    for (int c = 0; c < 4; ++c) {  // record start / end, height range, known polarity: chunk by chunk
-                        uint4 q = *reinterpret_cast<const uint4*>(buf + t * 64 + c * 16);
-                        if (SGN) { q.x ^= 0x80008000u; q.y ^= 0x80008000u; q.z ^= 0x80008000u; q.w ^= 0x80008000u; }
-                        feat_generic(q, vc0 + c);
-                    }
-                }
-            }
-            // class of the block
+            // class of the block; with features the sample sum of a block of 32 record samples serves the area and the FULL
+            // aggregate, without them only the aggregate needs it
             bool any = false, full = false, last = false;
-            unsigned kvmin = 0xffffu;
-            if (wholeblk) {
+            unsigned kvmin = 0xffffu, ssum = 0u;
+            if ((unsigned)(32 * B - mis) < whn) {
+                if (FEAT) ssum = csum4(q1, csum4(q0)) + csum4(q3, csum4(q2));
                 const unsigned mn2 = __vimin3_u16x2(
                     __vimin3_u16x2(__vimin3_u16x2(q0.x, q0.y, q0.z), __vimin3_u16x2(q0.w, q1.x, q1.y), __vimin3_u16x2(q1.z, q1.w, q2.x)),
                     __vimin3_u16x2(__vimin3_u16x2(q2.y, q2.z, q2.w), __vimin3_u16x2(q3.x, q3.y, q3.z), q3.w), 0xffffffffu);
@@ -522,11 +519,11 @@ __device__ __forceinline__ void blk_stream(const FHArgs& a, const uint16_t* pool
                 kvmin = (r.positive ? wmax : wmin) ^ xm16;
                 const unsigned kvmax = (r.positive ? wmin : wmax) ^ xm16;
                 any = (int)kvmin <= r.kmax;
-                full = !r.degen && (int)kvmax <= r.kmax;
+                full = (int)kvmax <= kfull;
                 last = (int)((q3.w >> 16) ^ xm16) <= r.kmax;
-            } else if (vc0 < nch) {  // record start / end: by position
-                const int i0 = vc0 * 8 - mis;
-                const unsigned short* hwb = reinterpret_cast<const unsigned short*>(buf + t * 64);
+            } else if (4 * B < nch) {  // record start / end: by position
+                const int i0 = 32 * B - mis;
+                const unsigned short* hwb = reinterpret_cast<const unsigned short*>(blk);
                 for (int j = 0; j < 32; ++j) {
                     const int i = i0 + j;
                     const unsigned w = (unsigned)hwb[j] ^ (SGN ? 0x8000u : 0u);
@@ -535,9 +532,30 @@ __device__ __forceinline__ void blk_stream(const FHArgs& a, const uint16_t* pool
                     last = ab;
                 }
             }
+            if (FEAT) {
+                if ((unsigned)(B - f0) < fn0 || (unsigned)(B - f1) < fn1) {  // inside the blocks of 32 record samples
+                    unsigned e[16];
+                    absdiff4(q0, fs.prev_w, e[0], e[1], e[2], e[3]);
+                    absdiff4(q1, q0.w, e[4], e[5], e[6], e[7]);
+                    absdiff4(q2, q1.w, e[8], e[9], e[10], e[11]);
+                    absdiff4(q3, q2.w, e[12], e[13], e[14], e[15]);
+                    fs.pdiff = __vimax3_u16x2(
+                        __vimax3_u16x2(__vimax3_u16x2(e[0], e[1], e[2]), __vimax3_u16x2(e[3], e[4], e[5]), __vimax3_u16x2(e[6], e[7], e[8])),
+                        __vimax3_u16x2(__vimax3_u16x2(e[9], e[10], e[11]), __vimax3_u16x2(e[12], e[13], e[14]), e[15]), fs.pdiff);
+                    fs.isum32 += ssum;
+                    fs.prev_w = q3.w;
+                } else {
+#pragma unroll 1
+                    for (int c = 0; c < 4; ++c) {  // record start / end, height range, known polarity: chunk by chunk
+                        uint4 q = blk[c];
+                        if (SGN) { q.x ^= 0x80008000u; q.y ^= 0x80008000u; q.z ^= 0x80008000u; q.w ^= 0x80008000u; }
+                        feat_generic(q, 4 * B + c);
+                    }
+                }
+            }
             if (full && open) {
                 fa_key = min(fa_key, (kvmin << 16) | (unsigned)B);
-                fa_sum += (s0 + s1) + (s2 + s3);
+                fa_sum += FEAT ? ssum : csum4(q1, csum4(q0)) + csum4(q3, csum4(q2));
             }
             const bool item = full ? !open : (any || open);
             const unsigned bal = __ballot_sync(kFull, item);
@@ -552,7 +570,7 @@ __device__ __forceinline__ void blk_stream(const FHArgs& a, const uint16_t* pool
                 sl[18] = (unsigned)lane | ((unsigned)B << 5);
                 sl[19] = fa_key;
                 sl[20] = fa_sum;
-                myslot = sl;
+                myslot = slot * kBQWords + 17;
                 fa_key = 0xffffffffu;
                 fa_sum = 0u;
             }
