@@ -284,6 +284,20 @@ int wfb_waveform_width(const void* waves_dev, int64_t n_waves, int32_t length, i
                        int64_t n_hits, const wfb_width_params* params, void* out_dev,
                        uint8_t* valid_dev, void* stream);
 
+/* The same widths for hit rows that live on the device, against a device-resident run (records + pool, e.g. a time
+ * shard).  hits_dev: n_hits packed HIT_DTYPE rows (48 B).  A hit's waveform is run row record_id - row_base, used only
+ * when it lies in [0, n) and meta_dev[row].record_id == record_id (otherwise the hit gives no row, like a hit without a
+ * matching waveform row in wfb_waveform_width); its samples are the record's own event_length samples at
+ * pool_dev[wave_offset - pool_base].  A record whose samples lie outside [0, pool_len) gives no row either.
+ * pool_is_f32: 0 = 16-bit samples read as int16 (what st_waveforms rows of the same samples hold), 1 = float32;
+ * params->wave_is_f32 is not read.  out_dev receives the WAVEFORM_WIDTH rows (56 B, room for n_hits) compacted in hit
+ * order, *n_out_dev (device int64) their number.  Asynchronous: nothing is read back. */
+size_t wfb_waveform_width_run_workspace_bytes(int64_t n_hits);
+int wfb_waveform_width_run(const void* pool_dev, int32_t pool_is_f32, int64_t pool_len, const wfb_rec_meta* meta_dev,
+                           int64_t n, int64_t pool_base, int64_t row_base, const void* hits_dev, int64_t n_hits,
+                           const wfb_width_params* params, void* out_dev, int64_t* n_out_dev, void* workspace_dev,
+                           size_t workspace_bytes, void* stream);
+
 /* Per record cumulative-charge quantile indices.  Replaces
  * WaveformWidthIntegralPlugin.compute records branch (waveform_width_integral.py:166-231).
  * pool_is_f32: 0 uint16 pool, 1 float32 pool, 2 int16 samples (structured st_waveforms rows used in place).
@@ -424,6 +438,8 @@ typedef struct wfb_peak_params {
     int32_t height_window_extension;
     int32_t lmax;           /* longest record (samples) */
     int32_t level_f32;      /* WFB_WAVE_AOS_F32 without derivative: baseline - wave in float32 (the baseline is np.mean of the float32 row) */
+    int64_t pool_base;      /* records sources: record samples start at waves_dev[wave_offset - pool_base] (a time shard holds only its
+                               own pool slice); the AoS sources require 0 */
 } wfb_peak_params;
 size_t wfb_find_peaks_workspace_bytes(int64_t n);
 int wfb_find_peaks(const void* waves_dev, int64_t waves_len, const wfb_rec_meta* meta_dev, int64_t n,
@@ -514,8 +530,8 @@ int wfb_df_columns(const void* feat_rows_dev, const int64_t* record_id_dev, int6
                    size_t workspace_bytes, void* stream);
 
 /* `s1_s2` (core/plugins/builtin/cpu/s1_s2_classifier.py:133-228): one packed S1_S2_CLASSIFIER row (45 B)
- * per waveform_width row (56 B).  height / area come from feat_rows_dev[record_id] (36-B rows) when
- * 0 <= record_id < n_feat, else NaN (:170-180).  A range with present == 0 always passes; a NaN value fails
+ * per waveform_width row (56 B).  height / area come from feat_rows_dev[record_id - feat_row_base] (36-B rows) when
+ * 0 <= record_id - feat_row_base < n_feat, else NaN (:170-180).  A range with present == 0 always passes; a NaN value fails
  * a present range (:54-68).  width_in_samples selects total_width_samples instead of total_width (:182).
  * conflict_policy: 0 unknown, 1 prefer_s1, 2 prefer_s2 (:194-204). */
 typedef struct wfb_range {
@@ -529,6 +545,7 @@ typedef struct wfb_s1s2_params {
     wfb_range s2_width, s2_area, s2_height;
     int32_t width_in_samples;
     int32_t conflict_policy;
+    int64_t feat_row_base;  /* record_id of feat_rows_dev[0]: a time shard's feature rows start at its first record */
 } wfb_s1s2_params;
 int wfb_s1s2_classify(const void* width_rows_dev, int64_t n_peaks, const void* feat_rows_dev, int64_t n_feat,
                       const wfb_s1s2_params* params, void* out_rows_dev, void* stream);

@@ -37,7 +37,15 @@ on the whole run) and checks the gathered df columns, event table, members and d
 (ended by a device synchronize), the events and member rows of every rank and the peak extra device memory of the stage;
 with --verify 1 every rank gathers the hit_grouped frame of the whole run (``distributed.gather_hit_grouped_frame``) and
 rank 0 checks it against ``ops.group_hit_windows`` on the single-GPU hit_merged rows, packaged as B200HitGroupedPlugin
-does."""
+does.
+
+--peaks adds the wave_pool_filtered -> hit -> waveform_width -> s1_s2 leg on a positive-pulse copy of every rank's
+shard (samples and baselines mirrored around the 14-bit mid-scale, as bench.py's c3 leg makes them: waveform_width keeps
+only peaks above the row's baseline): ``distributed.peaks_sharded`` with the SG filter (11 / 2), hit (height 8, width
+2), waveform_width (0.25 GHz) and s1_s2 on the shard's basic_features.  It reports the row counts, the time of every
+stage (each ended by a device synchronize) and the peak extra device memory of the leg; with --verify 1 rank 0 runs
+the same chain on the whole run (the rank-order concatenation of the shards) and checks the gathered filtered pool,
+hit, waveform_width and s1_s2 rows byte for byte."""
 import argparse
 import os
 import sys
@@ -63,6 +71,7 @@ ap.add_argument("--mixed-widths", action="store_true", help="--source raw: odd g
 ap.add_argument("--samples", type=int, default=800)
 ap.add_argument("--events", action="store_true", help="also run the sharded df -> df_events -> df_paired leg")
 ap.add_argument("--hit-events", action="store_true", help="also build the sharded hit_grouped event table")
+ap.add_argument("--peaks", action="store_true", help="also run the sharded filter -> hit -> waveform_width -> s1_s2 leg")
 args = ap.parse_args()
 
 D.init_process_group("nccl")
@@ -322,6 +331,80 @@ def hit_events_leg():
     return f"hit events={int(hev['events_per_rank'].sum())}", frame
 
 
+PEAK_FILTER = {"filter_type": "SG", "sg_window_size": 11, "sg_poly_order": 2}
+PEAK_OPTS = {"height": 8.0, "width": 2}
+WIDTH_OPTS = {"sampling_rate": 0.25}
+S1S2_OPTS = {"s1_width_range": (None, 60.0), "s2_width_range": (40.0, None), "conflict_policy": "prefer_s2"}
+
+
+def positive_copy(r):
+    """A copy of a run with positive pulses, as bench.py's c3 leg makes them: samples and baselines mirrored around the
+    14-bit mid-scale, records marked positive (waveform_width keeps only peaks above the row's baseline)."""
+    meta = r.meta.clone()
+    m = meta.view(-1, 48)
+    base = m[:, 8:16].contiguous().view(torch.float64).view(-1)
+    m[:, 8:16] = (16383.0 - base).view(torch.uint8).view(-1, 8)
+    m[:, 36] = 1  # WFB_POL_POSITIVE
+    out = engine.DeviceRun(meta, 16383 - r.pool, r.n, 0, r.lmax, records_rows=r.records_rows, pool_base=r.pool_base, row_base=r.row_base)
+    out.lmin = r.lmin
+    return out
+
+
+def peaks_rows_host(x: dict):
+    from waveformanalysis_b200.dtypes import HIT_DTYPE, S1_S2_CLASSIFIER_DTYPE, WAVEFORM_WIDTH_DTYPE
+
+    return tuple(x[k][: x["n_" + k] * dt.itemsize].cpu().numpy().tobytes()
+                 for k, dt in (("hits", HIT_DTYPE), ("widths", WAVEFORM_WIDTH_DTYPE), ("labels", S1_S2_CLASSIFIER_DTYPE)))
+
+
+def peaks_leg() -> str:
+    """filter -> hit -> waveform_width -> s1_s2 on this rank's shard (positive copy) with distributed.peaks_sharded; with
+    --verify rank 0 runs the same chain on the whole run (the rank-order concatenation of the shards) on its GPU."""
+    prun = positive_copy(run)
+    feats = prun.features_hits(hits=False)["features"]
+    torch.cuda.synchronize()
+    torch.cuda.reset_peak_memory_stats()
+    base_mem = torch.cuda.memory_allocated()
+    if ws > 1:
+        dist.barrier()
+    t = time.perf_counter()
+    ph = D.peaks_sharded(prun, filter_cfg=PEAK_FILTER, features=feats, peak_opts=PEAK_OPTS, width_opts=WIDTH_OPTS, s1s2_opts=S1S2_OPTS)
+    torch.cuda.synchronize()
+    wall = time.perf_counter() - t
+    peak = torch.cuda.max_memory_allocated() - base_mem
+    line = (f"rank {rank}: records {prun.n} hits {ph['n_hits']} widths {ph['n_widths']} labels {ph['n_labels']} (bases {ph['hit_base']} / "
+            f"{ph['width_base']} / {ph['label_base']}) | " + " ".join(f"{k} {1e3 * v:.1f} ms" for k, v in ph["timings"].items()) +
+            f" | leg wall {1e3 * wall:.1f} ms | peak extra device memory {peak / 1e9:.3f} GB "
+            f"({peak / max(2 * prun.pool_len, 1):.2f} x the shard's 16-bit sample bytes) | {gpu_name()}")
+    lines = D.gather_rows(np.frombuffer(line.encode().ljust(1024)[:1024], dtype="S1024")) if ws > 1 else [line.encode()]
+    if rank == 0:
+        print(f"peaks leg: world={ws} records/rank={n} samples/record={L} filter SG 11/2, hit height 8 width 2, waveform_width 0.25 GHz")
+        for ln in lines:
+            print("  " + ln.decode().strip())
+    out = f"peaks: hits={ph['n_hits_total']} widths={ph['n_widths_total']} labels={ph['n_labels_total']}"
+    if not args.verify:
+        return out
+    got_sg = D.gather_rows(ph["filtered"].cpu().numpy())
+    got = D.gather_peak_rows(ph)
+    if ingest is not None:
+        recs_all = D.gather_rows(run.records_rows[: run.n * 102].cpu().numpy().view(RECORDS_DTYPE))
+        pool_all = D.gather_rows(run.pool.cpu().numpy().view([("s", "<u2")]))["s"]
+    del ph, prun, feats
+    if rank != 0:
+        return out
+    torch.cuda.empty_cache()
+    whole = engine.DeviceRun.from_host(recs_all, pool_all) if ingest is not None else engine.DeviceRun.synth(n * ws, L, NCH, seed=SEED)
+    whole = positive_copy(whole)
+    want = D.peaks_local(whole, filter_cfg=PEAK_FILTER, features=whole.features_hits(hits=False)["features"], peak_opts=PEAK_OPTS,
+                         width_opts=WIDTH_OPTS, s1s2_opts=S1S2_OPTS)
+    assert want["filtered"].cpu().numpy().tobytes() == got_sg.tobytes(), "filtered pool differs"
+    for name, g, w in zip(("hit", "waveform_width", "s1_s2"), got, peaks_rows_host(want)):
+        assert g.tobytes() == w, f"{name} rows differ"
+    labels = got[2]["label"]
+    return out + (f" | filtered pool, hit, waveform_width and s1_s2 rows byte-identical to the single-GPU chain on the whole run "
+                  f"({whole.n} records; labels S1 {int((labels == 1).sum())}, S2 {int((labels == 2).sum())}, unknown {int((labels == 0).sum())})")
+
+
 def frames_equal(got, want) -> bool:
     if list(got.columns) != list(want.columns) or len(got) != len(want) or not got.index.equals(want.index):
         return False
@@ -338,6 +421,8 @@ def frames_equal(got, want) -> bool:
 
 if args.events:
     msg += " | " + events_leg()
+if args.peaks:
+    msg += " | " + peaks_leg()
 hit_frame = None
 if args.hit_events:
     out, hit_frame = hit_events_leg()

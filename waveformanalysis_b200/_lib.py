@@ -109,7 +109,8 @@ _vp, _i64, _i32, _sz, _dbl = C.c_void_p, C.c_int64, C.c_int32, C.c_size_t, C.c_d
 class PeakParams(C.Structure):  # wfb_peak_params
     _fields_ = [("wave_kind", C.c_int32), ("use_derivative", C.c_int32), ("height", C.c_double), ("prominence", C.c_double),
                 ("width", C.c_double), ("threshold", C.c_double), ("has_threshold", C.c_int32), ("distance", C.c_int32),
-                ("height_method", C.c_int32), ("height_window_extension", C.c_int32), ("lmax", C.c_int32), ("level_f32", C.c_int32)]
+                ("height_method", C.c_int32), ("height_window_extension", C.c_int32), ("lmax", C.c_int32), ("level_f32", C.c_int32),
+                ("pool_base", C.c_int64)]
 
 
 class GainRule(C.Structure):  # wfb_gain_rule
@@ -123,7 +124,7 @@ class Range(C.Structure):  # wfb_range
 
 class S1S2Params(C.Structure):  # wfb_s1s2_params
     _fields_ = [("s1_width", Range), ("s1_area", Range), ("s1_height", Range), ("s2_width", Range), ("s2_area", Range),
-                ("s2_height", Range), ("width_in_samples", C.c_int32), ("conflict_policy", C.c_int32)]
+                ("s2_height", Range), ("width_in_samples", C.c_int32), ("conflict_policy", C.c_int32), ("feat_row_base", C.c_int64)]
 
 
 WAVE_AOS_I16, WAVE_AOS_F32, WAVE_REC_U16, WAVE_REC_F32, WAVE_AOS_F32_AS_F64, WAVE_AOS_U16 = 0, 1, 2, 3, 4, 5
@@ -167,6 +168,8 @@ PROTOTYPES = {
     "wfb_filter_pool": (C.c_int, [_vp, _i32, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _sz, _i32, _vp]),
     "wfb_filter_workspace_bytes": (_sz, [_i64, _i32]),
     "wfb_waveform_width": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64, C.POINTER(WidthParams), _vp, _vp, _vp]),
+    "wfb_waveform_width_run_workspace_bytes": (_sz, [_i64]),
+    "wfb_waveform_width_run": (C.c_int, [_vp, _i32, _i64, _vp, _i64, _i64, _i64, _vp, _i64, C.POINTER(WidthParams), _vp, _vp, _vp, _sz, _vp]),
     "wfb_width_integral": (C.c_int, [_vp, _i32, _i64, _vp, _i64, _dbl, _dbl, _dbl, _i64, _i64, _vp, _vp]),
     "wfb_group_workspace_bytes": (_sz, [_i64]),
     "wfb_group_hit_windows": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _dbl, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),

@@ -33,6 +33,7 @@ constexpr int kRecordsRowBytes = 102;  // RECORDS_DTYPE
 constexpr int kFeatRowBytes = 36;      // BASIC_FEATURES_DTYPE
 constexpr int kHitRowBytes = 60;       // THRESHOLD_HIT_DTYPE
 constexpr int kWidthRowBytes = 56;     // WAVEFORM_WIDTH_DTYPE
+constexpr int kPeakRowBytes = 48;      // HIT_DTYPE
 constexpr int kWidthIntRowBytes = 52;  // WAVEFORM_WIDTH_INTEGRAL_DTYPE
 
 constexpr unsigned kFull = 0xffffffffu;

@@ -88,9 +88,10 @@ __global__ void __launch_bounds__(kS1S2Block) s1s2_kernel(const uint8_t* widths,
         const long long ts = ld_i64_u4(w + 36);
         const unsigned bc = *reinterpret_cast<const unsigned*>(w + 44);
         const long long rid = ld_i64_u4(w + 48);
+        const long long frow = rid - p.feat_row_base;
         float height = nanf(""), area = nanf("");
-        if (rid >= 0 && rid < n_feat) {
-            const float* f = reinterpret_cast<const float*>(feat + rid * kFeatRow);
+        if (frow >= 0 && frow < n_feat) {
+            const float* f = reinterpret_cast<const float*>(feat + frow * kFeatRow);
             height = f[0];
             area = f[2];
         }

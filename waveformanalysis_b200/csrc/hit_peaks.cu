@@ -21,7 +21,6 @@
 namespace wfb {
 
 constexpr int kPeakWarps = 4;
-constexpr int kPeakRowBytes = 48;  // HIT_DTYPE
 constexpr int kPeakCache = 6;      // peaks per record the counting pass remembers (position, left / right edge)
 
 struct PeakCacheEnt {  // 24 bytes
@@ -170,7 +169,7 @@ __global__ void __launch_bounds__(256) peaks_emit_cached_kernel(const void* __re
     r.deriv = p.use_derivative != 0;
     r.m = r.deriv ? max(r.len - 1, 0) : r.len;
     r.baseline = mrec.baseline;
-    r.w = Wave{waves, mrec.wave_offset, p.wave_kind, (float)mrec.baseline, mrec.polarity == WFB_POL_POSITIVE};
+    r.w = Wave{waves, mrec.wave_offset - p.pool_base, p.wave_kind, (float)mrec.baseline, mrec.polarity == WFB_POL_POSITIVE};
     r.x = nullptr;
     const PeakCacheEnt e = cache[rec * kPeakCache + k];
     const long long row = row_incl[rec] - c + k;
@@ -198,7 +197,7 @@ __global__ void __launch_bounds__(kPeakWarps * 32) find_peaks_kernel(const void*
     auto do_record = [&](const long long rec) {
     const wfb_rec_meta mrec = meta[rec];
     int len = mrec.event_length;
-    const long long off = mrec.wave_offset;
+    const long long off = mrec.wave_offset - p.pool_base;  // 0 for the AoS sources
     if (len < 0) len = 0;
     if (len > 0 && (off < 0 || off + len > waves_len)) {
         if (lane == 0) atomicExch(err, 1);
@@ -491,6 +490,8 @@ extern "C" int wfb_find_peaks(const void* waves_dev, int64_t waves_len, const wf
     WFB_REQUIRE(meta_dev && workspace_dev && (waves_dev || waves_len == 0), "wfb_find_peaks: NULL pointer");
     WFB_REQUIRE(row_cap == 0 || rows_out_dev != nullptr, "wfb_find_peaks: NULL row buffer");
     WFB_REQUIRE(params->wave_kind >= WFB_WAVE_AOS_I16 && params->wave_kind <= WFB_WAVE_AOS_U16, "wfb_find_peaks: unknown wave_kind");
+    WFB_REQUIRE(params->pool_base == 0 || params->wave_kind == WFB_WAVE_REC_U16 || params->wave_kind == WFB_WAVE_REC_F32,
+                "wfb_find_peaks: pool_base %lld needs a records wave_kind (the AoS sources take pool_base 0)", (long long)params->pool_base);
     WFB_REQUIRE(params->height_method >= 0 && params->height_method <= 2, "unsupported height_method");
     WFB_REQUIRE(params->lmax > 0, "wfb_find_peaks: lmax must be the longest record");
     WFB_REQUIRE(workspace_bytes >= wfb_find_peaks_workspace_bytes(n), "wfb_find_peaks: workspace too small");

@@ -3,8 +3,11 @@
 //
 // Reference: core/plugins/builtin/cpu/waveform_width.py:205-374,
 //            core/plugins/builtin/cpu/waveform_width_integral.py:166-231.
+#include <algorithm>
+
 #include "common.cuh"
 #include "np_sum.cuh"
+#include "sort_scan.cuh"
 
 namespace wfb {
 
@@ -96,31 +99,73 @@ __device__ __forceinline__ void warp_find_first2(int lo, int hi, V val, PA pa, P
     }
 }
 
+// Where a hit's samples and its row fields come from.  `locate` gives the hit's waveform and its length (false: no
+// waveform, the hit gives no row); the other members give the hit's own fields.
 template <typename T>
-__global__ void __launch_bounds__(256) waveform_width_kernel(const T* __restrict__ waves, long long n_waves, int length,
-                                                            long long stride, const long long* __restrict__ hit_row,
-                                                            const long long* __restrict__ hit_pos,
-                                                            const long long* __restrict__ hit_ts,
-                                                            const short* __restrict__ hit_board,
-                                                            const short* __restrict__ hit_channel,
-                                                            const long long* __restrict__ hit_rid, long long n_hits,
-                                                            const wfb_width_params p, uint8_t* __restrict__ out,
-                                                            uint8_t* __restrict__ valid) {
+struct WidthRowsSrc {  // structured rows of one width, hits as device columns (wfb_waveform_width)
+    const T* waves;
+    long long n_waves;
+    int length;
+    long long stride;
+    const long long *row, *pos, *ts;
+    const short *board, *channel;
+    const long long* rid;
+    __device__ __forceinline__ bool locate(long long hit, const T*& w, int& len) const {
+        const long long r = row[hit];
+        if (r < 0 || r >= n_waves) return false;
+        w = waves + r * stride;
+        len = length;
+        return true;
+    }
+    __device__ __forceinline__ long long position(long long hit) const { return pos[hit]; }
+    __device__ __forceinline__ long long timestamp(long long hit) const { return ts[hit]; }
+    __device__ __forceinline__ unsigned board_channel(long long hit) const {
+        return ((unsigned)(unsigned short)(board ? board[hit] : 0)) | ((unsigned)(unsigned short)channel[hit] << 16);
+    }
+    __device__ __forceinline__ long long record_id(long long hit) const { return rid[hit]; }
+};
+
+template <typename T>
+struct WidthRunSrc {  // a device-resident run (records meta + pool slice), hits as packed HIT rows (wfb_waveform_width_run)
+    const T* pool;
+    long long pool_len;
+    const wfb_rec_meta* meta;
+    long long n, pool_base, row_base;
+    const unsigned* hits;  // HIT_DTYPE rows as words
+    __device__ __forceinline__ long long word64(long long hit, int k) const {
+        const unsigned* h = hits + hit * (kPeakRowBytes / 4);
+        return (long long)(((unsigned long long)h[k + 1] << 32) | h[k]);
+    }
+    __device__ __forceinline__ bool locate(long long hit, const T*& w, int& len) const {
+        const long long rid = record_id(hit);
+        const long long r = rid - row_base;
+        if (r < 0 || r >= n || meta[r].record_id != rid) return false;
+        const long long off = meta[r].wave_offset - pool_base;
+        len = meta[r].event_length;
+        if (off < 0 || len < 0 || off + len > pool_len) return false;
+        w = pool + off;
+        return true;
+    }
+    __device__ __forceinline__ long long position(long long hit) const { return word64(hit, 0); }
+    __device__ __forceinline__ long long timestamp(long long hit) const { return word64(hit, 7); }
+    __device__ __forceinline__ unsigned board_channel(long long hit) const { return hits[hit * (kPeakRowBytes / 4) + 9]; }
+    __device__ __forceinline__ long long record_id(long long hit) const { return word64(hit, 10); }
+};
+
+// One hit, by its whole warp.  Returns whether the hit gives a row (the same value in every lane); with ROWS the row's
+// 14 words are written to `out`, without it the work ends once that is known (the counting pass of the run variant).
+template <typename T, bool ROWS, typename Src>
+__device__ __forceinline__ bool width_of_hit(const Src& src, long long hit, const wfb_width_params& p, unsigned* __restrict__ out) {
     constexpr bool F32 = sizeof(T) == 4;
     const int lane = lane_id();
-    const long long hit = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
-    if (hit >= n_hits) return;
-    const long long row = hit_row[hit];
-    const long long pos64 = hit_pos[hit];
-    bool ok = row >= 0 && row < n_waves && pos64 < length && length > 0;
+    const T* w = nullptr;
+    int length = 0;
+    if (!src.locate(hit, w, length)) return false;
+    const long long pos64 = src.position(hit);
+    if (!(pos64 < length && length > 0)) return false;
     // numpy negative indices wrap: position in [-length, 0) addresses from the end
-    long long posw = pos64 < 0 ? pos64 + length : pos64;
-    ok = ok && posw >= 0 && posw < length;
-    if (!ok) {
-        if (lane == 0) valid[hit] = 0;
-        return;
-    }
-    const T* w = waves + row * stride;
+    const long long posw = pos64 < 0 ? pos64 + length : pos64;
+    if (!(posw >= 0 && posw < length)) return false;
     const int pos = (int)posw;
     const int nb = min(50, length);
     double bl64 = 0.0;
@@ -136,14 +181,10 @@ __global__ void __launch_bounds__(256) waveform_width_kernel(const T* __restrict
     auto wc64 = [&](int i) -> double { return __dsub_rn((double)w[i], bl64); };
     auto wc32 = [&](int i) -> float { return __fsub_rn((float)w[i], bl32); };
     const double pv = F32 ? (double)wc32(pos) : wc64(pos);
-    if (!(pv > 0.0)) {  // peak_value <= 0 (or NaN compares false in the reference too: NaN <= 0 is False!)
-        if (pv <= 0.0) {
-            if (lane == 0) valid[hit] = 0;
-            return;
-        }
-    }
+    if (pv <= 0.0) return false;  // peak_value <= 0 (NaN compares false in the reference too: NaN <= 0 is False!)
+    if (!ROWS) return true;
     // the slices wave[:pos] / wave[pos:] use the raw (possibly negative) position
-    const int left_hi = pos64 < 0 ? pos : pos;
+    const int left_hi = pos;
     // thresholds
     double t64[4];
     float t32[4];
@@ -222,15 +263,45 @@ __global__ void __launch_bounds__(256) waveform_width_kernel(const T* __restrict
             case 6: word = (unsigned)(pos64 & 0xffffffffll); break;
             case 7: word = (unsigned)((unsigned long long)pos64 >> 32); break;
             case 8: word = __float_as_uint((float)pv); break;
-            case 9: word = (unsigned)(hit_ts[hit] & 0xffffffffll); break;
-            case 10: word = (unsigned)((unsigned long long)hit_ts[hit] >> 32); break;
-            case 11: word = ((unsigned)(unsigned short)(hit_board ? hit_board[hit] : 0)) | ((unsigned)(unsigned short)hit_channel[hit] << 16); break;
-            case 12: word = (unsigned)(hit_rid[hit] & 0xffffffffll); break;
-            default: word = (unsigned)((unsigned long long)hit_rid[hit] >> 32); break;
+            case 9: word = (unsigned)(src.timestamp(hit) & 0xffffffffll); break;
+            case 10: word = (unsigned)((unsigned long long)src.timestamp(hit) >> 32); break;
+            case 11: word = src.board_channel(hit); break;
+            case 12: word = (unsigned)(src.record_id(hit) & 0xffffffffll); break;
+            default: word = (unsigned)((unsigned long long)src.record_id(hit) >> 32); break;
         }
-        reinterpret_cast<unsigned*>(out + hit * kWidthRowBytes)[lane] = word;
+        out[lane] = word;
     }
-    if (lane == 0) valid[hit] = 1;
+    return true;
+}
+
+// six blocks of the float32 instance fit an SM at 40 registers (the row source's fields would otherwise take it to 46)
+template <typename T>
+__global__ void __launch_bounds__(256, sizeof(T) == 4 ? 6 : 5) waveform_width_kernel(const WidthRowsSrc<T> src, long long n_hits, const wfb_width_params p,
+                                                            uint8_t* __restrict__ out, uint8_t* __restrict__ valid) {
+    const long long hit = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    if (hit >= n_hits) return;
+    const bool ok = width_of_hit<T, true>(src, hit, p, reinterpret_cast<unsigned*>(out + hit * kWidthRowBytes));
+    if (lane_id() == 0) valid[hit] = ok ? 1 : 0;
+}
+
+// wfb_waveform_width_run: a counting pass (which hits give a row), an inclusive scan of the counts, and the pass that
+// writes every row at its place in hit order
+template <typename T>
+__global__ void __launch_bounds__(256) waveform_width_run_count_kernel(const WidthRunSrc<T> src, long long n_hits, const wfb_width_params p,
+                                                                      long long* __restrict__ has_row) {
+    const long long hit = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    if (hit >= n_hits) return;
+    const bool ok = width_of_hit<T, false>(src, hit, p, nullptr);
+    if (lane_id() == 0) has_row[hit] = ok ? 1 : 0;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) waveform_width_run_kernel(const WidthRunSrc<T> src, long long n_hits, const wfb_width_params p,
+                                                                const long long* __restrict__ has_row, const long long* __restrict__ row_incl,
+                                                                uint8_t* __restrict__ out) {
+    const long long hit = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    if (hit >= n_hits || !has_row[hit]) return;
+    width_of_hit<T, true>(src, hit, p, reinterpret_cast<unsigned*>(out + (row_incl[hit] - 1) * kWidthRowBytes));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -490,13 +561,67 @@ extern "C" int wfb_waveform_width(const void* waves_dev, int64_t n_waves, int32_
     const long long* ts = reinterpret_cast<const long long*>(hit_timestamp_dev);
     const long long* rid = reinterpret_cast<const long long*>(hit_record_id_dev);
     if (params->wave_is_f32)
-        waveform_width_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(waves_dev), n_waves, length, stride, row, pos, ts,
-                                                           hit_board_dev, hit_channel_dev, rid, n_hits, *params,
-                                                           static_cast<uint8_t*>(out_dev), valid_dev);
+        waveform_width_kernel<float><<<blocks, 256, 0, st>>>(
+            WidthRowsSrc<float>{static_cast<const float*>(waves_dev), n_waves, length, stride, row, pos, ts, hit_board_dev, hit_channel_dev, rid},
+            n_hits, *params, static_cast<uint8_t*>(out_dev), valid_dev);
     else
-        waveform_width_kernel<short><<<blocks, 256, 0, st>>>(static_cast<const short*>(waves_dev), n_waves, length, stride, row, pos, ts,
-                                                           hit_board_dev, hit_channel_dev, rid, n_hits, *params,
-                                                           static_cast<uint8_t*>(out_dev), valid_dev);
+        waveform_width_kernel<short><<<blocks, 256, 0, st>>>(
+            WidthRowsSrc<short>{static_cast<const short*>(waves_dev), n_waves, length, stride, row, pos, ts, hit_board_dev, hit_channel_dev, rid},
+            n_hits, *params, static_cast<uint8_t*>(out_dev), valid_dev);
+    WFB_CUDA(cudaGetLastError());
+    return WFB_OK;
+}
+
+static size_t wr_al256(size_t x) { return (x + 255) & ~(size_t)255; }
+
+extern "C" size_t wfb_waveform_width_run_workspace_bytes(int64_t n_hits) {
+    const size_t m = wr_al256((size_t)std::max<int64_t>(n_hits, 1) * 8);
+    return 2 * m + scan_workspace_bytes(n_hits);
+}
+
+template <typename T>
+static void launch_width_run(const WidthRunSrc<T>& src, long long n_hits, const wfb_width_params& p, long long* has_row, long long* incl,
+                             void* scan_ws, uint8_t* out, int* rc, cudaStream_t st) {
+    const unsigned blocks = (unsigned)((n_hits * 32 + 255) / 256);
+    waveform_width_run_count_kernel<T><<<blocks, 256, 0, st>>>(src, n_hits, p, has_row);
+    *rc = inclusive_scan_sum_i64(has_row, incl, n_hits, scan_ws, st);
+    if (*rc != WFB_OK) return;
+    waveform_width_run_kernel<T><<<blocks, 256, 0, st>>>(src, n_hits, p, has_row, incl, out);
+}
+
+extern "C" int wfb_waveform_width_run(const void* pool_dev, int32_t pool_is_f32, int64_t pool_len, const wfb_rec_meta* meta_dev,
+                                      int64_t n, int64_t pool_base, int64_t row_base, const void* hits_dev, int64_t n_hits,
+                                      const wfb_width_params* params, void* out_dev, int64_t* n_out_dev, void* workspace_dev,
+                                      size_t workspace_bytes, void* stream) {
+    WFB_REQUIRE(params != nullptr && n_out_dev != nullptr, "wfb_waveform_width_run: NULL params / count");
+    WFB_REQUIRE(n_hits >= 0 && n >= 0 && pool_len >= 0, "wfb_waveform_width_run: negative size");
+    WFB_REQUIRE(pool_is_f32 == 0 || pool_is_f32 == 1, "wfb_waveform_width_run: pool_is_f32 must be 0 or 1, got %d", pool_is_f32);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (n_hits == 0) {
+        WFB_CUDA(cudaMemsetAsync(n_out_dev, 0, 8, st));
+        return WFB_OK;
+    }
+    WFB_REQUIRE(hits_dev && out_dev && workspace_dev && (meta_dev || n == 0) && (pool_dev || pool_len == 0),
+                "wfb_waveform_width_run: NULL pointer");
+    WFB_REQUIRE(((uintptr_t)hits_dev & 3) == 0, "wfb_waveform_width_run: hit rows must be 4-byte aligned");
+    WFB_REQUIRE(params->sampling_rate != 0.0, "wfb_waveform_width_run: sampling_rate is 0");
+    WFB_REQUIRE(workspace_bytes >= wfb_waveform_width_run_workspace_bytes(n_hits), "wfb_waveform_width_run: workspace too small");
+    uint8_t* ws = static_cast<uint8_t*>(workspace_dev);
+    const size_t m = wr_al256((size_t)n_hits * 8);
+    long long* has_row = reinterpret_cast<long long*>(ws);
+    long long* incl = reinterpret_cast<long long*>(ws + m);
+    void* scan_ws = ws + 2 * m;
+    const unsigned* hits = static_cast<const unsigned*>(hits_dev);
+    uint8_t* out = static_cast<uint8_t*>(out_dev);
+    int rc = WFB_OK;
+    if (pool_is_f32)
+        launch_width_run(WidthRunSrc<float>{static_cast<const float*>(pool_dev), pool_len, meta_dev, n, pool_base, row_base, hits}, n_hits, *params,
+                         has_row, incl, scan_ws, out, &rc, st);
+    else
+        launch_width_run(WidthRunSrc<short>{static_cast<const short*>(pool_dev), pool_len, meta_dev, n, pool_base, row_base, hits}, n_hits, *params,
+                         has_row, incl, scan_ws, out, &rc, st);
+    if (rc != WFB_OK) return rc;
+    WFB_CUDA(cudaMemcpyAsync(n_out_dev, incl + n_hits - 1, 8, cudaMemcpyDeviceToDevice, st));
     WFB_CUDA(cudaGetLastError());
     return WFB_OK;
 }

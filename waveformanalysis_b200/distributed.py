@@ -1419,3 +1419,136 @@ def gather_event_frames(df_sh: dict, ev_sh: dict):
     out = dict(keep=ev_rows["keep"].astype(bool), delta_t=np.ascontiguousarray(ev_rows["delta_t"]),
                area_ch=np.ascontiguousarray(ev_rows["area_ch"]).reshape(-1, nc), height_ch=np.ascontiguousarray(ev_rows["height_ch"]).reshape(-1, nc))
     return df, df_events, paired_frame(df_events, offsets, out, nc, start)
+
+
+# ------------------------------------------------------------------------------------------------
+# Time-sharded wave_pool_filtered -> hit -> waveform_width -> s1_s2: per-record rows, no boundary zones
+# ------------------------------------------------------------------------------------------------
+# Every row of this branch depends on one record only: the filtered samples of a record, its find_peaks rows, the
+# width of each of its peaks and that width's label (with the record's own basic_features row).  So a rank runs the
+# chain on its time shard alone and the rank-order concatenation of the shards' rows is the single-GPU result.  The
+# only collective is ONE fixed-size all_gather per rank: an error flag, a digest of the options and the three row
+# counts, which number every rank's rows globally.
+
+
+def _sync():
+    import torch
+
+    torch.cuda.current_stream().synchronize()
+
+
+def peaks_local(run, *, filter_cfg: dict | None = None, features=None, peak_opts: dict | None = None, width_opts: dict | None = None,
+                s1s2_opts: dict | None = None) -> dict:
+    """The filter -> hit -> waveform_width -> s1_s2 chain on ONE time shard (a ``DeviceRun`` with its own records and
+    pool slice, ``pool_base`` / ``row_base`` set), with no collective.  Everything stays on the device.
+
+    1. ``filter_cfg`` (the form ``ops.filter_run_device`` takes: one configuration for every record; per-channel
+       configurations are not supported on a shard) filters the shard into a float32 pool; ``None`` keeps the raw
+       16-bit pool (the ``use_filtered=False`` route).
+    2. ``ops.find_peaks_device`` on those samples (``WFB_WAVE_REC_F32`` / ``WFB_WAVE_REC_U16``) with ``peak_opts``
+       (``find_peaks_launch``'s options): the `hit` rows of ``B200HitFinderPlugin(wave_source="records")``.
+    3. ``ops.waveform_width_run`` on the same samples with ``width_opts`` (sampling_rate, rise_low, rise_high,
+       fall_high, fall_low, interpolation): ``B200WaveformWidthPlugin`` on the shard's st_waveforms / filtered rows.
+    4. With ``features`` (the shard's packed basic_features rows, as ``run.features_hits()["features"]`` returns
+       them): ``ops.s1s2_classify_device`` with ``feat_row_base = run.row_base`` and ``s1s2_opts`` (width_unit,
+       normalised ranges, conflict_policy).
+
+    Returns ``filtered`` (float32 device pool or None), ``hits`` / ``widths`` / ``labels`` (packed rows as device
+    uint8 tensors; ``labels`` None without features) with ``n_hits`` / ``n_widths`` / ``n_labels``, and ``timings``
+    (seconds per stage, each ended by a device synchronize)."""
+    import time
+
+    from . import _lib, ops
+    from .engine import DeviceRun
+
+    T: dict = {}
+    t = time.perf_counter()
+    src, filtered = run, None
+    if filter_cfg is not None:
+        filtered = ops.filter_run_device(run, filter_cfg)
+        src = DeviceRun(run.meta, filtered, run.n, 1, run.lmax, records_rows=run.records_rows, pool_base=run.pool_base, row_base=run.row_base)
+        _sync()
+        T["filter"] = time.perf_counter() - t
+    t = time.perf_counter()
+    if run.n and run.lmax > 0:
+        kind = _lib.WAVE_REC_F32 if src.pool_is_f32 else _lib.WAVE_REC_U16
+        hits, n_hits = ops.find_peaks_device(src, kind, src.lmax, **(peak_opts or {}))
+    else:
+        hits, n_hits = ops._empty(0), 0
+    _sync()
+    T["hit"] = time.perf_counter() - t
+    t = time.perf_counter()
+    widths, n_widths = ops.waveform_width_run(src, hits, n_hits, **(width_opts or {}))
+    _sync()
+    T["width"] = time.perf_counter() - t
+    labels, n_labels = None, 0
+    if features is not None:
+        t = time.perf_counter()
+        labels = ops.s1s2_classify_device(widths, n_widths, features, run.n, feat_row_base=run.row_base, **(s1s2_opts or {}))
+        n_labels = n_widths
+        _sync()
+        T["s1_s2"] = time.perf_counter() - t
+    return dict(filtered=filtered, hits=hits, n_hits=int(n_hits), widths=widths, n_widths=int(n_widths), labels=labels, n_labels=int(n_labels),
+                timings=T)
+
+
+def peaks_options_digest(filter_cfg, with_features: bool, peak_opts, width_opts, s1s2_opts) -> int:
+    """64-bit digest of the options of the peaks leg, equal on every process for equal options."""
+    import hashlib
+    import json
+
+    def plain(x):
+        return np.asarray(x).tolist()
+
+    blob = json.dumps([filter_cfg, bool(with_features), peak_opts or {}, width_opts or {}, s1s2_opts or {}], sort_keys=True, default=plain)
+    return int(np.frombuffer(hashlib.blake2b(blob.encode(), digest_size=8).digest(), dtype="<i8")[0])
+
+
+def peaks_sharded(run, *, filter_cfg: dict | None = None, features=None, peak_opts: dict | None = None, width_opts: dict | None = None,
+                  s1s2_opts: dict | None = None, local_fn=None) -> dict:
+    """``peaks_local`` on this rank's time shard plus ONE fixed-size all_gather (error flag, options digest, the three
+    row counts).  Options that differ between ranks, or an error on any rank, raise ValueError on every rank (the
+    rank that failed raises its own error).  Per-channel filter configurations are not supported on shards.
+
+    Returns ``peaks_local``'s result plus ``hit_base`` / ``width_base`` / ``label_base`` (global index of the rank's
+    first row), ``hits_per_rank`` / ``widths_per_rank`` / ``labels_per_rank`` and the totals ``n_hits_total`` /
+    ``n_widths_total`` / ``n_labels_total``.  ``local_fn`` replaces ``peaks_local`` (tests of the collective)."""
+    local_fn = local_fn if local_fn is not None else peaks_local
+    _, rank, _ = _dist()
+    digest = peaks_options_digest(filter_cfg, features is not None, peak_opts, width_opts, s1s2_opts)
+    err, res = None, {}
+    try:
+        res = local_fn(run, filter_cfg=filter_cfg, features=features, peak_opts=peak_opts, width_opts=width_opts, s1s2_opts=s1s2_opts)
+        counts = [int(res["n_hits"]), int(res["n_widths"]), int(res["n_labels"])]
+    except Exception as e:  # noqa: BLE001 - every rank must reach the gather, the error is raised after it
+        err, counts = e, [0, 0, 0]
+    table = _allgather_i64([int(err is not None), digest, *counts])
+    if table[:, 0].any():
+        if err is not None:
+            raise err
+        raise ValueError(f"the peaks leg failed on ranks {np.flatnonzero(table[:, 0]).tolist()}")
+    if np.any(table[:, 1] != table[0, 1]):
+        raise ValueError("filter_cfg, features (given or not), peak_opts, width_opts and s1s2_opts must be the same on every rank")
+    me = rank if len(table) > 1 else 0
+    res = dict(res)
+    for j, k in enumerate(("hit", "width", "label")):
+        res[f"{k}_base"] = int(table[:me, 2 + j].sum())
+        res[f"{k}s_per_rank"] = table[:, 2 + j].copy()
+        res[f"n_{k}s_total"] = int(table[:, 2 + j].sum())
+    return res
+
+
+def gather_peak_rows(sh: dict):
+    """(hit, waveform_width, s1_s2) rows of the WHOLE run on every rank, as HIT_DTYPE, WAVEFORM_WIDTH_DTYPE and
+    S1_S2_CLASSIFIER_DTYPE arrays (s1_s2 None when the leg ran without features).  Every rank receives every row,
+    like ``gather_rows``: for checks and small runs."""
+    from .dtypes import HIT_DTYPE, S1_S2_CLASSIFIER_DTYPE, WAVEFORM_WIDTH_DTYPE
+
+    def rows(t, n, dt):
+        n = int(n)
+        return _host(t[: n * dt.itemsize]).view(dt) if n else np.zeros(0, dtype=dt)
+
+    hits = gather_rows(rows(sh["hits"], sh["n_hits"], HIT_DTYPE))
+    widths = gather_rows(rows(sh["widths"], sh["n_widths"], WAVEFORM_WIDTH_DTYPE))
+    labels = None if sh["labels"] is None else gather_rows(rows(sh["labels"], sh["n_labels"], S1_S2_CLASSIFIER_DTYPE))
+    return hits, widths, labels

@@ -330,6 +330,27 @@ def waveform_width(hits: np.ndarray, wave_record_ids: np.ndarray, waves: np.ndar
     return rows[keep].copy()
 
 
+def waveform_width_run(run: DeviceRun, d_hits, n_hits: int, *, sampling_rate=None, rise_low=0.1, rise_high=0.9, fall_high=0.9,
+                       fall_low=0.1, interpolation=True):
+    """``waveform_width`` for packed HIT_DTYPE rows that live on the device (``d_hits``, uint8 tensor) against a
+    device-resident run, a time shard included: a hit's waveform is run row ``record_id - run.row_base`` when that row
+    holds the record, its samples the record's own event_length samples (float32 pool: the filtered_waveforms rows,
+    16-bit pool: the st_waveforms rows read as int16).  Returns (WAVEFORM_WIDTH rows as a device uint8 tensor in hit
+    order, row count); only the count crosses PCIe."""
+    lib = _lib.load()
+    torch = _torch()
+    n_hits = int(n_hits)
+    p = _lib.WidthParams(float(rise_low), float(rise_high), float(fall_high), float(fall_low), float(0.5 if sampling_rate is None else sampling_rate),
+                         1 if interpolation else 0, int(run.pool_is_f32))
+    out = _empty(n_hits * WAVEFORM_WIDTH_DTYPE.itemsize)
+    count = torch.zeros(1, dtype=torch.int64, device="cuda")
+    ws = _empty(lib.wfb_waveform_width_run_workspace_bytes(n_hits))
+    _lib.check(lib.wfb_waveform_width_run(_ptr(run.pool), run.pool_is_f32, run.pool_len, _ptr(run.meta), run.n, run.pool_base, run.row_base,
+                                          _ptr(d_hits) if n_hits else None, n_hits, C.byref(p), _ptr(out), _ptr(count), _ptr(ws), ws.numel(),
+                                          _stream()), "wfb_waveform_width_run")
+    return out, int(count.item())
+
+
 def width_integral(records: np.ndarray, pool: np.ndarray, *, q_low=0.10, q_high=0.90, sampling_rate=0.5, dt=None,
                    run: DeviceRun | None = None, signed_samples: bool = False) -> np.ndarray:
     """Per-record cumulative-charge quantile widths (waveform_width_integral.py:83-231).  ``signed_samples``: the
@@ -747,7 +768,7 @@ def find_peaks_launch(run: DeviceRun, kind: int, lmax: int, *, use_derivative=Tr
                         has_threshold=int(threshold is not None), distance=int(distance if distance is not None else 1),
                         height_method=0 if height_method == "minmax" else (2 if cumsum_diff else 1),
                         height_window_extension=int(height_window_extension),
-                        lmax=int(lmax), level_f32=int(bool(level_f32)))
+                        lmax=int(lmax), level_f32=int(bool(level_f32)), pool_base=run.pool_base)
     ws = _empty(lib.wfb_find_peaks_workspace_bytes(n))
     total = torch.zeros(1, dtype=torch.int64, device="cuda")
     cap = max(1024, 2 * n) if cap is None else int(cap)
@@ -759,8 +780,9 @@ def find_peaks_launch(run: DeviceRun, kind: int, lmax: int, *, use_derivative=Tr
     return dict(run=run, params=p, ws=ws, total=total, total_h=total_h, rows=rows, cap=cap)
 
 
-def find_peaks_collect(job: dict) -> np.ndarray:
-    """Wait for a ``find_peaks_launch`` and return its HIT_DTYPE rows (launches again if the row buffer was too small)."""
+def find_peaks_finish(job: dict):
+    """Wait for a ``find_peaks_launch`` and return its HIT_DTYPE rows as (device uint8 tensor, row count); launches
+    again with a row buffer of the right size when the first one was too small."""
     from .dtypes import HIT_DTYPE
 
     lib = _lib.load()
@@ -776,6 +798,21 @@ def find_peaks_collect(job: dict) -> np.ndarray:
         _lib.check(lib.wfb_find_peaks(_ptr(run.pool), run.pool_len, _ptr(run.meta), run.n, C.byref(p), _ptr(rows), cap, C.c_void_p(0),
                                       _ptr(job["total"]), _ptr(job["ws"]), job["ws"].numel(), _stream()), "wfb_find_peaks")
         nt = int(job["total"].item())
+    return rows, nt
+
+
+def find_peaks_device(run: DeviceRun, kind: int, lmax: int, **opts):
+    """``wfb_find_peaks`` on a device-resident run (a time shard included: the records sources read
+    ``wave_offset - run.pool_base``): (packed HIT_DTYPE rows as a device uint8 tensor, row count).  The rows stay on
+    the device; ``opts`` as ``find_peaks_launch`` takes them."""
+    return find_peaks_finish(find_peaks_launch(run, kind, lmax, **opts))
+
+
+def find_peaks_collect(job: dict) -> np.ndarray:
+    """Wait for a ``find_peaks_launch`` and return its HIT_DTYPE rows on the host."""
+    from .dtypes import HIT_DTYPE
+
+    rows, nt = find_peaks_finish(job)
     return rows[: nt * HIT_DTYPE.itemsize].cpu().numpy().view(HIT_DTYPE).copy()
 
 
@@ -949,8 +986,6 @@ def s1s2_classify(widths: np.ndarray, features: np.ndarray, *, width_unit: str =
     already normalised (a (None, None) range is passed as None)."""
     from .dtypes import BASIC_FEATURES_DTYPE, S1_S2_CLASSIFIER_DTYPE, WAVEFORM_WIDTH_DTYPE
 
-    lib = _lib.load()
-    torch = _torch()
     widths = np.ascontiguousarray(widths)
     features = np.ascontiguousarray(features)
     if widths.dtype != WAVEFORM_WIDTH_DTYPE or features.dtype != BASIC_FEATURES_DTYPE:
@@ -958,16 +993,34 @@ def s1s2_classify(widths: np.ndarray, features: np.ndarray, *, width_unit: str =
     n = len(widths)
     if n == 0:
         return np.zeros(0, dtype=S1_S2_CLASSIFIER_DTYPE)
+    out = s1s2_classify_device(_dev(widths), n, _dev(features) if len(features) else _empty(16), len(features), feat_row_base=0,
+                               width_unit=width_unit, s1_width_range=s1_width_range, s2_width_range=s2_width_range,
+                               s1_area_range=s1_area_range, s2_area_range=s2_area_range, s1_height_range=s1_height_range,
+                               s2_height_range=s2_height_range, conflict_policy=conflict_policy)
+    return out.cpu().numpy().view(S1_S2_CLASSIFIER_DTYPE)
+
+
+def s1s2_classify_device(d_widths, n: int, d_feat, n_feat: int, *, feat_row_base: int = 0, width_unit: str = "ns", s1_width_range=None,
+                         s2_width_range=None, s1_area_range=None, s2_area_range=None, s1_height_range=None, s2_height_range=None,
+                         conflict_policy: str = "unknown"):
+    """``s1s2_classify`` on packed rows that live on the device (uint8 tensors): ``n`` WAVEFORM_WIDTH rows and
+    ``n_feat`` BASIC_FEATURES rows, the first of them for record ``feat_row_base`` (a time shard's ``row_base``).
+    Returns the S1_S2_CLASSIFIER rows as a device uint8 tensor (45 B per row); the same normalised ranges."""
+    from .dtypes import S1_S2_CLASSIFIER_DTYPE
+
+    lib = _lib.load()
+    torch = _torch()
+    n = int(n)
     p = _lib.S1S2Params()
     p.s1_width, p.s1_area, p.s1_height = _range_struct(s1_width_range), _range_struct(s1_area_range), _range_struct(s1_height_range)
     p.s2_width, p.s2_area, p.s2_height = _range_struct(s2_width_range), _range_struct(s2_area_range), _range_struct(s2_height_range)
     p.width_in_samples = 1 if width_unit == "samples" else 0
     p.conflict_policy = {"unknown": 0, "prefer_s1": 1, "prefer_s2": 2}[conflict_policy]
-    d_w = _dev(widths)
-    d_f = _dev(features) if len(features) else _empty(16)
-    out = torch.empty(n * S1_S2_CLASSIFIER_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
-    _lib.check(lib.wfb_s1s2_classify(_ptr(d_w), n, _ptr(d_f), len(features), C.byref(p), _ptr(out), _stream()), "wfb_s1s2_classify")
-    return out.cpu().numpy().view(S1_S2_CLASSIFIER_DTYPE)
+    p.feat_row_base = int(feat_row_base)
+    out = torch.empty(max(n, 1) * S1_S2_CLASSIFIER_DTYPE.itemsize, dtype=torch.uint8, device="cuda")[: n * S1_S2_CLASSIFIER_DTYPE.itemsize]
+    _lib.check(lib.wfb_s1s2_classify(_ptr(d_widths) if n else None, n, _ptr(d_feat) if n_feat else None, int(n_feat), C.byref(p), _ptr(out),
+                                     _stream()), "wfb_s1s2_classify")
+    return out
 
 
 def pair_events(offsets: np.ndarray, member_ts: np.ndarray, member_area: np.ndarray, member_height: np.ndarray, dt_ns: np.ndarray,
