@@ -138,6 +138,23 @@ int wfb_meta_stats(const wfb_rec_meta* meta_dev, int64_t n, int32_t* scratch_dev
  * source's event_length (hit_finder.py:183-230, 388-391).  Lengths up to 2^24 - 2. */
 int wfb_meta_set_clamp(wfb_rec_meta* meta_dev, int64_t n, const int32_t* clamp_len_dev, void* stream);
 
+/* ---- per-channel tables -------------------------------------------------------------------------------------------
+ * A channel's key is board * 65536 + (channel & 0xFFFF) (the order of channel_config.unique_channels).  Key tables are
+ * sorted, without duplicates, and hold at most WFB_MAX_CHANNEL_KEYS entries (they are staged in shared memory). */
+#define WFB_MAX_CHANNEL_KEYS 8192
+
+typedef struct wfb_polarity_entry {
+    int32_t key;
+    uint32_t image[8]; /* the 32 bytes of the RECORDS_DTYPE polarity field (U8, UTF-32) */
+} wfb_polarity_entry;
+
+/* records["polarity"] from channel metadata (records.py:40-63 of the reference): every record whose key is in the table
+ * gets the entry's image in its packed row (records_aos_dev, may be NULL) and the matching WFB_POL_* code in its
+ * wfb_rec_meta, decoded the way wfb_records_unpack decodes rows.  Other records, and the edge clamp in pad_, are left
+ * as they are.  One thread per record. */
+int wfb_apply_polarity(wfb_rec_meta* meta_dev, void* records_aos_dev, int64_t n, const wfb_polarity_entry* table_dev,
+                       int32_t n_table, void* stream);
+
 /* Raw int16 rows -> time-sorted records + wave_pool.  Replaces
  * _build_records_part_from_raw_array + _records_sort_order + _merge_records_part_refs
  * (core/processing/records_builder.py:212-302, 115-120, 341-426).
@@ -232,7 +249,7 @@ int wfb_release_cache(void);
 #define WFB_MAX_SG_WINDOW 129
 #define WFB_MAX_SOS_SECTIONS 16
 
-/* One filter configuration (host side builds one per distinct (board, channel) config;
+/* One filter configuration (host side builds one per distinct resolved configuration;
  * filtering.py:47-130).  SG: taps = savgol coefficients (window), edge = (halflen x window)
  * projection rows for the first half-window (the last half-window uses the mirrored rows).
  * BW: sos[n_sections][6] and zi[n_sections][2] (sosfilt_zi). */
@@ -261,6 +278,15 @@ int wfb_filter_pool(const void* pool_dev, int32_t pool_is_f32, int64_t pool_len,
 /* Scratch for the Butterworth forward pass (float64, one row of lmax + 2*padlen per resident
  * thread); SG-only runs may pass a NULL workspace. */
 size_t wfb_filter_workspace_bytes(int64_t n, int32_t lmax);
+
+/* The per-record arguments of wfb_filter_pool, one thread per record: cfg_index_out[i] = cfg_of_key_dev[j] for the
+ * entry j of keys_dev that holds record i's channel key, default_cfg when there is none.  For an SG configuration c
+ * (sg_lut_off_of_cfg_dev[c] >= 0), sg_table_offset_out[i] = sg_lut_dev[sg_lut_off_of_cfg_dev[c] + min(max(L, 0),
+ * sg_wcap_of_cfg_dev[c])] with L the record's event_length: the host lists the table offset of each effective window
+ * min(window, L) (forced odd, -1 = identity when <= poly) for L = 0 .. wcap.  Otherwise -1. */
+int wfb_filter_plan(const wfb_rec_meta* meta_dev, int64_t n, const int32_t* keys_dev, const int32_t* cfg_of_key_dev, int32_t n_keys,
+                    int32_t default_cfg, const int32_t* sg_lut_dev, const int32_t* sg_lut_off_of_cfg_dev, const int32_t* sg_wcap_of_cfg_dev,
+                    int32_t* cfg_index_out, int32_t* sg_table_offset_out, void* stream);
 
 /* ---- waveform_width / waveform_width_integral --------------------------------------------- */
 

@@ -45,7 +45,13 @@ only peaks above the row's baseline): ``distributed.peaks_sharded`` with the SG 
 2), waveform_width (0.25 GHz) and s1_s2 on the shard's basic_features.  It reports the row counts, the time of every
 stage (each ended by a device synchronize) and the peak extra device memory of the leg; with --verify 1 rank 0 runs
 the same chain on the whole run (the rank-order concatenation of the shards) and checks the gathered filtered pool,
-hit, waveform_width and s1_s2 rows byte for byte."""
+hit, waveform_width and s1_s2 rows byte for byte.
+
+--peaks --channels runs the leg as a detector whose channels are not configured alike: the polarity comes from a
+channel map (even channels positive, odd channels left unknown; ``ops.apply_polarity``, its time reported as
+``polarity``) instead of marking every record positive, and the filter from ``B200WavePoolFilteredPlugin`` options with
+a ``channel_config`` that gives a quarter of the channels a Butterworth band-pass (order 4, 0.01-0.1 at 0.25 GHz) and
+leaves the rest on SG 11/2; --verify 1 compares with the same chain on the whole run."""
 import argparse
 import os
 import sys
@@ -72,6 +78,7 @@ ap.add_argument("--samples", type=int, default=800)
 ap.add_argument("--events", action="store_true", help="also run the sharded df -> df_events -> df_paired leg")
 ap.add_argument("--hit-events", action="store_true", help="also build the sharded hit_grouped event table")
 ap.add_argument("--peaks", action="store_true", help="also run the sharded filter -> hit -> waveform_width -> s1_s2 leg")
+ap.add_argument("--channels", action="store_true", help="--peaks with a polarity map and per-channel filters")
 args = ap.parse_args()
 
 D.init_process_group("nccl")
@@ -204,7 +211,7 @@ elif args.source == "raw":
     widths = f"{L} and {L - L // 4}" if args.mixed_widths else f"{L}"
     run, n, n_all = report_ingest(f"raw ingest: world={ws} groups={G} widths={widths}", wall, peak)
 else:
-    run = engine.DeviceRun.synth(n, L, NCH, seed=SEED, record_base=rank * n)
+    run = engine.DeviceRun.synth(n, L, NCH, seed=SEED, record_base=rank * n, with_rows=args.channels)
 res, total = fused(run)
 if ws > 1:
     dist.barrier()
@@ -337,17 +344,39 @@ WIDTH_OPTS = {"sampling_rate": 0.25}
 S1S2_OPTS = {"s1_width_range": (None, 60.0), "s2_width_range": (40.0, None), "conflict_policy": "prefer_s2"}
 
 
+# --channels: the same map and filter options on every rank (every board a run of up to 64 files can have)
+CH_POLARITY = {(b, c): "positive" if c % 2 == 0 else "unknown" for b in range(64) for c in range(NCH)}
+CH_FILTER = {"filter_type": "SG", "sg_window_size": 11, "sg_poly_order": 2, "filter_order": 4, "lowcut": 0.01, "highcut": 0.1, "fs": 0.25}
+CH_CONFIG = {"channels": {f"{b}:{c}": {"filter_type": "BW"} for b in range(64) for c in range(0, NCH, 4)}}
+
+
 def positive_copy(r):
     """A copy of a run with positive pulses, as bench.py's c3 leg makes them: samples and baselines mirrored around the
-    14-bit mid-scale, records marked positive (waveform_width keeps only peaks above the row's baseline)."""
+    14-bit mid-scale, records marked positive (waveform_width keeps only peaks above the row's baseline); with
+    --channels the polarity comes from CH_POLARITY instead.  Returns the copy and the seconds of ops.apply_polarity."""
     meta = r.meta.clone()
     m = meta.view(-1, 48)
     base = m[:, 8:16].contiguous().view(torch.float64).view(-1)
     m[:, 8:16] = (16383.0 - base).view(torch.uint8).view(-1, 8)
-    m[:, 36] = 1  # WFB_POL_POSITIVE
-    out = engine.DeviceRun(meta, 16383 - r.pool, r.n, 0, r.lmax, records_rows=r.records_rows, pool_base=r.pool_base, row_base=r.row_base)
+    rows = r.records_rows
+    if not args.channels:
+        m[:, 36] = 1  # WFB_POL_POSITIVE
+    elif rows is not None:
+        rows = rows.clone()
+    out = engine.DeviceRun(meta, 16383 - r.pool, r.n, 0, r.lmax, records_rows=rows, pool_base=r.pool_base, row_base=r.row_base)
     out.lmin = r.lmin
-    return out
+    t_pol = 0.0
+    if args.channels:
+        torch.cuda.synchronize()
+        t = time.perf_counter()
+        ops.apply_polarity(out, CH_POLARITY)
+        torch.cuda.synchronize()
+        t_pol = time.perf_counter() - t
+    return out, t_pol
+
+
+def peaks_filter() -> dict:
+    return dict(filter_options=CH_FILTER, channel_config=CH_CONFIG, run_id="run") if args.channels else dict(filter_cfg=PEAK_FILTER)
 
 
 def peaks_rows_host(x: dict):
@@ -360,25 +389,30 @@ def peaks_rows_host(x: dict):
 def peaks_leg() -> str:
     """filter -> hit -> waveform_width -> s1_s2 on this rank's shard (positive copy) with distributed.peaks_sharded; with
     --verify rank 0 runs the same chain on the whole run (the rank-order concatenation of the shards) on its GPU."""
-    prun = positive_copy(run)
+    positive_copy(run)  # warm-up: the first launch of the polarity kernel loads the module
+    prun, t_pol = positive_copy(run)
     feats = prun.features_hits(hits=False)["features"]
+    if args.channels:  # warm-up: the first Butterworth design imports scipy.signal
+        ops.filter_run_device(prun, **peaks_filter())
     torch.cuda.synchronize()
     torch.cuda.reset_peak_memory_stats()
     base_mem = torch.cuda.memory_allocated()
     if ws > 1:
         dist.barrier()
     t = time.perf_counter()
-    ph = D.peaks_sharded(prun, filter_cfg=PEAK_FILTER, features=feats, peak_opts=PEAK_OPTS, width_opts=WIDTH_OPTS, s1s2_opts=S1S2_OPTS)
+    ph = D.peaks_sharded(prun, features=feats, peak_opts=PEAK_OPTS, width_opts=WIDTH_OPTS, s1s2_opts=S1S2_OPTS, **peaks_filter())
     torch.cuda.synchronize()
     wall = time.perf_counter() - t
     peak = torch.cuda.max_memory_allocated() - base_mem
     line = (f"rank {rank}: records {prun.n} hits {ph['n_hits']} widths {ph['n_widths']} labels {ph['n_labels']} (bases {ph['hit_base']} / "
-            f"{ph['width_base']} / {ph['label_base']}) | " + " ".join(f"{k} {1e3 * v:.1f} ms" for k, v in ph["timings"].items()) +
+            f"{ph['width_base']} / {ph['label_base']}) | " + (f"polarity {1e3 * t_pol:.2f} ms " if args.channels else "") + " ".join(f"{k} {1e3 * v:.1f} ms" for k, v in ph["timings"].items()) +
             f" | leg wall {1e3 * wall:.1f} ms | peak extra device memory {peak / 1e9:.3f} GB "
             f"({peak / max(2 * prun.pool_len, 1):.2f} x the shard's 16-bit sample bytes) | {gpu_name()}")
     lines = D.gather_rows(np.frombuffer(line.encode().ljust(1024)[:1024], dtype="S1024")) if ws > 1 else [line.encode()]
     if rank == 0:
-        print(f"peaks leg: world={ws} records/rank={n} samples/record={L} filter SG 11/2, hit height 8 width 2, waveform_width 0.25 GHz")
+        what = ("polarity map (even channels positive, odd unknown), filter per channel (BW order 4 on a quarter, SG 11/2 on the rest)"
+                if args.channels else "filter SG 11/2")
+        print(f"peaks leg: world={ws} records/rank={n} samples/record={L} {what}, hit height 8 width 2, waveform_width 0.25 GHz")
         for ln in lines:
             print("  " + ln.decode().strip())
     out = f"peaks: hits={ph['n_hits_total']} widths={ph['n_widths_total']} labels={ph['n_labels_total']}"
@@ -394,9 +428,9 @@ def peaks_leg() -> str:
         return out
     torch.cuda.empty_cache()
     whole = engine.DeviceRun.from_host(recs_all, pool_all) if ingest is not None else engine.DeviceRun.synth(n * ws, L, NCH, seed=SEED)
-    whole = positive_copy(whole)
-    want = D.peaks_local(whole, filter_cfg=PEAK_FILTER, features=whole.features_hits(hits=False)["features"], peak_opts=PEAK_OPTS,
-                         width_opts=WIDTH_OPTS, s1s2_opts=S1S2_OPTS)
+    whole, _ = positive_copy(whole)
+    want = D.peaks_local(whole, features=whole.features_hits(hits=False)["features"], peak_opts=PEAK_OPTS, width_opts=WIDTH_OPTS,
+                         s1s2_opts=S1S2_OPTS, **peaks_filter())
     assert want["filtered"].cpu().numpy().tobytes() == got_sg.tobytes(), "filtered pool differs"
     for name, g, w in zip(("hit", "waveform_width", "s1_s2"), got, peaks_rows_host(want)):
         assert g.tobytes() == w, f"{name} rows differ"

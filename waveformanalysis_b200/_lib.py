@@ -25,6 +25,7 @@ DO_FEATURES = 1
 DO_HITS = 2
 SLICE_END_NONE = 2**63 - 1
 MAX_SOS_SECTIONS = 16
+MAX_CHANNEL_KEYS = 8192
 
 
 class RecMeta(C.Structure):
@@ -167,6 +168,8 @@ PROTOTYPES = {
     "wfb_hit_merge": (C.c_int, [_vp, _i64, _dbl, _dbl, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "wfb_filter_pool": (C.c_int, [_vp, _i32, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _sz, _i32, _vp]),
     "wfb_filter_workspace_bytes": (_sz, [_i64, _i32]),
+    "wfb_filter_plan": (C.c_int, [_vp, _i64, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "wfb_apply_polarity": (C.c_int, [_vp, _vp, _i64, _vp, _i32, _vp]),
     "wfb_waveform_width": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64, C.POINTER(WidthParams), _vp, _vp, _vp]),
     "wfb_waveform_width_run_workspace_bytes": (_sz, [_i64]),
     "wfb_waveform_width_run": (C.c_int, [_vp, _i32, _i64, _vp, _i64, _i64, _i64, _vp, _i64, C.POINTER(WidthParams), _vp, _vp, _vp, _sz, _vp]),

@@ -122,15 +122,11 @@ __device__ __forceinline__ unsigned long long rd64(const uint16_t* h) {
 }
 __device__ __forceinline__ unsigned rd32(const uint16_t* h) { return (unsigned)h[0] | ((unsigned)h[1] << 16); }
 
-__device__ __forceinline__ wfb_rec_meta rec_meta_from_row(const uint16_t* h) {
-    wfb_rec_meta m;
-    m.timestamp = (long long)rd64(h + 0);
-    m.board = (short)h[6];
-    m.channel = (short)h[7];
-    m.baseline = __longlong_as_double((long long)rd64(h + 8));
-    // polarity: 'positive' / 'negative' / other, compared on the first UTF-32 code units and the
-    // terminator so that e.g. 'pos' is not mistaken for 'positive'
-    unsigned c0 = rd32(h + 16), c1 = rd32(h + 18), c7 = rd32(h + 30);
+// The WFB_POL_* code of a polarity field (U8: 8 UTF-32 code units as 16 half-words): 'positive' / 'negative' / other,
+// compared on the first code units and the last one so that e.g. 'pos' is not mistaken for 'positive'.  The one place
+// that maps polarity strings to codes (wfb_records_unpack, wfb_apply_polarity).
+__device__ __forceinline__ int polarity_code(const uint16_t* p) {
+    unsigned c0 = rd32(p), c1 = rd32(p + 2), c7 = rd32(p + 14);
     int pol = WFB_POL_UNKNOWN;
     if (c7 == 'e') {
         // full 8-character compare
@@ -138,7 +134,7 @@ __device__ __forceinline__ wfb_rec_meta rec_meta_from_row(const uint16_t* h) {
         const char* neg = "negative";
         bool isp = true, isn = true;
         for (int k = 0; k < 8; ++k) {
-            unsigned ck = rd32(h + 16 + 2 * k);
+            unsigned ck = rd32(p + 2 * k);
             isp = isp && ck == (unsigned)pos[k];
             isn = isn && ck == (unsigned)neg[k];
         }
@@ -147,10 +143,19 @@ __device__ __forceinline__ wfb_rec_meta rec_meta_from_row(const uint16_t* h) {
     if (c0 == 'r' && c1 == 'a') {  // internal tag "rawpos" (waveformanalysis_b200/aos.py)
         const char* rp = "rawpos";
         bool isr = true;
-        for (int k = 0; k < 8; ++k) isr = isr && rd32(h + 16 + 2 * k) == (k < 6 ? (unsigned)rp[k] : 0u);
+        for (int k = 0; k < 8; ++k) isr = isr && rd32(p + 2 * k) == (k < 6 ? (unsigned)rp[k] : 0u);
         if (isr) pol = WFB_POL_RAW_POSITIVE;
     }
-    m.polarity = (uint8_t)pol;
+    return pol;
+}
+
+__device__ __forceinline__ wfb_rec_meta rec_meta_from_row(const uint16_t* h) {
+    wfb_rec_meta m;
+    m.timestamp = (long long)rd64(h + 0);
+    m.board = (short)h[6];
+    m.channel = (short)h[7];
+    m.baseline = __longlong_as_double((long long)rd64(h + 8));
+    m.polarity = (uint8_t)polarity_code(h + 16);
     m.pad_[0] = m.pad_[1] = m.pad_[2] = 0;
     m.record_id = (long long)rd64(h + 32);
     m.dt = (int)rd32(h + 36);

@@ -754,6 +754,15 @@ class HostRecords:
 
         return SimpleNamespace(records=shard[0], pool=shard[1], n=len(shard[0]), lmax=lmax, pool_base=pool_base, row_base=record_base)
 
+    def apply_polarity(self, run, polarity):
+        """The numpy assignment of plugins.records._apply_polarity."""
+        from .ops import polarity_entries
+
+        rec = run.records
+        for b, c, v in polarity_entries(polarity):
+            if v != "unknown":
+                rec["polarity"][(rec["board"] == b) & (rec["channel"] == c)] = v
+
 
 class DeviceRecords:
     """Backend for the records of a rank on its GPU: libwfb200's scan, build (with seq), split points and merge."""
@@ -849,8 +858,13 @@ class DeviceRecords:
         rows, pool, meta, n = shard
         return DeviceRun(meta, pool, n, 0, lmax, records_rows=rows, pool_base=pool_base, row_base=record_base)
 
+    def apply_polarity(self, run, polarity):
+        from . import ops
 
-def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None) -> dict:
+        ops.apply_polarity(run, polarity)
+
+
+def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None, polarity: dict | None = None) -> dict:
     """This rank's time shard of the V1725 run made of ``paths`` (the full ordered file list, the same on every rank;
     file names give the board id), without any process holding the whole run.
 
@@ -862,7 +876,11 @@ def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None) -
     pool slice, the run-wide longest record as ``lmax``: ``run.features_hits`` gives global event indices and
     ``merge_group_sharded`` takes its hits unchanged), ``record_base``, ``n_total``, ``records_per_rank``,
     ``exchange_bytes`` (row and sample bytes this rank received from the other ranks) and ``timings`` (seconds per
-    stage, each ended by a device synchronize)."""
+    stage, each ended by a device synchronize).
+
+    ``polarity``: {(board, channel): "positive" | "negative" | "unknown"}, applied to the shard's records as
+    ``plugins.records`` applies the channel metadata to a single-GPU build (``ops.apply_polarity``).  It must be the
+    same on every rank; maps that differ, or an invalid map on any rank, raise ValueError on every rank."""
     import time
 
     backend = backend if backend is not None else DeviceRecords()
@@ -871,6 +889,7 @@ def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None) -
     F = len(paths)
     T: dict = {}
     err = None
+    pol_err, pol_digest = _polarity_digest(polarity)
 
     if mine is None:
         sizes = []
@@ -904,16 +923,17 @@ def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None) -
             T["scan"] = time.perf_counter() - t
     except (OSError, ValueError) as e:
         err = e
-    status = np.zeros(F + 1, dtype=np.int64)
-    status[0] = int(err is not None)
+    status = np.zeros(F + 3, dtype=np.int64)
+    status[:3] = [int(err is not None), int(pol_err is not None), pol_digest]
     for f, s in zip(own, scans):
-        status[1 + f] = len(s["channel"])
+        status[3 + f] = len(s["channel"])
     table = _allgather_i64(status)
     if table[:, 0].any():
         if err is not None:
             raise err
         raise RuntimeError(f"ranks {np.flatnonzero(table[:, 0]).tolist()} could not read their V1725 files")
-    counts = table[:, 1:].sum(axis=0)
+    _check_polarity(table[:, 1], table[:, 2], pol_err)
+    counts = table[:, 3:].sum(axis=0)
     seq_base = np.cumsum(counts) - counts
     seq = np.concatenate([seq_base[f] + np.arange(counts[f], dtype=np.int64) for f in own] or [np.zeros(0, np.int64)])
 
@@ -928,14 +948,35 @@ def build_records_sharded_v1725(paths, *, dt_ns: int, mine=None, backend=None) -
     del up  # the stream bytes
     backend.sync()
     T["build"] = time.perf_counter() - t
-    return _time_shard(built, backend, T)
+    return _time_shard(built, backend, T, polarity)
 
 
-def _time_shard(built: list, backend, T: dict) -> dict:
+def _polarity_digest(polarity) -> tuple:
+    """(the ValueError of an invalid map or None, digest of the validated map)."""
+    from .ops import polarity_entries
+
+    try:
+        return None, _digest(polarity_entries(polarity))
+    except ValueError as e:
+        return e, 0
+
+
+def _check_polarity(bad, digests, own_err) -> None:
+    """Raise on every rank when a rank's polarity map is invalid or the maps differ (gathered flag / digest columns)."""
+    if np.any(bad):
+        if own_err is not None:
+            raise own_err
+        raise ValueError(f"ranks {np.flatnonzero(bad).tolist()} were given an invalid polarity map")
+    if np.any(digests != digests[0]):
+        raise ValueError("polarity must be the same on every rank")
+
+
+def _time_shard(built: list, backend, T: dict, polarity: dict | None = None) -> dict:
     """Stages 2-6 of the distributed time sort on a rank's locally built rows (record_id = global seq, sorted by
-    (timestamp, board, channel, seq)): splitters, split points, exchange, global bases, merge, run-wide lmax.
-    ``built`` holds the local build and is emptied, so that the rows are freed once they are sent; ``T`` gets the
-    stage timings.  Returns the dict of build_records_sharded_v1725."""
+    (timestamp, board, channel, seq)): splitters, split points, exchange, global bases, merge, run-wide lmax, then the
+    polarity map (validated by the caller) on the merged records.  ``built`` holds the local build and is emptied, so
+    that the rows are freed once they are sent; ``T`` gets the stage timings.  Returns the dict of
+    build_records_sharded_v1725."""
     import time
 
     _, rank, P = _dist()
@@ -974,7 +1015,13 @@ def _time_shard(built: list, backend, T: dict) -> dict:
     backend.sync()
     T["merge"] = time.perf_counter() - t
     lmax = _allreduce_max(backend.lmax(shard))
-    return dict(run=backend.run(shard, lmax, record_base, pool_base), record_base=record_base, pool_base=pool_base,
+    run = backend.run(shard, lmax, record_base, pool_base)
+    if polarity:
+        t = time.perf_counter()
+        backend.apply_polarity(run, polarity)
+        backend.sync()
+        T["polarity"] = time.perf_counter() - t
+    return dict(run=run, record_base=record_base, pool_base=pool_base,
                 n_total=int(bases[:, 0].sum()), records_per_rank=bases[:, 0].copy(), exchange_bytes=exchange_bytes, timings=T)
 
 
@@ -997,7 +1044,7 @@ def _check_group(g: int, cols) -> tuple:
 
 
 def build_records_sharded(groups, *, n_groups: int, dt_ns: int, baseline_window=(0, 40), epoch_ns: int | None = None,
-                          backend=None) -> dict:
+                          backend=None, polarity: dict | None = None) -> dict:
     """This rank's time shard of a run made of ``n_groups`` groups of raw rows, without any process holding the whole
     run: the result of ``ops.build_records`` / ``ops.build_records_ragged`` (as ``plugins.records.build_bundle`` picks
     them) on all groups concatenated in group-index order.
@@ -1011,12 +1058,14 @@ def build_records_sharded(groups, *, n_groups: int, dt_ns: int, baseline_window=
     Each row's seq is its index in the concatenation of all groups; every rank builds its own rows with record_id =
     seq (``wfb_build_records_ragged_seq``), which orders them by (timestamp, board, channel, seq), the single-GPU
     order, and the distributed time sort of build_records_sharded_v1725 does the rest.  Returns the same dict;
-    ``timings`` has h2d, build, splitters, exchange and merge."""
+    ``timings`` has h2d, build, splitters, exchange and merge (and polarity).  ``polarity`` as in
+    build_records_sharded_v1725."""
     import time
 
     backend = backend if backend is not None else DeviceRecords()
     T: dict = {}
     err = None
+    pol_err, pol_digest = _polarity_digest(polarity)
     own: list = []
     cols: list = []
     params = np.zeros(6, dtype=np.int64)
@@ -1032,13 +1081,14 @@ def build_records_sharded(groups, *, n_groups: int, dt_ns: int, baseline_window=
         err, own, cols = e, [], []
 
     # parameters and local errors first (fixed size, so a rank with different arguments cannot stall the gather)
-    table = _allgather_i64(np.r_[int(err is not None), params])
+    table = _allgather_i64(np.r_[int(err is not None), params, int(pol_err is not None), pol_digest])
     if table[:, 0].any():
         if err is not None:
             raise err
         raise ValueError(f"ranks {np.flatnonzero(table[:, 0]).tolist()} were given malformed row groups or arguments")
-    if np.any(table[:, 1:] != table[:1, 1:]):
+    if np.any(table[:, 1:7] != table[:1, 1:7]):
         raise ValueError("n_groups, dt_ns, baseline_window and epoch_ns must be the same on every rank")
+    _check_polarity(table[:, 7], table[:, 8], pol_err)
 
     # ownership, checked on the gathered claims so that every rank raises
     G = int(n_groups)
@@ -1067,7 +1117,7 @@ def build_records_sharded(groups, *, n_groups: int, dt_ns: int, baseline_window=
     del up
     backend.sync()
     T["build"] = time.perf_counter() - t
-    return _time_shard(built, backend, T)
+    return _time_shard(built, backend, T, polarity)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -1438,13 +1488,14 @@ def _sync():
 
 
 def peaks_local(run, *, filter_cfg: dict | None = None, features=None, peak_opts: dict | None = None, width_opts: dict | None = None,
-                s1s2_opts: dict | None = None) -> dict:
+                s1s2_opts: dict | None = None, filter_options: dict | None = None, channel_config=None, run_id: str | None = None) -> dict:
     """The filter -> hit -> waveform_width -> s1_s2 chain on ONE time shard (a ``DeviceRun`` with its own records and
     pool slice, ``pool_base`` / ``row_base`` set), with no collective.  Everything stays on the device.
 
-    1. ``filter_cfg`` (the form ``ops.filter_run_device`` takes: one configuration for every record; per-channel
-       configurations are not supported on a shard) filters the shard into a float32 pool; ``None`` keeps the raw
-       16-bit pool (the ``use_filtered=False`` route).
+    1. ``filter_cfg`` (one configuration for every record) or ``filter_options`` with ``channel_config`` and ``run_id``
+       (``B200WavePoolFilteredPlugin``'s options, resolved for each channel of the shard as the plugin resolves
+       them) filters the shard into a float32 pool through ``ops.filter_run_device``; neither keeps the raw 16-bit
+       pool (the ``use_filtered=False`` route).  Both is a ValueError.
     2. ``ops.find_peaks_device`` on those samples (``WFB_WAVE_REC_F32`` / ``WFB_WAVE_REC_U16``) with ``peak_opts``
        (``find_peaks_launch``'s options): the `hit` rows of ``B200HitFinderPlugin(wave_source="records")``.
     3. ``ops.waveform_width_run`` on the same samples with ``width_opts`` (sampling_rate, rise_low, rise_high,
@@ -1461,11 +1512,13 @@ def peaks_local(run, *, filter_cfg: dict | None = None, features=None, peak_opts
     from . import _lib, ops
     from .engine import DeviceRun
 
+    if filter_cfg is not None and filter_options is not None:
+        raise ValueError("peaks_local takes filter_cfg or filter_options, not both")
     T: dict = {}
     t = time.perf_counter()
     src, filtered = run, None
-    if filter_cfg is not None:
-        filtered = ops.filter_run_device(run, filter_cfg)
+    if filter_cfg is not None or filter_options is not None:
+        filtered = ops.filter_run_device(run, filter_cfg, filter_options=filter_options, channel_config=channel_config, run_id=run_id)
         src = DeviceRun(run.meta, filtered, run.n, 1, run.lmax, records_rows=run.records_rows, pool_base=run.pool_base, row_base=run.row_base)
         _sync()
         T["filter"] = time.perf_counter() - t
@@ -1492,33 +1545,65 @@ def peaks_local(run, *, filter_cfg: dict | None = None, features=None, peak_opts
                 timings=T)
 
 
-def peaks_options_digest(filter_cfg, with_features: bool, peak_opts, width_opts, s1s2_opts) -> int:
-    """64-bit digest of the options of the peaks leg, equal on every process for equal options."""
+def _canonical(x):
+    """A JSON-able form of an options tree that equal options share: mappings become key-sorted [key, value] pairs,
+    channel keys (HardwareChannel-like objects, (board, channel) pairs, "board:channel" strings) one form, arrays and
+    tuples lists."""
+    import json
+    from collections.abc import Mapping
+
+    from .channel_config import parse_channel_ref
+
+    if isinstance(x, Mapping):
+        items = []
+        for k, v in x.items():
+            ref = parse_channel_ref(k) if not isinstance(k, (int, float)) else None
+            items.append([["channel", *ref] if ref is not None else _canonical(k), _canonical(v)])
+        return ["map", sorted(items, key=lambda kv: json.dumps(kv[0]))]
+    if isinstance(x, (str, bool, int, float)) or x is None:
+        return x
+    if isinstance(x, (list, tuple)):
+        return [_canonical(v) for v in x]
+    if isinstance(x, (np.ndarray, np.generic)):
+        return np.asarray(x).tolist()
+    return repr(x)
+
+
+def _digest(x) -> int:
+    """64-bit digest of ``_canonical(x)``: equal on every process for equal options."""
     import hashlib
     import json
 
-    def plain(x):
-        return np.asarray(x).tolist()
-
-    blob = json.dumps([filter_cfg, bool(with_features), peak_opts or {}, width_opts or {}, s1s2_opts or {}], sort_keys=True, default=plain)
+    blob = json.dumps(_canonical(x))
     return int(np.frombuffer(hashlib.blake2b(blob.encode(), digest_size=8).digest(), dtype="<i8")[0])
 
 
+def peaks_options_digest(filter_cfg, with_features: bool, peak_opts, width_opts, s1s2_opts, *, filter_options=None, channel_config=None,
+                         run_id=None) -> int:
+    """64-bit digest of the options of the peaks leg, equal on every process for equal options."""
+    return _digest([filter_cfg, bool(with_features), peak_opts or {}, width_opts or {}, s1s2_opts or {}, filter_options, channel_config,
+                    run_id])
+
+
 def peaks_sharded(run, *, filter_cfg: dict | None = None, features=None, peak_opts: dict | None = None, width_opts: dict | None = None,
-                  s1s2_opts: dict | None = None, local_fn=None) -> dict:
+                  s1s2_opts: dict | None = None, filter_options: dict | None = None, channel_config=None, run_id: str | None = None,
+                  local_fn=None) -> dict:
     """``peaks_local`` on this rank's time shard plus ONE fixed-size all_gather (error flag, options digest, the three
     row counts).  Options that differ between ranks, or an error on any rank, raise ValueError on every rank (the
-    rank that failed raises its own error).  Per-channel filter configurations are not supported on shards.
+    rank that failed raises its own error).  With ``filter_options`` / ``channel_config`` each rank resolves the
+    filters of its own channels; the resolution depends on (run_id, board, channel) only, so the ranks agree.
 
     Returns ``peaks_local``'s result plus ``hit_base`` / ``width_base`` / ``label_base`` (global index of the rank's
     first row), ``hits_per_rank`` / ``widths_per_rank`` / ``labels_per_rank`` and the totals ``n_hits_total`` /
     ``n_widths_total`` / ``n_labels_total``.  ``local_fn`` replaces ``peaks_local`` (tests of the collective)."""
     local_fn = local_fn if local_fn is not None else peaks_local
     _, rank, _ = _dist()
-    digest = peaks_options_digest(filter_cfg, features is not None, peak_opts, width_opts, s1s2_opts)
-    err, res = None, {}
+    err, res, digest = None, {}, 0
     try:
-        res = local_fn(run, filter_cfg=filter_cfg, features=features, peak_opts=peak_opts, width_opts=width_opts, s1s2_opts=s1s2_opts)
+        digest = peaks_options_digest(filter_cfg, features is not None, peak_opts, width_opts, s1s2_opts, filter_options=filter_options,
+                                      channel_config=channel_config, run_id=run_id)
+        res = local_fn(run, filter_cfg=filter_cfg, features=features, peak_opts=peak_opts, width_opts=width_opts, s1s2_opts=s1s2_opts,
+                       filter_options=filter_options, channel_config=channel_config, run_id=run_id)
         counts = [int(res["n_hits"]), int(res["n_widths"]), int(res["n_labels"])]
     except Exception as e:  # noqa: BLE001 - every rank must reach the gather, the error is raised after it
         err, counts = e, [0, 0, 0]
@@ -1528,7 +1613,8 @@ def peaks_sharded(run, *, filter_cfg: dict | None = None, features=None, peak_op
             raise err
         raise ValueError(f"the peaks leg failed on ranks {np.flatnonzero(table[:, 0]).tolist()}")
     if np.any(table[:, 1] != table[0, 1]):
-        raise ValueError("filter_cfg, features (given or not), peak_opts, width_opts and s1s2_opts must be the same on every rank")
+        raise ValueError("filter_cfg, filter_options, channel_config, run_id, features (given or not), peak_opts, width_opts and s1s2_opts "
+                         "must be the same on every rank")
     me = rank if len(table) > 1 else 0
     res = dict(res)
     for j, k in enumerate(("hit", "width", "label")):
@@ -1552,3 +1638,23 @@ def gather_peak_rows(sh: dict):
     widths = gather_rows(rows(sh["widths"], sh["n_widths"], WAVEFORM_WIDTH_DTYPE))
     labels = None if sh["labels"] is None else gather_rows(rows(sh["labels"], sh["n_labels"], S1_S2_CLASSIFIER_DTYPE))
     return hits, widths, labels
+
+
+def channel_rules(run, channel_config, *, run_id: str | None, threshold: float, fixed_baseline: float | None = None) -> np.ndarray:
+    """The wfb_chan_rule array for ``run.features_hits(threshold=threshold, rules=...)`` on a time shard: the
+    ``threshold`` and ``fixed_baseline`` of each channel of the shard resolved from ``channel_config`` the way
+    ``B200ThresholdHitPlugin`` and ``B200BasicFeaturesPlugin`` resolve them for ``run_id`` (a rule only for a channel
+    whose threshold differs from ``threshold`` or that has a fixed baseline)."""
+    from .channel_config import resolve_channel_values
+    from .engine import make_rules
+    from .ops import shard_channels
+
+    base = {"threshold": threshold, "fixed_baseline": fixed_baseline}
+    thr, fixed = {}, {}
+    for b, c in shard_channels(run):
+        v = resolve_channel_values(channel_config, run_id, b, c, base)
+        if float(v["threshold"]) != float(threshold):
+            thr[(b, c)] = float(v["threshold"])
+        if v.get("fixed_baseline") is not None:
+            fixed[(b, c)] = float(v["fixed_baseline"])
+    return make_rules(thr, fixed)

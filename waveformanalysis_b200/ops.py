@@ -206,6 +206,185 @@ def sos_zi(sos: np.ndarray) -> np.ndarray:
     return zi
 
 
+# --------------------------------------------------------------------------------------------
+# per-channel tables: channel keys, polarity, filter plan
+# --------------------------------------------------------------------------------------------
+POLARITY_VALUES = ("positive", "negative", "unknown")
+POLARITY_ENTRY_DTYPE = np.dtype([("key", "<i4"), ("image", "<u4", 8)])  # wfb_polarity_entry
+assert POLARITY_ENTRY_DTYPE.itemsize == 36
+
+
+def channel_key(board: int, channel: int) -> int:
+    """The key the device tables are sorted by (channel_config.unique_channels' order)."""
+    return int(board) * 65536 + (int(channel) & 0xFFFF)
+
+
+def _in_i16(*v) -> bool:
+    return all(-32768 <= int(x) <= 32767 for x in v)
+
+
+def shard_channels(run: DeviceRun) -> list[tuple[int, int]]:
+    """The distinct (board, channel) pairs of a device run's records, sorted (``channel_config.unique_channels``)."""
+    torch = _torch()
+    n = run.n
+    if n == 0:
+        return []
+    bc = run.meta[: n * 48].view(n, 48)[:, 32:36].contiguous().view(torch.int16).view(n, 2).long()  # wfb_rec_meta board, channel
+    keys = torch.unique(bc[:, 0] * 65536 + (bc[:, 1] & 0xFFFF)).cpu().numpy()
+    return sorted((int(k) >> 16, ((int(k) & 0xFFFF) ^ 0x8000) - 0x8000) for k in keys.tolist())
+
+
+def polarity_entries(polarity: dict | None) -> list[tuple[int, int, str]]:
+    """The sorted (board, channel, value) entries of a polarity map {(board, channel): "positive" | "negative" |
+    "unknown"}.  Any other value, a key that is not a pair of integers, or one channel given two values raise
+    ValueError."""
+    out: dict[tuple[int, int], str] = {}
+    for k, v in dict(polarity or {}).items():
+        try:
+            b, c = (int(x) for x in k)
+        except (TypeError, ValueError):
+            raise ValueError(f"polarity keys are (board, channel) pairs, got {k!r}") from None
+        if not isinstance(v, str) or v not in POLARITY_VALUES:
+            raise ValueError(f"polarity of channel {(b, c)} must be one of {POLARITY_VALUES}, got {v!r}")
+        if out.setdefault((b, c), v) != v:
+            raise ValueError(f"channel {(b, c)} is given two polarities")
+    return sorted((b, c, v) for (b, c), v in out.items())
+
+
+def polarity_table(polarity: dict | None) -> np.ndarray:
+    """wfb_polarity_entry rows of a polarity map: its "positive" / "negative" channels sorted by key, each with the
+    UTF-32 image numpy stores for that string in a RECORDS_DTYPE polarity field.  "unknown" entries and channels
+    outside the int16 range of records' board / channel match no record change and are left out."""
+    ent = [(channel_key(b, c), v) for b, c, v in polarity_entries(polarity) if v != "unknown" and _in_i16(b, c)]
+    ent.sort()
+    table = np.zeros(len(ent), dtype=POLARITY_ENTRY_DTYPE)
+    for i, (k, v) in enumerate(ent):
+        table[i]["key"] = k
+        table[i]["image"] = np.array([v], dtype="U8").view(np.uint32)
+    if len(table) > _lib.MAX_CHANNEL_KEYS:
+        raise ValueError(f"a polarity map sets at most {_lib.MAX_CHANNEL_KEYS} channels, got {len(table)}")
+    return table
+
+
+def apply_polarity(run: DeviceRun, polarity: dict | None) -> None:
+    """records["polarity"] of a device run from a channel map, as plugins.records._apply_polarity sets it on host
+    records: every record of a "positive" / "negative" channel gets that value in ``run.records_rows`` (when the run
+    has them) and the matching code in ``run.meta``; records of other channels and of "unknown" channels keep theirs.
+    In place, on the current stream."""
+    table = polarity_table(polarity)
+    if run.n == 0 or len(table) == 0:
+        return
+    _lib.check(_lib.load().wfb_apply_polarity(_ptr(run.meta), _ptr(run.records_rows), run.n, _ptr(upload(table)), len(table), _stream()),
+               "wfb_apply_polarity")
+
+
+def _filter_cfg_struct(cfg: dict) -> "_lib.FilterCfg":
+    c = _lib.FilterCfg()
+    if cfg["filter_type"] == "BW":
+        sos = np.asarray(cfg["sos"], dtype=np.float64)
+        if sos.shape[0] > _lib.MAX_SOS_SECTIONS:
+            raise ValueError(f"filter_order too high: {sos.shape[0]} sections > {_lib.MAX_SOS_SECTIONS}")
+        zi = sos_zi(sos)
+        c.type, c.n_sections = 1, sos.shape[0]
+        for s in range(sos.shape[0]):
+            for j in range(6):
+                c.sos[s][j] = sos[s, j]
+            c.zi[s][0], c.zi[s][1] = zi[s, 0], zi[s, 1]
+    else:
+        c.type, c.sg_window, c.sg_poly = 0, int(cfg["sg_window_size"]), int(cfg["sg_poly_order"])
+    return c
+
+
+def filter_plan(run: DeviceRun, configs: dict, default: dict | None = None, *, lengths: np.ndarray | None = None) -> dict:
+    """The per-record arguments of wfb_filter_pool, planned on the device by wfb_filter_plan.
+
+    ``configs[(board, channel)]`` / ``default``: configurations as ``filter_pool`` takes them.  Without ``default``,
+    ``configs`` must hold every channel of the run.  One wfb_filter_cfg per DISTINCT configuration (so channels that
+    share one Butterworth filter take the uniform kernel), one Savitzky-Golay table per effective (window, poly); for
+    every SG configuration a table offset per record length 0 .. min(window, lmax).  ``lengths``: the record lengths
+    that occur (host records); otherwise those of [run.lmin, lmax], or of 0 .. lmax, get a table."""
+    torch = _torch()
+    distinct: list[dict] = []
+    at: dict = {}
+
+    def index(cfg: dict) -> int:
+        ident = (("BW", np.asarray(cfg["sos"], dtype=np.float64).tobytes()) if cfg["filter_type"] == "BW"
+                 else ("SG", int(cfg["sg_window_size"]), int(cfg["sg_poly_order"])))
+        if ident not in at:
+            at[ident] = len(distinct)
+            distinct.append(cfg)
+        return at[ident]
+
+    keyed = sorted((channel_key(b, c), index(cfg)) for (b, c), cfg in configs.items() if _in_i16(b, c))
+    default_cfg = index(default) if default is not None else 0
+    if not distinct:
+        raise ValueError("filter_plan: no filter configuration")
+    if len(keyed) > _lib.MAX_CHANNEL_KEYS:
+        raise ValueError(f"at most {_lib.MAX_CHANNEL_KEYS} per-channel filter configurations, got {len(keyed)}")
+    lmax = max(run.lmax, 0)
+    present = None
+    if lengths is not None:
+        present = np.unique(np.clip(np.asarray(lengths, dtype=np.int64), 0, lmax))
+    tables, table_at, cursor = [], {}, 0
+    lut_parts, lut_off, wcaps, lut_len = [], [], [], 0
+    for cfg in distinct:
+        if cfg["filter_type"] == "BW":
+            lut_off.append(-1)
+            wcaps.append(0)
+            continue
+        w0, poly = int(cfg["sg_window_size"]), int(cfg["sg_poly_order"])
+        wcap = min(w0, lmax)
+        need = np.zeros(wcap + 1, dtype=bool)
+        if present is not None:
+            need[np.minimum(present, wcap)] = True
+        else:
+            need[min(run.lmin or 0, wcap):] = True
+        lut = np.full(wcap + 1, -1, dtype=np.int32)
+        for L in np.flatnonzero(need).tolist():
+            w = min(w0, L)
+            w -= (w % 2 == 0)
+            if w <= poly or w <= 0:
+                continue  # identity (filtering.py:193-194, 231-232)
+            if (w, poly) not in table_at:
+                tables.append(sg_tables(w, poly))
+                table_at[(w, poly)] = cursor
+                cursor += len(tables[-1])
+            lut[L] = table_at[(w, poly)]
+        lut_parts.append(lut)
+        lut_off.append(lut_len)
+        wcaps.append(wcap)
+        lut_len += len(lut)
+    n = run.n
+    cfgs = (_lib.FilterCfg * len(distinct))(*[_filter_cfg_struct(c) for c in distinct])
+    plan = dict(
+        n_cfg=len(distinct), configs=distinct, has_bw=any(c["filter_type"] == "BW" for c in distinct),
+        d_cfg=upload(np.frombuffer(bytes(cfgs), dtype=np.uint8).copy()),
+        d_tab=upload(np.concatenate(tables) if tables else np.zeros(1)),
+        d_idx=torch.empty(max(n, 1), dtype=torch.int32, device="cuda"),
+        d_toff=torch.empty(max(n, 1), dtype=torch.int32, device="cuda"),
+    )
+    keys = np.array([k for k, _ in keyed] or [0], dtype=np.int32)
+    cfg_of_key = np.array([c for _, c in keyed] or [0], dtype=np.int32)
+    d_keys, d_cok = upload(keys), upload(cfg_of_key)
+    d_lut = upload(np.concatenate(lut_parts) if lut_parts else np.full(1, -1, np.int32))
+    d_off, d_wcap = upload(np.array(lut_off, dtype=np.int32)), upload(np.array(wcaps, dtype=np.int32))
+    _lib.check(_lib.load().wfb_filter_plan(_ptr(run.meta), n, _ptr(d_keys), _ptr(d_cok), len(keyed), default_cfg, _ptr(d_lut), _ptr(d_off),
+                                           _ptr(d_wcap), _ptr(plan["d_idx"]), _ptr(plan["d_toff"]), _stream()), "wfb_filter_plan")
+    return plan
+
+
+def _filter_launch(run: DeviceRun, plan: dict, pool_len: int, lmax: int):
+    """wfb_filter_pool on a planned run -> the float32 pool (device tensor)."""
+    lib = _lib.load()
+    torch = _torch()
+    d_out = torch.empty(pool_len + 16, dtype=torch.float32, device="cuda")[:pool_len]
+    ws = _empty(lib.wfb_filter_workspace_bytes(run.n, lmax)) if plan["has_bw"] else None
+    _lib.check(lib.wfb_filter_pool(_ptr(run.pool), run.pool_is_f32, pool_len, _ptr(run.meta), run.n, _ptr(plan["d_cfg"]), plan["n_cfg"],
+                                   _ptr(plan["d_idx"]), _ptr(plan["d_tab"]), _ptr(plan["d_toff"]), _ptr(d_out), run.pool_base, _ptr(ws),
+                                   0 if ws is None else ws.numel(), lmax, _stream()), "wfb_filter_pool")
+    return d_out
+
+
 def filter_pool(records: np.ndarray, pool: np.ndarray, *, configs: dict, default: dict, run: DeviceRun | None = None,
                 return_device: bool = False):
     """uint16 wave_pool -> float32 wave_pool_filtered (records.py:368-438).
@@ -213,74 +392,24 @@ def filter_pool(records: np.ndarray, pool: np.ndarray, *, configs: dict, default
     ``default`` / ``configs[(board, channel)]``: {"filter_type": "SG", "sg_window_size", "sg_poly_order"} or
     {"filter_type": "BW", "sos": ndarray (n_sections, 6)}.
     """
-    lib = _lib.load()
-    torch = _torch()
+    from .channel_config import unique_channels
+
     pool_h, is_f32 = check_pool(pool)
     out = np.zeros(len(pool_h), dtype=np.float32)
     rec = packed_records(records, explicit_dt=1)
     n = len(rec)
     if n == 0 or len(pool_h) == 0:
         return (out, None) if return_device else out
-    # distinct configs -> wfb_filter_cfg[]
-    keys = rec["board"].astype(np.int64) * 65536 + (rec["channel"].astype(np.int64) & 0xFFFF)
-    uniq, inv = np.unique(keys, return_inverse=True)
-    cfg_list = []
-    for k in uniq.tolist():
-        b, c = int(k >> 16), ((int(k) & 0xFFFF) ^ 0x8000) - 0x8000
-        cfg_list.append(configs.get((b, c), default))
-    cfgs = (_lib.FilterCfg * len(cfg_list))()
-    tables: list[np.ndarray] = []
-    table_off: dict[tuple[int, int], int] = {}
-    cursor = 0
-    lens = rec["event_length"].astype(np.int64)
-    tab_off = np.full(n, -1, dtype=np.int32)
-    for ci, cfg in enumerate(cfg_list):
-        if cfg["filter_type"] == "BW":
-            sos = np.asarray(cfg["sos"], dtype=np.float64)
-            if sos.shape[0] > _lib.MAX_SOS_SECTIONS:
-                raise ValueError(f"filter_order too high: {sos.shape[0]} sections > {_lib.MAX_SOS_SECTIONS}")
-            zi = sos_zi(sos)
-            cfgs[ci].type = 1
-            cfgs[ci].n_sections = sos.shape[0]
-            for s in range(sos.shape[0]):
-                for j in range(6):
-                    cfgs[ci].sos[s][j] = sos[s, j]
-                cfgs[ci].zi[s][0], cfgs[ci].zi[s][1] = zi[s, 0], zi[s, 1]
-        else:
-            w0, poly = int(cfg["sg_window_size"]), int(cfg["sg_poly_order"])
-            cfgs[ci].type = 0
-            cfgs[ci].sg_window = w0
-            cfgs[ci].sg_poly = poly
-            sel = np.flatnonzero(inv == ci)
-            weff = np.minimum(w0, lens[sel])
-            weff = weff - (weff % 2 == 0)
-            for w in np.unique(weff).tolist():
-                if w <= poly or w <= 0:
-                    continue  # identity (filtering.py:193-194)
-                if (w, poly) not in table_off:
-                    t = sg_tables(int(w), poly)
-                    table_off[(w, poly)] = cursor
-                    tables.append(t)
-                    cursor += len(t)
-                tab_off[sel[weff == w]] = table_off[(w, poly)]
-    d_cfg = torch.from_numpy(np.frombuffer(bytes(cfgs), dtype=np.uint8).copy()).cuda()
-    d_idx = _dev(inv.astype(np.int32))
-    d_tab = _dev(np.concatenate(tables) if tables else np.zeros(1))
-    d_toff = _dev(tab_off)
     if run is None:
         run = DeviceRun.from_host(rec, pool_h)
-    d_out = torch.empty(len(pool_h) + 16, dtype=torch.float32, device="cuda")[: len(pool_h)]
-    lmax = max(int(lens.max()), 1)
-    has_bw = any(c["filter_type"] == "BW" for c in cfg_list)
-    ws = _empty(lib.wfb_filter_workspace_bytes(n, lmax)) if has_bw else None
-    _lib.check(lib.wfb_filter_pool(_ptr(run.pool), is_f32, len(pool_h), _ptr(run.meta), n, _ptr(d_cfg), len(cfg_list), _ptr(d_idx),
-                                   _ptr(d_tab), _ptr(d_toff), _ptr(d_out), 0, _ptr(ws), 0 if ws is None else ws.numel(), lmax,
-                                   _stream()), "wfb_filter_pool")
+    lens = rec["event_length"]
+    per_channel = {bc: configs.get(bc, default) for bc in unique_channels(rec["board"], rec["channel"])}
+    plan = filter_plan(run, per_channel, lengths=np.unique(lens))
+    d_out = _filter_launch(run, plan, len(pool_h), max(int(lens.max()), 1))
     host = d_out.cpu().numpy()
     if return_device:  # the filtered pool stays in HBM for the next plugin (same records metadata, float32 samples)
         return host, DeviceRun(run.meta, d_out, n, 1, run.lmax, records_rows=run.records_rows, pool_base=run.pool_base, row_base=run.row_base)
     return host
-
 
 # --------------------------------------------------------------------------------------------
 # waveform_width / waveform_width_integral
@@ -1124,71 +1253,26 @@ def hit_event_table_device(d_rows, n: int, row_bytes: int, group: dict) -> dict:
                             group["dt"], group["abs_start"], group["abs_end"], rows=d_rows, row_bytes=rb)
 
 
-def _sg_tables_by_length(w0: int, poly: int, wcap: int):
-    """SG tables of every effective window a record of length 0..wcap can get (min(w0, L), forced odd, identity when
-    <= poly): (concatenated tables, int32 offset per length, -1 = identity).  The table of the longest records comes
-    first, at offset 0."""
-    eff = np.minimum(w0, np.arange(wcap + 1))
-    eff = eff - (eff % 2 == 0)
-    tables, at = [], {}
-    cursor = 0
-    for w in sorted(set(eff.tolist()), reverse=True):
-        if w <= poly or w <= 0:
-            continue
-        at[w] = cursor
-        tables.append(sg_tables(int(w), poly))
-        cursor += len(tables[-1])
-    lut = np.array([at.get(w, -1) for w in eff.tolist()], dtype=np.int32)
-    return (np.concatenate(tables) if tables else np.zeros(1)), lut
+def filter_run_device(run: DeviceRun, cfg: dict | None = None, *, filter_options: dict | None = None, channel_config=None,
+                      run_id: str | None = None):
+    """wfb_filter_pool on a device-resident run (benchmarks, multi-GPU shards): returns the float32 pool as a device
+    tensor, nothing crosses PCIe.
 
-
-def filter_run_device(run: DeviceRun, cfg: dict):
-    """wfb_filter_pool on a device-resident run with ONE configuration for every record (benchmarks, multi-GPU shards):
-    returns the float32 pool as a device tensor, nothing crosses PCIe.  ``cfg`` as ``filter_pool``'s ``default``.
-
-    An SG record shorter than the window is filtered with its own effective window min(window, L) (forced odd; left
-    unchanged when that is <= poly): one table per effective window, the record's table offset looked up on the device
-    from its event_length.  A run whose records are all at least the window long (``run.lmin``) uses one table."""
-    lib = _lib.load()
-    torch = _torch()
-    n, L = run.n, max(run.lmax, 1)
-    cfgs = (_lib.FilterCfg * 1)()
-    tab = np.zeros(1)
-    toff = -1
-    d_toff = None
-    if cfg["filter_type"] == "BW":
-        sos = np.asarray(cfg["sos"], dtype=np.float64)
-        zi = sos_zi(sos)
-        cfgs[0].type = 1
-        cfgs[0].n_sections = sos.shape[0]
-        for s in range(sos.shape[0]):
-            for j in range(6):
-                cfgs[0].sos[s][j] = sos[s, j]
-            cfgs[0].zi[s][0], cfgs[0].zi[s][1] = zi[s, 0], zi[s, 1]
+    ``cfg`` (as ``filter_pool``'s ``default``): one configuration for every record.  ``filter_options`` (the
+    ``B200WavePoolFilteredPlugin`` options named in ``FILTER_OPTION_NAMES``; missing ones take the plugin's defaults)
+    with ``channel_config``: every channel of the run resolved the way the plugin resolves it for ``run_id``.  Each
+    record gets its configuration and its Savitzky-Golay table (effective window min(window, L), forced odd, left
+    unchanged when that is <= poly) from wfb_filter_plan on the device."""
+    if (cfg is None) == (filter_options is None):
+        raise ValueError("filter_run_device takes one of cfg and filter_options")
+    if cfg is not None:
+        plan = filter_plan(run, {}, cfg)
     else:
-        w0, poly = int(cfg["sg_window_size"]), int(cfg["sg_poly_order"])
-        cfgs[0].type, cfgs[0].sg_window, cfgs[0].sg_poly = 0, w0, poly
-        wcap = min(w0, L)
-        if run.lmin is not None and run.lmin >= wcap:  # every record gets the same window
-            w = wcap - (wcap % 2 == 0)
-            if w > poly and w > 0:
-                tab, toff = sg_tables(int(w), poly), 0
-        elif n:
-            tab, lut = _sg_tables_by_length(w0, poly, wcap)
-            lens = run.meta[: n * 48].view(n, 48)[:, 24:28].contiguous().view(torch.int32).view(-1)  # wfb_rec_meta.event_length
-            d_toff = upload(lut)[lens.clamp(0, wcap).long()]
-    d_cfg = upload(np.frombuffer(bytes(cfgs), dtype=np.uint8).copy())
-    d_idx = torch.zeros(max(n, 1), dtype=torch.int32, device="cuda")
-    d_tab = upload(np.ascontiguousarray(tab, dtype=np.float64))
-    if d_toff is None:
-        d_toff = torch.full((max(n, 1),), toff, dtype=torch.int32, device="cuda")
-    d_out = torch.empty(run.pool_len + 16, dtype=torch.float32, device="cuda")[: run.pool_len]
-    ws = _empty(lib.wfb_filter_workspace_bytes(n, L)) if cfg["filter_type"] == "BW" else None
-    _lib.check(lib.wfb_filter_pool(_ptr(run.pool), run.pool_is_f32, run.pool_len, _ptr(run.meta), n, _ptr(d_cfg), 1, _ptr(d_idx), _ptr(d_tab),
-                                   _ptr(d_toff), _ptr(d_out), run.pool_base, _ptr(ws), 0 if ws is None else ws.numel(), L, _stream()),
-               "wfb_filter_pool")
-    return d_out
+        from .plugins.filtering import channel_filter_configs
 
+        per_channel, default = channel_filter_configs(shard_channels(run), filter_options, channel_config, run_id)
+        plan = filter_plan(run, per_channel, None if per_channel else default)
+    return _filter_launch(run, plan, run.pool_len, max(run.lmax, 1))
 
 # --------------------------------------------------------------------------------------------
 # st_waveforms: structured rows with the dual baseline (waveforms.py:644-799)

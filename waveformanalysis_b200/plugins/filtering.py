@@ -49,6 +49,21 @@ def resolve_filter_config(values: dict) -> dict:
     return {"filter_type": "SG", "sg_window_size": w, "sg_poly_order": p}
 
 
+def channel_filter_configs(channels, filter_options: dict, channel_config: Any, run_id: str | None) -> tuple[dict, dict]:
+    """({(board, channel): designed filter} for ``channels``, the designed filter of the options themselves).
+
+    ``filter_options``: values of the options in FILTER_OPTION_NAMES (missing ones take the plugin's defaults),
+    overridden per channel by ``channel_config`` for ``run_id``.  Resolution is a function of (run_id, board, channel)
+    alone, so processes that hold different channels of one run agree on every channel they share."""
+    unknown = sorted(set(filter_options) - set(FILTER_OPTION_NAMES))
+    if unknown:
+        raise ValueError(f"unknown filter options {unknown}; expected a subset of {FILTER_OPTION_NAMES}")
+    base_values = {k: B200WavePoolFilteredPlugin.options[k].default for k in FILTER_OPTION_NAMES}
+    base_values.update(filter_options)
+    default = resolve_filter_config(base_values)
+    return {(b, c): resolve_filter_config(resolve_channel_values(channel_config, run_id, b, c, base_values)) for b, c in channels}, default
+
+
 class B200WavePoolFilteredPlugin(Plugin):
     """Build a filtered wave_pool aligned to the existing records layout."""
 
@@ -92,10 +107,8 @@ class B200WavePoolFilteredPlugin(Plugin):
         boards = records["board"] if "board" in names else np.zeros(len(records), np.int16)
         channels = records["channel"] if "channel" in names else np.zeros(len(records), np.int16)
         base_values = {k: context.get_config(self, k) for k in FILTER_OPTION_NAMES}
-        channel_config = context.get_config(self, "channel_config")
-        configs = {}
-        for b, c in unique_channels(boards, channels):
-            configs[(b, c)] = resolve_filter_config(resolve_channel_values(channel_config, run_id, b, c, base_values))
+        configs, default = channel_filter_configs(unique_channels(boards, channels), base_values, context.get_config(self, "channel_config"),
+                                                  run_id)
         off = records["wave_offset"].astype(np.int64)
         ln = records["event_length"].astype(np.int64)
         if np.any((ln > 0) & ((off < 0) | (off + ln > len(wave_pool)))):
@@ -104,12 +117,11 @@ class B200WavePoolFilteredPlugin(Plugin):
         from ..dtypes import RECORDS_DTYPE
 
         if records.dtype != RECORDS_DTYPE or not residency.fits_device(int(wave_pool.nbytes) * 3):
-            return ops.filter_pool(records, wave_pool, configs=configs, default=resolve_filter_config(base_values))
+            return ops.filter_pool(records, wave_pool, configs=configs, default=default)
         # the raw pool is (or becomes) resident; the filtered pool stays in HBM under the host array handed back, so a
         # hit / feature plugin with use_filtered finds it there (the reference shares its bundle: records.py:441-464)
         run = residency.device_run(run_id, records, wave_pool, "wave_pool")
-        host, frun = ops.filter_pool(records, wave_pool, configs=configs, default=resolve_filter_config(base_values), run=run,
-                                     return_device=True)
+        host, frun = ops.filter_pool(records, wave_pool, configs=configs, default=default, run=run, return_device=True)
         if frun is not None:
             residency.adopt_run(run_id, records, host, "wave_pool_filtered", frun)
         return host
